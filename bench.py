@@ -2,6 +2,7 @@
 """bench.py -- the hot path's headline benchmark (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3|cfg2|cfg4|cfg5] [--scaling strong|weak]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference's CPU path (oracle port) on host cores
 
@@ -436,6 +437,10 @@ def run_pair(args, cfg, rig):
     launches = ctx.launch_count - launches0
     clocks = sampler.stop() if sampler else None
     m, res = result()
+    if args.dump_outputs and rank == 0:
+        # the outputs are identical on every rank of a strong-scaling clique; weak scaling dumps rank 0's own pair
+        dump_outputs(args.dump_outputs, {"n_matches": m, **dmatch_arrays(d_matches[:m].cpu().numpy()),
+                                         "inlier_mask": d_mask[:m].cpu().numpy(), **pose_arrays(res)})
     sc_stats = ctx.last_score_stats()
     stats = ctx.last_knn_stats()
     # max over ranks of the device-timed sums (the step of a rank ends when its pose is done; collectives inside)
@@ -578,6 +583,36 @@ def run_pair(args, cfg, rig):
     }
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes what the timed path returned in its last step as <out_dir>/<name>.npy, so that two builds can be compared
+    output for output on identical (seeded) inputs.  float32 results stay float32; everything else (indices, counts,
+    fp64 matrices) is stored as float64, which holds every int32 exactly."""
+    arrays = {k: (a if a.dtype == np.float32 else a.astype(np.float64)) for k, a in ((k, np.asarray(v)) for k, v in arrays.items())}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"dump of {total} bytes exceeds {DUMP_LIMIT}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dmatch_arrays(m, prefix="matches_"):
+    """erp_dmatch records (cv::DMatch layout) as one array per field."""
+    from erp_match_eightpoint_test_b200 import binding
+
+    m = np.ascontiguousarray(m).view(binding.DMATCH).reshape(-1)
+    return {prefix + "query_idx": m["queryIdx"], prefix + "train_idx": m["trainIdx"], prefix + "img_idx": m["imgIdx"],
+            prefix + "distance": m["distance"]}
+
+
+def pose_arrays(res):
+    """The fields of erp_ransac_result a caller reads (`packed` is count and hyp_id together)."""
+    return {"hyp_id": res["hyp"], "count": res["count"], "n_refit": res["n_refit"], "E_best": res["E"], "E_refit": res["E_refit"],
+            "pose": res["pose"]}
+
+
 def C_sizeof_result():
     import ctypes
 
@@ -635,6 +670,9 @@ def run_match(args, cfg, rig):
     launches = ctx.launch_count - launches0
     clocks = sampler.stop() if sampler else None
     n_local = int(d_n.item())
+    if args.dump_outputs and rank == 0:
+        # strong scaling: rank 0's query rows (global query ids) are what its caller receives
+        dump_outputs(args.dump_outputs, {"n_matches": n_local, **dmatch_arrays(d_matches[:n_local].cpu().numpy())})
     stats = ctx.last_knn_stats()
     t_match, t_kernel = rig.max_over_ranks([t_match, t_kernel])
     n_total, launches_all = rig.sum_over_ranks([n_local if (strong or world == 1) else n_local / world, launches])
@@ -642,7 +680,7 @@ def run_match(args, cfg, rig):
     pq, pt = h_q.numpy(), h_t.numpy()
     t_e2e = 0.0
     mt = None
-    e2e_steps = max(1, min(args.steps, 10))
+    e2e_steps = args.steps
     for it in range(e2e_steps + 1):
         torch.cuda.synchronize()
         a = time.perf_counter()
@@ -701,7 +739,7 @@ def run_video(args, cfg, rig):
     first = [None] * cfg["distinct"]
     errs = []
 
-    def batch(check):
+    def batch(check, keep=None):
         def work(tid):
             try:
                 c = ctxs[tid]
@@ -710,6 +748,8 @@ def run_video(args, cfg, rig):
                     h = host[d]
                     m, r = c.pair_pose(h["q"], h["t"], h["left"], h["right"], cfg["W"], cfg["H"], ratio=RATIO, seed=1, H=cfg["hyps"],
                                        S=SAMPLE, metric=METRIC, tau=TAU)
+                    if keep is not None:
+                        keep[j] = (len(m), r, m if j < cfg["distinct"] else None)      # records of the first pairs only (size cap)
                     key = (len(m), r["packed"])
                     if check:
                         if first[d] is None:
@@ -733,8 +773,9 @@ def run_video(args, cfg, rig):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     wall0 = time.perf_counter()
-    for _ in range(args.steps):
-        batch(False)
+    last = {} if args.dump_outputs else None
+    for s in range(args.steps):
+        batch(False, last if s == args.steps - 1 else None)
     e1.record()
     e1.synchronize()
     rig.barrier()
@@ -752,6 +793,18 @@ def run_video(args, cfg, rig):
         c.close()
     if rank != 0:
         return None
+    if last is not None:
+        # per pair of this rank (in `mine` order): match count and pose; match records and masks of its first `distinct` pairs
+        # (one per distinct input; all of them would exceed the dump's size cap)
+        rows = [pose_arrays(last[j][1]) for j in range(len(mine))]
+        out = {k: np.stack([np.asarray(r[k]) for r in rows]) for k in rows[0]}
+        out["pair"] = np.array(mine)
+        out["n_matches"] = np.array([last[j][0] for j in range(len(mine))])
+        first_pairs = range(min(cfg["distinct"], len(mine)))
+        out.update(dmatch_arrays(np.concatenate([last[j][2] for j in first_pairs])))
+        out["matches_pair"] = np.concatenate([np.full(last[j][0], mine[j]) for j in first_pairs])
+        out["inlier_mask"] = np.concatenate([last[j][1]["mask"] for j in first_pairs])
+        dump_outputs(args.dump_outputs, out)
     n_pl = int((distinct[0]["planted"] >= 0).sum())
     assert first[mine[0] % cfg["distinct"]][0] == int((distinct[mine[0] % cfg["distinct"]]["planted"] >= 0).sum())
     pairs = cfg["pairs"]
@@ -795,7 +848,13 @@ def main():
     ap.add_argument("--engine", type=int, default=None, help="0 auto, 1 exact SIMT, 2 tcgen05 3xTF32, 3 tcgen05 1xTF32")
     ap.add_argument("--threads", type=int, default=2, help="cfg5: host threads (contexts) per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the product arm")
     cfg = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, cfg)
@@ -808,4 +867,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
     main()

@@ -6,11 +6,13 @@ reference calls, as exposed by cv2:
   cv2.BFMatcher(NORM_L2).knnMatch(k=2) / crossCheck  <-> feature_matcher.cpp:45 (exact limit of FLANN)
   cv2.SVDecomp                                       <-> eight_point.cpp:39,46
   cv2.decomposeEssentialMat                          <-> eight_point.cpp:54
+  cv2.invert on 3x3 CV_64F                           <-> erp_rotation.cpp:103 (cv::Mat::inv)
 cv2 4.13 is built with LAPACK, so singular vectors can differ from OpenCV's own
 Jacobi SVD by per-vector sign; consumers compare up to those signs.
 
 Run from the repo root:  python tests/golden/make_golden.py
 """
+import hashlib
 import os
 import sys
 
@@ -81,8 +83,33 @@ def eight_point_cases():
     np.savez_compressed(os.path.join(HERE, "eight_point.npz"), **out)
 
 
+def cfg2_matching():
+    """configs[1] at full size (20k x 20k SURF-64, the inputs of tests/test_gpu_parity.py's cv2 comparison):
+    cv2.BFMatcher(NORM_L2).knnMatch(k=2) indices and fp32 distances, and digests of the inputs they belong to."""
+    q, t, _ = synth.descriptor_pair(20000, 20000, 64, seed=synth.SEED_BASE + 1)
+    t[137] = t[12]; t[5] = t[12]; q[3] = t[12]
+    kn = cv2.BFMatcher(cv2.NORM_L2).knnMatch(q, t, k=2)
+    np.savez_compressed(os.path.join(HERE, "cfg2_bfmatcher.npz"),
+                        idx=np.array([[m[0].trainIdx, m[1].trainIdx] for m in kn], np.int32),
+                        dist=np.array([[m[0].distance, m[1].distance] for m in kn], np.float32),
+                        q_sha1=hashlib.sha1(q.tobytes()).hexdigest(), t_sha1=hashlib.sha1(t.tobytes()).hexdigest())
+
+
+def inverse3():
+    """cv2.invert of the 3x3 matrices tests/test_oracle.py inverts: 20 normal draws and the oracle's eular2rot([0.3, -1.1, 2])."""
+    import oracle as O
+
+    rng = np.random.default_rng(0)
+    A = np.stack([rng.normal(size=(3, 3)) for _ in range(20)])
+    R = O.eular2rot([0.3, -1.1, 2.0])
+    np.savez_compressed(os.path.join(HERE, "inv3.npz"), A=A, A_inv=np.stack([cv2.invert(a)[1] for a in A]),
+                        R=R, R_inv=cv2.invert(R)[1])
+
+
 if __name__ == "__main__":
     matching()
     svd_and_decompose()
     eight_point_cases()
+    cfg2_matching()
+    inverse3()
     print("golden fixtures written to", HERE)

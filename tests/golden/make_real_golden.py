@@ -11,10 +11,12 @@ using the ORACLE's restatement of crop_rotated_image / rotate_keypoint (oracle/e
 matcher on the result: cv2.BFMatcher(NORM_L2).knnMatch(k=2) and the crossCheck match.  Real facade structure (repeated
 windows) produces the near-ties and low-contrast ratio tests that Gaussian synthetic descriptors never do.
 
-Run from the repo root IN THIS CONTAINER (needs /root/reference):  python tests/golden/make_real_golden.py
+Run from the repo root with a checkout of the reference:  python tests/golden/make_real_golden.py <reference checkout>
+The archive is written with LZMA members (np.load reads them) to keep the fixture under 1 MB.
 """
 import os
 import sys
+import zipfile
 
 import cv2
 import numpy as np
@@ -23,7 +25,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import oracle as O  # noqa: E402
 
-REF = "/root/reference/build"
 PER_STRIP = 1200          # strongest SIFT features kept per strip (fixture size: 2 x 4 x 1200 x 128 bytes)
 SCALE = 0.5               # the 5376 x 2688 originals are halved: 2688 x 1344 (a 4K-class ERP pair keeps the fixture small)
 
@@ -50,11 +51,11 @@ def describe(im):
     return np.concatenate(keys).astype(np.float32), np.concatenate(descs).astype(np.float32)
 
 
-def main():
+def main(ref):
     out = {}
     ims = {}
     for side in ("left", "right"):
-        im = cv2.imread(os.path.join(REF, side + "_building.jpg"), cv2.IMREAD_COLOR)
+        im = cv2.imread(os.path.join(ref, "build", side + "_building.jpg"), cv2.IMREAD_COLOR)
         im = cv2.resize(im, None, fx=SCALE, fy=SCALE, interpolation=cv2.INTER_AREA)
         ims[side] = im
         xy, d = describe(im)
@@ -68,9 +69,12 @@ def main():
     out["bf_dist"] = np.array([[m[0].distance, m[1].distance] for m in kn], np.float32)
     cc = cv2.BFMatcher(cv2.NORM_L2, crossCheck=True).match(q, t)
     out["bf_cross"] = np.array(sorted((m.queryIdx, m.trainIdx) for m in cc), np.int32)
-    np.savez_compressed(os.path.join(HERE, "real_building.npz"), **out)
+    with zipfile.ZipFile(os.path.join(HERE, "real_building.npz"), "w", compression=zipfile.ZIP_LZMA) as z:
+        for k, v in out.items():
+            with z.open(k + ".npy", "w") as f:
+                np.lib.format.write_array(f, np.asanyarray(v))
     print({k: (v.shape if hasattr(v, "shape") else v) for k, v in out.items()})
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

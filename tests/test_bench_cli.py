@@ -54,6 +54,46 @@ def test_reference_arm_runs_on_rank_zero_only():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_steps_and_dump_arguments_are_checked():
+    assert run_bench("--impl", "reference", "--workload", "cfg2", "--steps", "0").returncode == 2
+    assert run_bench("--impl", "reference", "--workload", "cfg2", "--dump-outputs", "unused").returncode == 2
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_timed_path_results(tmp_path):
+    """--dump-outputs writes the last timed step's outputs (cfg2: match records, inlier mask, winner and pose) as float32 /
+    float64 .npy files; they equal the oracle on the benchmark's seeded inputs, and a second run writes the same bytes."""
+    import numpy as np
+
+    import bench
+    import oracle as O
+
+    runs = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        r = run_bench("--workload", "cfg2", "--steps", "3", "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(out))
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+        assert line["steps"] == 3 and line["e2e"]["steps"] == 3
+        runs.append({f[:-4]: np.load(out / f) for f in sorted(os.listdir(out))})
+    d = runs[0]
+    assert sum(a.nbytes for a in d.values()) <= 64 << 20
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values())
+    assert d.keys() == runs[1].keys() and all(d[k].tobytes() == runs[1][k].tobytes() for k in d)
+    cfg = bench.WORKLOADS["cfg2"]
+    pair = bench.make_pair(cfg, 0xE8B0 + 3)
+    om = O.match(pair["q"], pair["t"], bench.RATIO, False)
+    assert int(d["n_matches"]) == len(om)
+    for key, field in (("query_idx", "queryIdx"), ("train_idx", "trainIdx"), ("img_idx", "imgIdx"), ("distance", "distance")):
+        assert np.array_equal(d["matches_" + key], om[field]), key
+    l = O.bearings(pair["left"][om["queryIdx"]], cfg["W"], cfg["H"])
+    r = O.bearings(pair["right"][om["trainIdx"]], cfg["W"], cfg["H"])
+    ref = O.ransac(l, r, seed=1, hyp0=0, H=cfg["hyps"], S=bench.SAMPLE, metric=bench.METRIC, tau=bench.TAU)
+    assert int(d["hyp_id"]) == ref["hyp"] and int(d["count"]) == ref["count"] == int(d["inlier_mask"].sum())
+    assert np.array_equal(d["inlier_mask"], O.inlier_mask(ref["E"], l, r, metric=bench.METRIC, tau=bench.TAU))
+    assert d["E_best"].shape == d["E_refit"].shape == (3, 3) and d["pose"].shape == (12,)
+
+
 def test_product_arm_has_no_cpu_fallback():
     import torch
     if torch.cuda.is_available():

@@ -6,12 +6,15 @@ Bars (north_star): match indices and distances bit-exact (the oracle and the dev
 the same fp64 chain); inlier counts and masks bit-exact (same fp32 fma chain); E within 1e-5
 Frobenius after sign/scale normalisation given the same samples; poses within 1e-5.
 """
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
 import erp_match_eightpoint_test_b200 as erp
 import oracle as O
-from conftest import e_dist
+from conftest import GOLDEN, e_dist
 from erp_match_eightpoint_test_b200 import binding, synth
 
 pytestmark = pytest.mark.gpu
@@ -593,13 +596,13 @@ def test_cfg2_full_size_against_cv2_bfmatcher_with_near_tie_report(ctx):
     """configs[1] at full size against the third-party matcher itself: cv2.BFMatcher(NORM_L2).knnMatch(k=2) computes
     and compares in fp32 (as src/feature_matcher.cpp:45,52 does); the device result is exact.  north_star: indices
     bit-exact except for documented fp32 distance ties.  Every query on which cv2 returns another index must be in the
-    near-tie report (erp_knn2_near_ties); the report itself is checked against its definition on a sub-sample."""
-    cv2 = pytest.importorskip("cv2")
+    near-tie report (erp_knn2_near_ties); the report itself is checked against its definition on a sub-sample.
+    cv2's output is tests/golden/cfg2_bfmatcher.npz (written by tests/golden/make_golden.py from these inputs)."""
     q, t, planted = synth.descriptor_pair(20000, 20000, 64, seed=synth.SEED_BASE + 1)
     t[137] = t[12]; t[5] = t[12]; q[3] = t[12]                          # exact ties: lowest trainIdx first, on both sides
-    kn = cv2.BFMatcher(cv2.NORM_L2).knnMatch(q, t, k=2)
-    cidx = np.array([[m[0].trainIdx, m[1].trainIdx] for m in kn], np.int32)
-    cdist = np.array([[m[0].distance, m[1].distance] for m in kn], np.float32)
+    g = np.load(os.path.join(GOLDEN, "cfg2_bfmatcher.npz"))
+    assert hashlib.sha1(q.tobytes()).hexdigest() == g["q_sha1"] and hashlib.sha1(t.tobytes()).hexdigest() == g["t_sha1"]
+    cidx, cdist = g["idx"], g["dist"]
     idx, dist = ctx.knn2_raw(q, t)
     # fp32 accumulation of 64 terms: documented tolerance of the report = 64 * 2^-24 relative on the distance
     tol = 64 * 2.0 ** -24
