@@ -21,6 +21,7 @@ POSE_FLOATS = 12
 
 METRIC_ALGEBRAIC, METRIC_SAMPSON, METRIC_ANGULAR = 0, 1, 2
 ENGINE_AUTO, ENGINE_EXACT_SIMT, ENGINE_TCGEN05, ENGINE_TCGEN05_1X = 0, 1, 2, 3
+OPERANDS_NONE, OPERANDS_TF32, OPERANDS_F16 = 0, 1, 2
 
 OK = 0
 E_ARG, E_DIM, E_TOO_FEW_TRAIN, E_TOO_FEW_POINTS, E_NO_CANDIDATE, E_LIMIT = 1, 2, 3, 4, 5, 6
@@ -54,6 +55,7 @@ _SIGNATURES = {
     "erp_ctx_device": (C.c_int, [C.c_void_p]),
     "erp_ctx_launch_count": (C.c_uint64, [C.c_void_p]),
     "erp_ctx_last_knn_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "erp_ctx_last_knn_operands": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "erp_ctx_last_knn_kernel_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "erp_ctx_last_score_kernel_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "erp_ctx_last_score_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
@@ -247,6 +249,13 @@ class Context:
         out = (C.c_int64 * 5)()
         _check(lib().erp_ctx_last_knn_stats(self._h, out))
         return dict(engine=out[0], rescanned=out[1], chunks=out[2], items=out[3], deviation=out[4] * 1e-12)
+
+    def last_knn_operands(self):
+        """Operand format of the last search's tensor products (OPERANDS_*), whether the f16 range guard fired, and how many
+        queries the f16 range checks sent to the exact re-scan."""
+        out = (C.c_int64 * 3)()
+        _check(lib().erp_ctx_last_knn_operands(self._h, out))
+        return dict(operands=out[0], guard=bool(out[1]), range_rescanned=out[2])
 
     def last_knn_kernel_ms(self) -> float:
         ms = C.c_float(0)

@@ -388,6 +388,24 @@ ERP_API int erp_ctx_last_knn_stats(erp_ctx* ctx, int64_t out[5])
     return ERP_OK;
 }
 
+ERP_API int erp_ctx_last_knn_operands(erp_ctx* ctx, int64_t out[3])
+{
+    ERP_ARG(ctx && out, ERP_E_ARG, "erp_ctx_last_knn_operands: bad argument");
+    const int64_t engine = ctx->knn_stats[0];
+    out[0] = engine == ERP_ENGINE_TCGEN05 ? ERP_OPERANDS_TF32
+           : engine == ERP_ENGINE_TCGEN05_1X ? (tc1_f16_operands() ? ERP_OPERANDS_F16 : ERP_OPERANDS_TF32) : ERP_OPERANDS_NONE;
+    out[1] = out[2] = 0;
+    if (out[0] == ERP_OPERANDS_F16 && ctx->tc_misc_dev) {
+        DeviceGuard g(ctx->device);
+        int32_t w[7] = {0, 0, 0, 0, 0, 0, 0};
+        ERP_CUDA(cudaMemcpyAsync(w, ctx->tc_misc_dev, sizeof w, cudaMemcpyDeviceToHost, ctx->stream));
+        ERP_CUDA(cudaStreamSynchronize(ctx->stream));
+        out[1] = w[5] != 0;
+        out[2] = w[6];
+    }
+    return ERP_OK;
+}
+
 // ======================================================================================
 // matching
 // ======================================================================================

@@ -190,12 +190,13 @@ bool knn2_tc_preferred(int nq, int nt, int dim);
 bool knn2_tc1_preferred(int nq, int nt, int dim);
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2);
+bool tc1_f16_operands();
 int near_ties(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim, const int32_t* d_idx2, const double* d_d2,
               double rel_tol, int32_t* d_third, uint8_t* d_flags);
 int tc_misc_begin(erp_ctx* ctx, int32_t* misc);
 int tc_misc_end(erp_ctx* ctx, int32_t* misc);
 int refine_launch(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim, int n_lists, int topk, double kappa,
-                  const int32_t* cand, const float* cand_s, const float* cand_thr, unsigned* misc, int32_t* d_idx2, float* d_dist2,
+                  double f16_abs, const int32_t* cand, const float* cand_s, const float* cand_thr, unsigned* misc, int32_t* d_idx2, float* d_dist2,
                   double* d_d2, int32_t* rescan_list);
 int knn2_exact_rescan(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
                       const int32_t* d_list, const int32_t* d_count, int max_rows,

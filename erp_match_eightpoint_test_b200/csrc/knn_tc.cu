@@ -329,8 +329,8 @@ __device__ __forceinline__ bool lex_less(double d, int i, double bd, int bi) { r
 template <int SPL>
 __global__ void __launch_bounds__(256)
 refine_kernel(const float* __restrict__ q, int nq, const float* __restrict__ t, int nt, int dim, int n_groups, int topk, double kappa,
-              const int32_t* __restrict__ cand_idx, const float* __restrict__ cand_s, const float* __restrict__ cand_thr,
-              unsigned* __restrict__ misc /* [0] re-scan count, [1] max |t|^2 bits, [2] max deviation bits */,
+              double f16_abs, const int32_t* __restrict__ cand_idx, const float* __restrict__ cand_s, const float* __restrict__ cand_thr,
+              unsigned* __restrict__ misc /* [0] re-scan count, [1] max |t|^2 bits, [2] max deviation bits, [5], [6]: below */,
               int32_t* __restrict__ idx2, float* __restrict__ dist2, double* __restrict__ d2out,
               int32_t* __restrict__ rescan_list)
 {
@@ -453,7 +453,15 @@ refine_kernel(const float* __restrict__ q, int nq, const float* __restrict__ t, 
         const double eps = kappa * scale;
         // non-finite input anywhere (NaN compares false, inf norms) -> exact re-scan
         bool finite_in = scale < (double)INFINITY && scale == scale;
-        bool certified = finite_in && I1 != 0x7fffffff &&
+        // f16 operands (f16_abs >= 0, knn_tc1.cu): the call's range guard (misc[5]) and the absolute error of subnormal operands;
+        // queries that fail either go to the re-scan and are counted in misc[6]
+        bool in_range = true;
+        if (f16_abs >= 0.0 && finite_in) {
+            const double sub = 0x1p-24 * sqrt((double)dim) * (2.0 * sqrt(qn) + sqrt(tn_max)) + 0x1p-36;
+            in_range = misc[5] == 0u && sub <= f16_abs * scale;
+            if (!in_range) atomicAdd(misc + 6, 1u);
+        }
+        bool certified = finite_in && in_range && I1 != 0x7fffffff &&
                          (!(thr < INFINITY) /* every train row was a candidate */ || B1 < (double)thr + qn - eps);
         if (certified) {
             if (idx2) { idx2[2 * qi] = I0; idx2[2 * qi + 1] = I1; }
@@ -468,7 +476,8 @@ refine_kernel(const float* __restrict__ q, int nq, const float* __restrict__ t, 
 
 // topk must be a power of two, n_lists * topk <= 128
 // misc words of a tcgen05 call: [0] re-scan count of THIS call (also the length of its re-scan list), [1] max |t|^2 bits,
-// [2] max deviation bits, [3] max |q|^2 bits, [4] re-scan count summed over the query chunks of one host call
+// [2] max deviation bits, [3] max |q|^2 bits, [4] re-scan count summed over the query chunks of one host call,
+// [5] f16 range guard raised (by the prep of any chunk), [6] queries the f16 range checks sent to the re-scan (all chunks)
 __global__ void misc_reset_kernel(int32_t* misc) { misc[0] = 0; misc[3] = 0; }
 __global__ void misc_accum_kernel(int32_t* misc) { misc[4] += misc[0]; }
 int tc_misc_begin(erp_ctx* ctx, int32_t* misc)
@@ -489,15 +498,15 @@ int tc_misc_end(erp_ctx* ctx, int32_t* misc)
 }
 
 int refine_launch(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim, int n_lists, int topk, double kappa,
-                  const int32_t* cand, const float* cand_s, const float* cand_thr, unsigned* misc, int32_t* d_idx2, float* d_dist2,
+                  double f16_abs, const int32_t* cand, const float* cand_s, const float* cand_thr, unsigned* misc, int32_t* d_idx2, float* d_dist2,
                   double* d_d2, int32_t* rescan_list)
 {
     if (n_lists * topk > 128) { set_error("refine: %d candidate slots per query", n_lists * topk); return ERP_E_LIMIT; }
     if (n_lists * topk <= 64)
-        refine_kernel<2><<<cdiv(nq, 8), 256, 0, ctx->stream>>>(d_q, nq, d_t, nt, dim, n_lists, topk, kappa, cand, cand_s, cand_thr, misc,
+        refine_kernel<2><<<cdiv(nq, 8), 256, 0, ctx->stream>>>(d_q, nq, d_t, nt, dim, n_lists, topk, kappa, f16_abs, cand, cand_s, cand_thr, misc,
                                                                d_idx2, d_dist2, d_d2, rescan_list);
     else
-        refine_kernel<4><<<cdiv(nq, 8), 256, 0, ctx->stream>>>(d_q, nq, d_t, nt, dim, n_lists, topk, kappa, cand, cand_s, cand_thr, misc,
+        refine_kernel<4><<<cdiv(nq, 8), 256, 0, ctx->stream>>>(d_q, nq, d_t, nt, dim, n_lists, topk, kappa, f16_abs, cand, cand_s, cand_thr, misc,
                                                                d_idx2, d_dist2, d_d2, rescan_list);
     ERP_LAUNCH(ctx, "refine_kernel");
     return ERP_OK;
@@ -597,7 +606,7 @@ int knn2_tc(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, in
     }
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
 
-    ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, TOPK, KAPPA, cand, cand_s, cand_thr, reinterpret_cast<unsigned*>(misc),
+    ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, TOPK, KAPPA, -1.0, cand, cand_s, cand_thr, reinterpret_cast<unsigned*>(misc),
                           d_idx2, d_dist2, d_d2, list));
     ERP_TRY(knn2_exact_rescan(ctx, d_q, nq, d_t, nt, dim, list, misc, nq, d_idx2, d_dist2, d_d2));
     ERP_TRY(tc_misc_end(ctx, misc));

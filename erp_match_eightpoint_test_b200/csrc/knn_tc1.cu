@@ -1,34 +1,40 @@
-// knn_tc1.cu -- the fast tcgen05 distance engine: ONE TF32 product per tile, a wider candidate list
-// and the same exact certificate.
+// knn_tc1.cu -- the fast tcgen05 distance engine: ONE product of 11-bit operands per tile (f16 by default, tf32 on request),
+// a wider candidate list and the same exact certificate.
 //
 // knn_tc.cu reproduces fp32 ranking by arithmetic (3xTF32).  The certificate of refine_kernel makes
 // that unnecessary: any approximate score with a known error bound yields the exact 2-NN as long as
 //     d2_exact(second) < min_lists(s_kth) + |q|^2 - eps        (otherwise the query is re-scanned)
-// holds, and a single TF32 product has a worst-case error of 2^-10 (|q|^2 + |t|^2) (inputs rounded
+// holds, and a single product of 11-bit operands (TF32 or IEEE FP16) has a worst-case error of 2^-10 (|q|^2 + |t|^2) (inputs rounded
 // to 11 significant bits, products exact, fp32 accumulation).  Only columns within twice that error
 // of the running second best are kept (up to 8 per list: near-ties overflow 4), which for SURF-like
 // data leaves almost nothing to re-scan, so the kernel issues a third of the tensor work:
 //     8 UMMA instructions per 128 x 256 tile instead of 24.
-// At that rate the L2 -> shared-memory feed becomes the limiter, so every 64 KB train tile that TMA
+// FP16 operands (the default) carry the same 11 significant bits at twice the tf32 rate and half the bytes: 5 UMMA
+// instructions per tile at D = 64 (4 + the norm step) instead of 9, and 32 KB of train operand per tile instead of 64 KB.
+// ERP_B200_TC1_OPERANDS=tf32 selects the tf32 operands (same results, the A/B baseline).
+// At the tf32 rate the L2 -> shared-memory feed becomes the limiter, so every 64 KB train tile that TMA
 // brings in is multiplied against TWO resident query tiles (256 queries), alternating between the
 // two TMEM accumulators.  Results are identical to the exact engine by construction.
 #include "tc_common.cuh"
 
+#include <cuda_fp16.h>
+
 namespace erp {
 
 constexpr int F_BM = 128;                 // queries per sub-tile (UMMA M)
-constexpr int F_SUB_MAX = 2;              // resident query sub-tiles sharing every train tile (1 when D > 96: smem)
+constexpr int F_SUB_MAX = 2;              // resident query sub-tiles sharing every train tile (1 beyond three k chunks: smem)
 constexpr int F_BN = 256;                 // train rows per tile (UMMA N)
-constexpr int F_KC = 32;                  // floats per k chunk (one 128-byte swizzle row)
-constexpr int F_QCH = F_BM * F_KC * 4;    // 16 KB
-constexpr int F_TCH = F_BN * F_KC * 4;    // 32 KB
+// a k chunk is one 128-byte swizzle row: 32 floats or 64 halves
+__host__ __device__ constexpr int f_kc(bool half) { return half ? 64 : 32; }
+constexpr int F_QCH = F_BM * 128;         // 16 KB
+constexpr int F_TCH = F_BN * 128;         // 32 KB
 constexpr int F_EPI_GROUPS = 2;
 constexpr int F_EPI_THREADS = F_EPI_GROUPS * 128;
 constexpr int F_THREADS = 128 + F_EPI_THREADS;
 constexpr int F_EPI_COLS = F_BN / F_EPI_GROUPS;
 constexpr int F_TOPK = 8;
 constexpr int F_MAX_SEG = 128 / (F_TOPK * F_EPI_GROUPS);    // up to 8 segments per query pair (refine_kernel: 128 candidate slots)
-constexpr int F_AUG_T = F_BN * 32;        // 8 KB: one extra k step (8 floats) per train row, 32-byte swizzle rows
+constexpr int F_AUG_T = F_BN * 32;        // 8 KB: one extra k step (8 floats or 16 halves) per train row, 32-byte swizzle rows
 constexpr int F_AUG_Q = F_BM * 32;        // 4 KB: the constant query side of that k step
 constexpr int F_BARS = 256;               // mbarriers + TMEM slot
 // Instrumented builds (scripts/build_variant.sh N): -DERP_TC_COUNTERS=1 adds clock64 phase timers to the MMA issuer and the
@@ -49,14 +55,31 @@ static __device__ unsigned long long erp_clk[8];
 #define TCC_FLUSH()
 #endif
 // |s_tc - s_exact| <= 2^-10 (|q|^2 + max|t|^2) in the worst case: both operands are rounded to 11
-// significant bits (relative error 2^-11 each), products are exact, and 2|q||t| <= |q|^2 + |t|^2.
+// significant bits (relative error 2^-11 each: tf32 rounds to nearest away, f16 to nearest even, the worst case is the same),
+// products are exact (11 x 11 bits fit fp32, and so do f16 subnormal products), and 2|q||t| <= |q|^2 + |t|^2.
 // On top of 2^-10: the second-order rounding term (2^-22 relative = 2^-12 of the budget), the column id packed into the
 // three low mantissa bits of a score (<= 7 ulp = 2^-21 relative), and the fp32 accumulation inside the tensor pipe,
 // whose rounding mode is not documented: with truncating adds over D + 3 <= 131 terms the worst case is 131 * 2^-24
 // of the scale = 0.8 % of 2^-10.  Together < 2 %; 5 % is taken.  refine_kernel reports the deviation it observes
 // (0.28 of the bound on the synthetic sets; tests/test_gpu_parity.py holds a worst-case-rounding adversarial set).
+// f16 adds two things the relative bound does not cover, both handled without a host round trip:
+//   - values f16 cannot hold (|x| >= 65520 after the query's x(-2), or |t|^2 >= 65520 * 2^8 for the norm step): the prep
+//     kernel raises misc[5] and refine_kernel re-scans every query of the call exactly;
+//   - subnormal f16 operands (|x| < 2^-14) carry an absolute error <= 2^-25 each instead of a relative one, so a product
+//     errs by at most 2^-25 (|a~| + |b~|) beyond the relative term, which sums to <= 2^-25 sqrt(D) (2|q| + max|t|) (1 + 2^-10);
+//     the norm step adds <= 2^-39.  refine_kernel certifies a query only while 2^-24 sqrt(D) (2|q| + max|t|) + 2^-36 -- twice
+//     that -- stays within F_F16_ABS of the scale, 2 % of 2^-10 of the 3 % the budget above leaves.  That holds whenever
+//     |q| or max|t| is above ~0.1 (SURF is unit-norm, SIFT far above), so real descriptors never take this path.
 constexpr double F_KAPPA = 1.05 / 1024.0;
-constexpr uint32_t F_IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(F_BN >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
+constexpr double F_F16_ABS = 0.02 / 1024.0;
+// instruction descriptors: D fp32, A/B tf32 (format 2) or f16 (format 0), both K-major, N = 256, M = 128
+constexpr uint32_t F_IDESC_TF32 = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(F_BN >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
+constexpr uint32_t F_IDESC_F16 = (1u << 4) | ((uint32_t)(F_BN >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
+// f16 norm step: train row (hi, mid, lo, 0 x 5 | 0 x 8), query row (2^8, 2^-3, 2^-14, 2^15 x 5) in both 16-byte halves, so
+// |t|^2 = 2^8 hi + 2^-3 mid + 2^-14 lo (a 33-bit split of the fp32 norm: exact while hi is normal, within 2^-39 below).  Padding
+// train rows put 65504 into the five 2^15 slots: 1.07e10, finite, and above any score the range guard lets through
+// (|2q| |t| <= 65504 sqrt(128) * 4096 = 3.0e9 plus |t|^2 < 1.7e7)
+__host__ __device__ constexpr float f16_norm_scale(int i) { return i == 0 ? 256.0f : i == 1 ? 0.125f : i == 2 ? 1.0f / 16384.0f : 32768.0f; }
 
 __host__ __device__ constexpr int f_sub(int kch) { return kch <= 3 ? F_SUB_MAX : 1; }
 // D <= 64: |t|^2 enters the accumulator through the tensor core (an extra k step whose train side is the
@@ -73,40 +96,52 @@ __host__ __device__ constexpr bool f_share(int kch) { return f_slots_for(kch, tr
 __host__ __device__ constexpr int f_slots(int kch) { return f_slots_for(kch, f_share(kch)); }
 __host__ __device__ constexpr int f_smem(int kch) { return f_sub(kch) * kch * F_QCH + f_slots(kch) * F_TCH + f_tail(kch, f_share(kch)); }
 
-// rows -> tf32-rounded rows (dpad floats), optional norms (+inf padding) and their maximum
-// LPR lanes own one row (4 floats per lane and pass); a warp covers 32 / LPR rows
-// one operand of a prep launch: rows x, scaled, rounded into out; norms (+inf padding up to n_pad), their maximum, and the
-// 8-float norm operand rows when aug is given
+// one operand of a prep launch: rows x, scaled, rounded to tf32 or f16 into out (dpad elements per row); norms (+inf padding up
+// to n_pad), their maximum, and the 32-byte norm operand rows when aug is given
+// LPR lanes own one row (4 elements per lane and pass); a warp covers 32 / LPR rows
 struct RoundJob {
-    const float* x; int n; float scale; float* out; float* norm; int n_pad; unsigned* max_bits; float* aug; int blocks;
+    const float* x; int n; float scale; void* out; float* norm; int n_pad; unsigned* max_bits; void* aug; int blocks;
 };
 
+// f16 of a scaled input; a finite input whose f16 is infinite marks the call for the exact re-scan
+__device__ __forceinline__ __half f16_guarded(float x, float scaled, bool& wide)
+{
+    const __half h = __float2half_rn(scaled);
+    wide |= __hisinf(h) != 0 && fabsf(x) <= 3.4028235e38f;
+    return h;
+}
+
 // both operands of a search in ONE launch: blocks [0, a.blocks) round the queries, the rest the train rows
-template <int LPR>
+template <int LPR, bool HALF>
 __global__ void __launch_bounds__(256)
-round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad)
+round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad, unsigned* wide_flag)
 {
     constexpr int RPW = 32 / LPR;
     const bool second = (int)blockIdx.x >= a.blocks;
     const RoundJob& j = second ? b : a;
     const float* __restrict__ x = j.x;
-    float* __restrict__ out = j.out;
     float* __restrict__ norm = j.norm;
-    float* __restrict__ aug = j.aug;
     unsigned* __restrict__ max_bits = j.max_bits;
     const int n = j.n, n_pad = j.n_pad;
     const float scale = j.scale;
     const int lane = threadIdx.x & 31, sub = lane / LPR, l = lane % LPR;
     const int row = (((int)blockIdx.x - (second ? a.blocks : 0)) * 8 + (threadIdx.x >> 5)) * RPW + sub;
     double acc = 0.0;
+    bool wide = false;
     if (row < n) {
         for (int k = l * 4; k < dpad; k += LPR * 4) {
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
             if (k < dim) v = *reinterpret_cast<const float4*>(x + (size_t)row * dim + k);
             acc += (double)v.x * v.x + (double)v.y * v.y + (double)v.z * v.z + (double)v.w * v.w;
-            float4 hi = make_float4(tf32_rna(__fmul_rn(v.x, scale)), tf32_rna(__fmul_rn(v.y, scale)),
-                                    tf32_rna(__fmul_rn(v.z, scale)), tf32_rna(__fmul_rn(v.w, scale)));
-            *reinterpret_cast<float4*>(out + (size_t)row * dpad + k) = hi;
+            if (HALF) {
+                __half2* o = reinterpret_cast<__half2*>(static_cast<__half*>(j.out) + (size_t)row * dpad + k);
+                o[0] = __halves2half2(f16_guarded(v.x, __fmul_rn(v.x, scale), wide), f16_guarded(v.y, __fmul_rn(v.y, scale), wide));
+                o[1] = __halves2half2(f16_guarded(v.z, __fmul_rn(v.z, scale), wide), f16_guarded(v.w, __fmul_rn(v.w, scale), wide));
+            } else {
+                float4 hi = make_float4(tf32_rna(__fmul_rn(v.x, scale)), tf32_rna(__fmul_rn(v.y, scale)),
+                                        tf32_rna(__fmul_rn(v.z, scale)), tf32_rna(__fmul_rn(v.w, scale)));
+                *reinterpret_cast<float4*>(static_cast<float*>(j.out) + (size_t)row * dpad + k) = hi;
+            }
         }
     }
     if (norm) {
@@ -115,10 +150,27 @@ round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad)
         if (l == 0 && row < n_pad) {
             float f = row < n ? (float)acc : INFINITY;
             norm[row] = f;
-            if (aug) {
+            if (j.aug && HALF) {
+                // |t|^2 = 2^8 hi + 2^-3 mid + 2^-14 lo (f16_norm_scale); rows past the end fill the 2^15 slots
+                unsigned short h[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+                if (row < n) {
+                    const __half hi = f16_guarded(f, __fmul_rn(f, 1.0f / f16_norm_scale(0)), wide);
+                    const float r1 = __fsub_rn(f, __fmul_rn(__half2float(hi), f16_norm_scale(0)));
+                    const __half mid = __float2half_rn(__fmul_rn(r1, 1.0f / f16_norm_scale(1)));
+                    const float r2 = __fsub_rn(r1, __fmul_rn(__half2float(mid), f16_norm_scale(1)));
+                    const __half lo = __float2half_rn(__fmul_rn(r2, 1.0f / f16_norm_scale(2)));
+                    h[0] = __half_as_ushort(hi); h[1] = __half_as_ushort(mid); h[2] = __half_as_ushort(lo);
+                } else {
+                    for (int i = 3; i < 8; i++) h[i] = 0x7bffu;   // 65504
+                }
+                uint4* o = reinterpret_cast<uint4*>(static_cast<__half*>(j.aug) + (size_t)row * 16);
+                o[0] = make_uint4(h[0] | (uint32_t)h[1] << 16, h[2] | (uint32_t)h[3] << 16, h[4] | (uint32_t)h[5] << 16, h[6] | (uint32_t)h[7] << 16);
+                o[1] = make_uint4(0u, 0u, 0u, 0u);
+            } else if (j.aug) {
                 // |t|^2 = hi + mid + lo exactly, every piece a tf32 number; rows past the end score 1e30
                 const float g = row < n ? f : 1e30f;
                 const float hi = tf32_rna(g), r1 = __fsub_rn(g, hi), mid = tf32_rna(r1), lo = __fsub_rn(r1, mid);
+                float* aug = static_cast<float*>(j.aug);
                 *reinterpret_cast<float4*>(aug + (size_t)row * 8) = make_float4(hi, mid, lo, 0.f);
                 *reinterpret_cast<float4*>(aug + (size_t)row * 8 + 4) = make_float4(0.f, 0.f, 0.f, 0.f);
             }
@@ -127,9 +179,18 @@ round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad)
             if (row < n && __float_as_uint(f) > *reinterpret_cast<volatile unsigned*>(max_bits)) atomicMax(max_bits, __float_as_uint(f));
         }
     }
+    if (HALF && wide) *wide_flag = 1u;
 }
 
-static int launch_prep(erp_ctx* ctx, RoundJob a, RoundJob b, int dim, int dpad)
+template <bool HALF>
+static void launch_round(erp_ctx* ctx, int lpr, int grid, const RoundJob& a, const RoundJob& b, int dim, int dpad, unsigned* wide_flag)
+{
+    if (lpr == 8) round_kernel<8, HALF><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
+    else if (lpr == 16) round_kernel<16, HALF><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
+    else round_kernel<32, HALF><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
+}
+
+static int launch_prep(erp_ctx* ctx, RoundJob a, RoundJob b, int dim, int dpad, bool half, unsigned* wide_flag)
 {
     // 8 / 16 / 32 lanes per row for dpad = 32 / 64 / (96, 128)
     const int lpr = dpad <= 32 ? 8 : dpad <= 64 ? 16 : 32;
@@ -137,9 +198,8 @@ static int launch_prep(erp_ctx* ctx, RoundJob a, RoundJob b, int dim, int dpad)
     a.blocks = cdiv(a.n_pad, rows_per_block);
     b.blocks = b.x ? cdiv(b.n_pad, rows_per_block) : 0;
     const int grid = a.blocks + b.blocks;
-    if (lpr == 8) round_kernel<8><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad);
-    else if (lpr == 16) round_kernel<16><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad);
-    else round_kernel<32><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad);
+    if (half) launch_round<true>(ctx, lpr, grid, a, b, dim, dpad, wide_flag);
+    else launch_round<false>(ctx, lpr, grid, a, b, dim, dpad, wide_flag);
     ERP_LAUNCH(ctx, "round_kernel");
     return ERP_OK;
 }
@@ -162,7 +222,14 @@ struct Tc1Params {
 __device__ __forceinline__ int32_t thr_key(float f) { const int32_t k = __float_as_int(f); return k >= 0 ? k : k ^ 0x7fffffff; }
 __device__ __forceinline__ float key_thr(int32_t k) { return __int_as_float(k >= 0 ? k : k ^ 0x7fffffff); }
 
-template <int KCH>   // k chunks of 32 floats: dpad = 32 * KCH
+template <bool HALF>
+__device__ __forceinline__ void f_mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate)
+{
+    if (HALF) tc_mma_f16(d_tmem, a_desc, b_desc, F_IDESC_F16, accumulate);
+    else tc_mma_tf32(d_tmem, a_desc, b_desc, F_IDESC_TF32, accumulate);
+}
+
+template <int KCH, bool HALF>   // KCH k chunks of 128 bytes: dpad = KCH * f_kc(HALF) elements
 __global__ void __launch_bounds__(F_THREADS, 1)
 knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_t,
                 const __grid_constant__ CUtensorMap map_aug, const Tc1Params p)
@@ -208,7 +275,12 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    if (FOLD) {
+    if (FOLD && HALF) {
+        // query side of the norm step: the same 8 halves in both 16-byte halves of every row, which the swizzle cannot change
+        for (int i = threadIdx.x; i < F_AUG_Q / 2; i += F_THREADS)
+            reinterpret_cast<__half*>(aug_q)[i] = __float2half_rn(f16_norm_scale(i & 7));
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    } else if (FOLD) {
         // query side of the norm step: (1,1,1,0) in both 16-byte halves of every row, which the swizzle cannot change
         for (int i = threadIdx.x; i < F_AUG_Q / 4; i += F_THREADS) reinterpret_cast<float*>(aug_q)[i] = (i & 3) != 3 ? 1.0f : 0.0f;
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -234,13 +306,13 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                 for (int sub = 0; sub < F_SUB; sub++)
 #pragma unroll
                     for (int c = 0; c < KCH; c++)
-                        tma_load_2d(&map_q, qfull, q_smem + (sub * KCH + c) * F_QCH, c * F_KC, (qp * F_SUB + sub) * F_BM);
+                        tma_load_2d(&map_q, qfull, q_smem + (sub * KCH + c) * F_QCH, c * f_kc(HALF), (qp * F_SUB + sub) * F_BM);
                 for (int tt = t0; tt < t1; tt++) {
 #pragma unroll
                     for (int c = 0; c < KCH; c++) {
                         mbar_wait(&empty[slot], ph ^ 1);
                         mbar_expect_tx(&full[slot], F_TCH);
-                        tma_load_2d(&map_t, &full[slot], t_smem + slot * F_TCH, c * F_KC, tt * F_BN);
+                        tma_load_2d(&map_t, &full[slot], t_smem + slot * F_TCH, c * f_kc(HALF), tt * F_BN);
                         if (++slot == NS) { slot = 0; ph ^= 1; }
                     }
                 }
@@ -275,9 +347,10 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                             TCC_ADD(5, clock64() - f0);
                             tc_fence_after();
                             const uint32_t a = q_base + (sub * KCH + c) * F_QCH, b = t_base + sl * F_TCH;
+                            // one instruction per 32 bytes of the 128-byte row: K = 8 tf32 or K = 16 f16
 #pragma unroll
-                            for (int k = 0; k < F_KC / 8; k++)
-                                tc_mma_tf32(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), F_IDESC, (c | k) != 0);
+                            for (int k = 0; k < 4; k++)
+                                f_mma<HALF>(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), (c | k) != 0);
                             if (sub == F_SUB - 1) tc_commit(&empty[sl]);
                             if (++sl == NS) { sl = 0; pp ^= 1; }
                         }
@@ -285,7 +358,7 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                             const uint32_t nb = tt_n & 1;
                             if (sub == 0) mbar_wait(&nfull[nb], (tt_n >> 1) & 1);
                             tc_fence_after();
-                            tc_mma_tf32(d_tmem, aq_desc, smem_desc_sw32(smem_u32(aug_t + nb * F_AUG_T)), F_IDESC, 1);
+                            f_mma<HALF>(d_tmem, aq_desc, smem_desc_sw32(smem_u32(aug_t + nb * F_AUG_T)), 1);
                             if (sub == F_SUB - 1) tc_commit(&nempty[nb]);
                         }
                         tc_commit(&tfull[acc]);
@@ -474,14 +547,14 @@ __global__ void dbg_print_kernel()
     for (int i = 0; i < 8; i++) erp_clk[i] = 0;
 }
 #endif
-template <int KCH>
+template <int KCH, bool HALF>
 static int launch_tc1(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt, const CUtensorMap& ma, const Tc1Params& p, int grid)
 {
     constexpr int smem = f_smem(KCH);
     static_assert(smem <= TC_SMEM_LIMIT, "shared memory budget");
     static std::atomic<uint64_t> configured{0};
-    ERP_TRY(ensure_dynamic_smem(ctx, knn2_tc1_kernel<KCH>, smem, configured));
-    knn2_tc1_kernel<KCH><<<grid, F_THREADS, smem, ctx->stream>>>(mq, mt, ma, p);
+    ERP_TRY(ensure_dynamic_smem(ctx, knn2_tc1_kernel<KCH, HALF>, smem, configured));
+    knn2_tc1_kernel<KCH, HALF><<<grid, F_THREADS, smem, ctx->stream>>>(mq, mt, ma, p);
     ERP_LAUNCH(ctx, "knn2_tc1_kernel");
 #if ERP_TC_COUNTERS
     dbg_print_kernel<<<1, 1, 0, ctx->stream>>>();
@@ -490,11 +563,19 @@ static int launch_tc1(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt
     return ERP_OK;
 }
 
+// operands of the one-product engine: f16 unless ERP_B200_TC1_OPERANDS=tf32 (read once)
+bool tc1_f16_operands()
+{
+    static const bool f16 = [] { const char* e = getenv("ERP_B200_TC1_OPERANDS"); return !(e && strcmp(e, "tf32") == 0); }();
+    return f16;
+}
+
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2)
 {
     if (!knn2_tc_supported(nq, nt, dim)) { set_error("tcgen05 engine: unsupported shape nq=%d nt=%d dim=%d", nq, nt, dim); return ERP_E_DIM; }
-    const int kch = (dim + F_KC - 1) / F_KC, dpad = kch * F_KC;
+    const bool half = tc1_f16_operands();
+    const int kc = f_kc(half), kch = (dim + kc - 1) / kc, dpad = kch * kc, esize = half ? 2 : 4;
     const int n_qpairs = cdiv(nq, F_BM * f_sub(kch)), n_ttiles = cdiv(nt, F_BN);
     // stream-K plan: equal contiguous unit ranges, a query pair cut in at most F_MAX_SEG segments
     long total = (long)n_qpairs * n_ttiles;
@@ -508,9 +589,9 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     const int n_lists = n_seg * F_EPI_GROUPS;
 
     int st = ERP_OK;
-    float* qs = ctx->scratch<float>(S_TC_Q, (size_t)nq * dpad, &st);
-    float* ts = ctx->scratch<float>(S_TC_T, (size_t)nt * dpad, &st);
-    float* tn = ctx->scratch<float>(S_TC_TN, (size_t)n_ttiles * F_BN * 9, &st);      // norms, then the 8-float norm operand rows
+    uint8_t* qs = ctx->scratch<uint8_t>(S_TC_Q, (size_t)nq * dpad * esize, &st);
+    uint8_t* ts = ctx->scratch<uint8_t>(S_TC_T, (size_t)nt * dpad * esize, &st);
+    float* tn = ctx->scratch<float>(S_TC_TN, (size_t)n_ttiles * F_BN * 9, &st);      // norms, then the 32-byte norm operand rows
     int32_t* cand = ctx->scratch<int32_t>(S_TC_CAND, (size_t)nq * n_lists * (F_TOPK * 2 + 1), &st);
     float* qn = ctx->scratch<float>(S_TC_QN, (size_t)nq + 8, &st);
     int32_t* list = ctx->scratch<int32_t>(S_TC_LIST, (size_t)nq + 8, &st);
@@ -531,13 +612,13 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     RoundJob jq = {d_q, nq, -2.0f, qs, qn, nq, reinterpret_cast<unsigned*>(misc + 3), nullptr, 0};
     RoundJob jt = {ctx->tc_chunk == 0 ? d_t : nullptr, nt, 1.0f, ts, tn, n_ttiles * F_BN, reinterpret_cast<unsigned*>(misc + 1),
                    f_fold(kch) ? aug : nullptr, 0};
-    ERP_TRY(launch_prep(ctx, jq, jt, dim, dpad));
+    ERP_TRY(launch_prep(ctx, jq, jt, dim, dpad, half, reinterpret_cast<unsigned*>(misc + 5)));
 
     CUtensorMap mq, mt;
-    ERP_TRY(make_map(&mq, qs, nq, dpad, F_BM));
-    ERP_TRY(make_map(&mt, ts, nt, dpad, F_BN));
+    ERP_TRY(make_map(&mq, qs, nq, dpad, F_BM, false, half));
+    ERP_TRY(make_map(&mt, ts, nt, dpad, F_BN, false, half));
     CUtensorMap ma = mt;
-    if (f_fold(kch)) ERP_TRY(make_map(&ma, aug, n_ttiles * F_BN, 8, F_BN, true));
+    if (f_fold(kch)) ERP_TRY(make_map(&ma, aug, n_ttiles * F_BN, 32 / esize, F_BN, true, half));
     Tc1Params p;
     p.nq = nq; p.nt = nt; p.n_qpairs = n_qpairs; p.n_ttiles = n_ttiles; p.units_per_cta = (int)L; p.n_seg = n_seg;
     p.tn = tn; p.cand_idx = cand; p.cand_s = cand_s; p.cand_thr = cand_thr; p.qn = qn;
@@ -545,15 +626,21 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     p.row_thr = row_thr;
 
     if (ctx->tc_chunk == 0) ERP_CUDA(record_timing(ctx, ctx->ev_k0));
-    switch (kch) {
-    case 1: ERP_TRY(launch_tc1<1>(ctx, mq, mt, ma, p, grid)); break;
-    case 2: ERP_TRY(launch_tc1<2>(ctx, mq, mt, ma, p, grid)); break;
-    case 3: ERP_TRY(launch_tc1<3>(ctx, mq, mt, ma, p, grid)); break;
-    default: ERP_TRY(launch_tc1<4>(ctx, mq, mt, ma, p, grid)); break;
+    if (half) {
+        if (kch == 1) ERP_TRY((launch_tc1<1, true>(ctx, mq, mt, ma, p, grid)));
+        else ERP_TRY((launch_tc1<2, true>(ctx, mq, mt, ma, p, grid)));
+    } else {
+        switch (kch) {
+        case 1: ERP_TRY((launch_tc1<1, false>(ctx, mq, mt, ma, p, grid))); break;
+        case 2: ERP_TRY((launch_tc1<2, false>(ctx, mq, mt, ma, p, grid))); break;
+        case 3: ERP_TRY((launch_tc1<3, false>(ctx, mq, mt, ma, p, grid))); break;
+        default: ERP_TRY((launch_tc1<4, false>(ctx, mq, mt, ma, p, grid))); break;
+        }
     }
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
 
-    ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, F_TOPK, F_KAPPA, cand, cand_s, cand_thr, reinterpret_cast<unsigned*>(misc),
+    ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, F_TOPK, F_KAPPA, half ? F_F16_ABS : -1.0, cand, cand_s, cand_thr,
+                          reinterpret_cast<unsigned*>(misc),
                           d_idx2, d_dist2, d_d2, list));
     ERP_TRY(knn2_exact_rescan(ctx, d_q, nq, d_t, nt, dim, list, misc, nq, d_idx2, d_dist2, d_d2));
     ERP_TRY(tc_misc_end(ctx, misc));

@@ -75,6 +75,17 @@ __device__ __forceinline__ void tc_mma_tf32(uint32_t d_tmem, uint64_t a_desc, ui
         ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem]^T, 128 x 256 x 16, f16 inputs, fp32 accumulate: the same 32 bytes of every operand row as
+// one tf32 instruction, at twice the rate
+__device__ __forceinline__ void tc_mma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 // the same with A read from tensor memory (lane = row, one tf32 per column): only B is fetched from shared memory
 __device__ __forceinline__ void tc_mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
 {
@@ -185,19 +196,20 @@ inline EncodeTiledFn encode_fn()
     return fn;
 }
 
-// rows x row_floats fp32, row major; box = 32 floats (one 128-byte swizzle row) x box_rows, zero fill out of bounds;
-// narrow = true: box = 8 floats (one 32-byte swizzle row) x box_rows for the single-k-step operands
-inline int make_map(CUtensorMap* map, const float* base, int rows, int row_floats, int box_rows, bool narrow = false)
+// rows x row_elems, row major, fp32 (or f16 with half = true); box = one 128-byte swizzle row (32 floats or 64 halves) x box_rows,
+// zero fill out of bounds; narrow = true: box = one 32-byte swizzle row x box_rows for the single-k-step operands
+inline int make_map(CUtensorMap* map, const void* base, int rows, int row_elems, int box_rows, bool narrow = false, bool half = false)
 {
     EncodeTiledFn fn = encode_fn();
     if (!fn) { set_error("cuTensorMapEncodeTiled is not available from this driver"); return ERP_E_CUDA; }
-    cuuint64_t dims[2] = {(cuuint64_t)row_floats, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)row_floats * sizeof(float)};
-    cuuint32_t box[2] = {narrow ? 8u : 32u, (cuuint32_t)box_rows};
+    const cuuint32_t esize = half ? 2 : 4;
+    cuuint64_t dims[2] = {(cuuint64_t)row_elems, (cuuint64_t)rows};
+    cuuint64_t strides[1] = {(cuuint64_t)row_elems * esize};
+    cuuint32_t box[2] = {(narrow ? 32u : 128u) / esize, (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, narrow ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = fn(map, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides,
+                    box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, narrow ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_128B,
+                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d", (int)r); return ERP_E_CUDA; }
     return ERP_OK;
 }

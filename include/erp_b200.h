@@ -64,8 +64,16 @@ typedef enum {
     ERP_ENGINE_AUTO = 0,       /* the fastest exact engine for the shape: TCGEN05_1X for large problems, else SIMT */
     ERP_ENGINE_EXACT_SIMT = 1, /* fp64 direct-form brute force (also the rescan path)            */
     ERP_ENGINE_TCGEN05 = 2,    /* 3xTF32 GEMM-form tiles + fused top-4, exact fp64 refine + certificate  */
-    ERP_ENGINE_TCGEN05_1X = 3  /* one TF32 product, top-8, same certificate: a third of the tensor work */
+    ERP_ENGINE_TCGEN05_1X = 3  /* one product of 11-bit operands (f16, or tf32 with ERP_B200_TC1_OPERANDS=tf32), top-8, same
+                                  certificate: 5 tensor instructions per tile at D = 64 where 3xTF32 issues 24 */
 } erp_engine;
+
+/* operand format of the tensor products of a distance search (erp_ctx_last_knn_operands) */
+typedef enum {
+    ERP_OPERANDS_NONE = 0,     /* no tensor product: ERP_ENGINE_EXACT_SIMT */
+    ERP_OPERANDS_TF32 = 1,
+    ERP_OPERANDS_F16 = 2
+} erp_operands;
 
 /* pose record per hypothesis: XYZ-euler of R1, of R2 (rad), t, validity flags (1.0/0.0), 1 pad */
 #define ERP_POSE_FLOATS 12
@@ -95,6 +103,10 @@ uint64_t erp_ctx_launch_count(erp_ctx* ctx);
 /* diagnostics of the last erp_knn2* call: [0] engine used, [1] queries re-scanned exactly,
  * [2] train chunks, [3] work items, [4] reserved */
 int  erp_ctx_last_knn_stats(erp_ctx* ctx, int64_t out[5]);
+/* operands of the last erp_knn2* call: [0] erp_operands, and for f16 operands [1] 1 if the range guard fired (a finite input
+ * f16 cannot hold: every query of the call was re-scanned exactly), [2] queries re-scanned because f16 could not represent
+ * them closely enough (the guard, or norms so small that subnormal rounding is outside the certificate); synchronises */
+int  erp_ctx_last_knn_operands(erp_ctx* ctx, int64_t out[3]);
 /* device time of the dominant distance kernel of the last erp_knn2* call, from CUDA events the
  * library records on its own stream around that launch (synchronises the stream) */
 int  erp_ctx_last_knn_kernel_ms(erp_ctx* ctx, float* ms);
