@@ -21,7 +21,7 @@ POSE_FLOATS = 12
 
 METRIC_ALGEBRAIC, METRIC_SAMPSON, METRIC_ANGULAR = 0, 1, 2
 ENGINE_AUTO, ENGINE_EXACT_SIMT, ENGINE_TCGEN05, ENGINE_TCGEN05_1X = 0, 1, 2, 3
-OPERANDS_NONE, OPERANDS_TF32, OPERANDS_F16 = 0, 1, 2
+OPERANDS_NONE, OPERANDS_TF32, OPERANDS_F16, OPERANDS_I8 = 0, 1, 2, 3
 
 OK = 0
 E_ARG, E_DIM, E_TOO_FEW_TRAIN, E_TOO_FEW_POINTS, E_NO_CANDIDATE, E_LIMIT = 1, 2, 3, 4, 5, 6
@@ -72,6 +72,19 @@ _SIGNATURES = {
     "erp_nn1_reverse_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "erp_match_filter_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "erp_knn2_match_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_void_p, C.c_void_p]),
+    "erp_knn2_match_bin": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_size_t, C.c_int,
+                                     C.c_float, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
+    "erp_knn2_raw_bin": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_size_t, C.c_int,
+                                   C.c_void_p, C.c_void_p]),
+    "erp_knn2_bin_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "erp_knn2_match_bin_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_void_p,
+                                         C.c_void_p]),
+    "erp_pair_pose_bin": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_size_t, C.c_int, C.c_float,
+                                    C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_uint64, C.c_int, C.c_int, C.c_int,
+                                    C.c_float, C.c_void_p, C.POINTER(C.c_int), C.POINTER(RansacResult), C.c_void_p]),
+    "erp_pair_pose_bin_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int,
+                                        C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_uint64, C.c_int, C.c_int, C.c_int,
+                                        C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "erp_bearings_from_pixels": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "erp_bearings_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "erp_pack_float4_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
@@ -185,6 +198,16 @@ def _f32(a):
 
 def _f64(a):
     return np.ascontiguousarray(a, dtype=np.float64)
+
+
+def _u8_rows(a):
+    """(n, nbytes) uint8 rows whose bytes within a row are contiguous (strided row views stay views): (array, row stride)."""
+    a = np.asarray(a)
+    if a.dtype != np.uint8 or a.ndim != 2:
+        raise ValueError("binary descriptors are (n, nbytes) uint8 arrays")
+    if a.strides[1] != 1 or a.strides[0] < a.shape[1]:
+        a = np.ascontiguousarray(a)
+    return a, (a.strides[0] if a.shape[0] > 1 else a.shape[1])
 
 
 def libstdcxx_sample_table(m: int, H: int = 80, S: int | None = None, seed: int = 1) -> np.ndarray:
@@ -323,6 +346,53 @@ class Context:
     def knn2_match_dev(self, d_q, nq, d_t, nt, dim, ratio, cross_check, d_out, d_n_out):
         _check(lib().erp_knn2_match_dev(self._h, _ptr(d_q), nq, _ptr(d_t), nt, dim, ratio, int(cross_check),
                                         _ptr(d_out), _ptr(d_n_out)))
+
+    # ---- binary descriptors (Hamming distance; include/erp_b200.h "binary descriptors")
+    def knn2_match_bin(self, q, t, ratio: float = 0.3, cross_check: bool = False) -> np.ndarray:
+        """match_two_image with cv::BFMatcher(NORM_HAMMING): (n, nbytes) uint8 rows -> DMatch records."""
+        (q, qs), (t, ts) = _u8_rows(q), _u8_rows(t)
+        out = np.empty(max(q.shape[0], 1), DMATCH)
+        n = C.c_int(0)
+        _check(lib().erp_knn2_match_bin(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1],
+                                        ratio, int(cross_check), _ptr(out), C.byref(n)))
+        return out[: n.value]
+
+    def knn2_raw_bin(self, q, t):
+        (q, qs), (t, ts) = _u8_rows(q), _u8_rows(t)
+        idx = np.empty((q.shape[0], 2), np.int32)
+        dist = np.empty((q.shape[0], 2), np.float32)
+        _check(lib().erp_knn2_raw_bin(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], _ptr(idx), _ptr(dist)))
+        return idx, dist
+
+    def knn2_bin_dev(self, d_q, nq, d_t, nt, nbytes, d_idx2, d_dist2, d_d2=None):
+        _check(lib().erp_knn2_bin_dev(self._h, _ptr(d_q), nq, _ptr(d_t), nt, nbytes, _ptr(d_idx2), _ptr(d_dist2), _ptr(d_d2)))
+
+    def knn2_match_bin_dev(self, d_q, nq, d_t, nt, nbytes, ratio, cross_check, d_out, d_n_out):
+        _check(lib().erp_knn2_match_bin_dev(self._h, _ptr(d_q), nq, _ptr(d_t), nt, nbytes, ratio, int(cross_check),
+                                            _ptr(d_out), _ptr(d_n_out)))
+
+    def pair_pose_bin(self, q, t, left_xy, right_xy, W, H_img, ratio=0.8, cross_check=False, seed=1, H=10000, S=8,
+                      metric=METRIC_ALGEBRAIC, tau=0.002):
+        """erp_pair_pose_bin: binary descriptors + all keypoints of both views -> (match records, RANSAC result with mask)."""
+        (q, qs), (t, ts) = _u8_rows(q), _u8_rows(t)
+        left_xy, right_xy = _f32(left_xy), _f32(right_xy)
+        out = np.empty(q.shape[0], DMATCH)
+        n = C.c_int(0)
+        res = RansacResult()
+        mask = np.empty(q.shape[0], np.uint8)
+        _check(lib().erp_pair_pose_bin(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], ratio, int(cross_check),
+                                       _ptr(left_xy), _ptr(right_xy), left_xy.strides[0], W, H_img, seed, H, S, metric, tau,
+                                       _ptr(out), C.byref(n), C.byref(res), _ptr(mask)))
+        r = self._result(res)
+        r["mask"] = mask[:n.value]
+        return out[:n.value], r
+
+    def pair_pose_bin_dev(self, d_q, nq, d_t, nt, nbytes, ratio, cross_check, d_left_xy, d_right_xy, kp_stride, W, H_img, seed, H,
+                          S, metric, tau, d_matches, d_n, d_mask, d_result):
+        """erp_pair_pose_bin_dev: enqueue only."""
+        _check(lib().erp_pair_pose_bin_dev(self._h, _ptr(d_q), nq, _ptr(d_t), nt, nbytes, ratio, int(cross_check), _ptr(d_left_xy),
+                                           _ptr(d_right_xy), kp_stride, W, H_img, seed, H, S, metric, tau, _ptr(d_matches), _ptr(d_n),
+                                           _ptr(d_mask), _ptr(d_result)))
 
     # ---- geometry
     def bearings(self, xy, W: int, H: int) -> np.ndarray:

@@ -15,7 +15,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(OUT_DIR, "liberp_b200.so")
-SOURCES = ["api.cu", "knn_exact.cu", "knn_tc.cu", "knn_tc1.cu", "geometry.cu", "score.cu", "score_tc.cu", "erp_image.cu", "dist.cu"]
+SOURCES = ["api.cu", "knn_exact.cu", "knn_tc.cu", "knn_tc1.cu", "knn_bin.cu", "geometry.cu", "score.cu", "score_tc.cu", "erp_image.cu", "dist.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

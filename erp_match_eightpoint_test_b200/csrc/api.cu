@@ -393,7 +393,8 @@ ERP_API int erp_ctx_last_knn_operands(erp_ctx* ctx, int64_t out[3])
     ERP_ARG(ctx && out, ERP_E_ARG, "erp_ctx_last_knn_operands: bad argument");
     const int64_t engine = ctx->knn_stats[0];
     out[0] = engine == ERP_ENGINE_TCGEN05 ? ERP_OPERANDS_TF32
-           : engine == ERP_ENGINE_TCGEN05_1X ? (tc1_f16_operands() ? ERP_OPERANDS_F16 : ERP_OPERANDS_TF32) : ERP_OPERANDS_NONE;
+           : engine == ERP_ENGINE_TCGEN05_1X ? (ctx->knn_bin ? ERP_OPERANDS_I8 : tc1_f16_operands() ? ERP_OPERANDS_F16 : ERP_OPERANDS_TF32)
+           : ERP_OPERANDS_NONE;
     out[1] = out[2] = 0;
     if (out[0] == ERP_OPERANDS_F16 && ctx->tc_misc_dev) {
         DeviceGuard g(ctx->device);
@@ -435,6 +436,7 @@ ERP_API int erp_knn2_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_
         return knn2_tc(ctx, d_q, nq, d_t, nt, dim, d_idx2, d_dist2, d_d2);
     ctx->knn_stats[0] = ERP_ENGINE_EXACT_SIMT; ctx->knn_stats[1] = 0; ctx->knn_stats[2] = 1; ctx->knn_stats[3] = cdiv(nq, 64);
     ctx->knn_stats[4] = 0;
+    ctx->knn_bin = false;
     ERP_CUDA(record_timing(ctx, ctx->ev_k0));
     ERP_TRY(knn2_exact(ctx, d_q, nq, d_t, nt, dim, nullptr, 0, 0, d_idx2, d_dist2, d_d2));
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
@@ -541,16 +543,11 @@ static int chunk_bounds(int nq, int nt, bool pageable, int (&bounds)[9])
     bounds[++n] = nq;
     return n;
 }
-static int knn2_host(erp_ctx* ctx, const float* q, int nq, size_t qs, const float* t, int nt, size_t ts, int dim,
-                     int32_t* d_idx2, float* d_dist2)
+// search(d_q_chunk, rows, idx2, dist2): the 2-NN of one uploaded query chunk against the uploaded train rows
+using ChunkSearch = std::function<int(const void*, int, int32_t*, float*)>;
+static int knn2_host_rows(erp_ctx* ctx, const void* q, int nq, size_t qs, const void* t, int nt, size_t ts, size_t row,
+                          uint8_t* dq, uint8_t* dt, const ChunkSearch& search, int32_t* d_idx2, float* d_dist2)
 {
-    size_t row = (size_t)dim * sizeof(float);
-    ERP_ARG((nq == 0 || q) && (nt == 0 || t), ERP_E_ARG, "null descriptor pointer");
-    ERP_ARG(qs >= row && ts >= row, ERP_E_ARG, "row stride smaller than a descriptor row (%zu < %zu)", qs < ts ? qs : ts, row);
-    int st = ERP_OK;
-    float* dq = ctx->scratch<float>(S_Q, (size_t)nq * dim + 4, &st);
-    float* dt = ctx->scratch<float>(S_T, (size_t)nt * dim + 4, &st);
-    ERP_TRY(st);
     int bounds[9];
     const int chunks = chunk_bounds(nq, nt, is_pageable(q), bounds);
     // fork: the copy stream starts after whatever the context stream still has queued
@@ -581,7 +578,7 @@ static int knn2_host(erp_ctx* ctx, const float* q, int nq, size_t qs, const floa
     for (int c = 0; c < chunks && rc == ERP_OK; c++) {
         const int r0 = bounds[c], n = bounds[c + 1] - r0;
         sw.to_copy();
-        rc = upload_rows(ctx, dq + (size_t)r0 * dim, reinterpret_cast<const char*>(q) + (size_t)r0 * qs, n, row, qs);
+        rc = upload_rows(ctx, dq + (size_t)r0 * row, reinterpret_cast<const char*>(q) + (size_t)r0 * qs, n, row, qs);
         if (rc == ERP_OK && cudaEventRecord(ctx->ev_copy[c], ctx->copy_stream) != cudaSuccess) rc = ERP_E_CUDA;
         mark(ctx->copy_stream);
         sw.to_main();
@@ -590,7 +587,7 @@ static int knn2_host(erp_ctx* ctx, const float* q, int nq, size_t qs, const floa
         mark(ctx->stream);
         ctx->tc_chunk = c;
         const double t_enq = now_s();
-        rc = erp_knn2_dev(ctx, dq + (size_t)r0 * dim, n, dt, nt, dim, d_idx2 + 2 * (size_t)r0, d_dist2 + 2 * (size_t)r0, nullptr);
+        rc = search(dq + (size_t)r0 * row, n, d_idx2 + 2 * (size_t)r0, d_dist2 + 2 * (size_t)r0);
         mark(ctx->stream);
         if (trace) fprintf(stderr, "[stage] chunk %d: search of %d rows enqueued in %.3f ms (host)\n", c, n, 1e3 * (now_s() - t_enq));
     }
@@ -604,6 +601,21 @@ static int knn2_host(erp_ctx* ctx, const float* q, int nq, size_t qs, const floa
         for (int i = 0; i < n_tr; i++) cudaEventDestroy(tr[i]);
     }
     return rc;
+}
+static int knn2_host(erp_ctx* ctx, const float* q, int nq, size_t qs, const float* t, int nt, size_t ts, int dim,
+                     int32_t* d_idx2, float* d_dist2)
+{
+    size_t row = (size_t)dim * sizeof(float);
+    ERP_ARG((nq == 0 || q) && (nt == 0 || t), ERP_E_ARG, "null descriptor pointer");
+    ERP_ARG(qs >= row && ts >= row, ERP_E_ARG, "row stride smaller than a descriptor row (%zu < %zu)", qs < ts ? qs : ts, row);
+    int st = ERP_OK;
+    float* dq = ctx->scratch<float>(S_Q, (size_t)nq * dim + 4, &st);
+    float* dt = ctx->scratch<float>(S_T, (size_t)nt * dim + 4, &st);
+    ERP_TRY(st);
+    return knn2_host_rows(ctx, q, nq, qs, t, nt, ts, row, reinterpret_cast<uint8_t*>(dq), reinterpret_cast<uint8_t*>(dt),
+                          [&](const void* cq, int n, int32_t* i2, float* d2) {
+                              return erp_knn2_dev(ctx, static_cast<const float*>(cq), n, dt, nt, dim, i2, d2, nullptr);
+                          }, d_idx2, d_dist2);
 }
 
 ERP_API int erp_knn2_match(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes,
@@ -683,6 +695,131 @@ ERP_API int erp_knn2_near_ties(erp_ctx* ctx, const float* q, int nq, size_t q_st
     ERP_CUDA(cudaMemcpyAsync(&n, d_third + nq, sizeof n, cudaMemcpyDeviceToHost, ctx->stream));
     ERP_CUDA(cudaStreamSynchronize(ctx->stream));
     *n_flagged = n;
+    return ERP_OK;
+}
+
+// ======================================================================================
+// binary descriptors (knn_bin.cu): feature_matcher::match_two_image with NORM_HAMMING
+// ======================================================================================
+static int check_bin_args(const char* who, erp_ctx* ctx, int nq, int nt, int nbytes)
+{
+    ERP_ARG(ctx, ERP_E_ARG, "%s: null context", who);
+    ERP_ARG(nq >= 0 && nt >= 0, ERP_E_ARG, "%s: negative size", who);
+    ERP_ARG(nbytes >= 1 && nbytes <= 64, ERP_E_DIM, "%s: binary descriptor size %d must be in [1,64] bytes", who, nbytes);
+    ERP_ARG(nq == 0 || nt >= 2, ERP_E_TOO_FEW_TRAIN, "%s: k=2 needs at least 2 train descriptors, got %d", who, nt);
+    return ERP_OK;
+}
+
+// both tensor engine settings select the kind::i8 engine; AUTO takes it where it is faster than SIMT
+static bool bin_uses_tc(erp_ctx* ctx, int nq, int nt)
+{
+    return ctx->engine == ERP_ENGINE_TCGEN05 || ctx->engine == ERP_ENGINE_TCGEN05_1X ||
+           (ctx->engine == ERP_ENGINE_AUTO && knn2_bin_preferred(nq, nt));
+}
+
+ERP_API int erp_knn2_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes,
+                             int32_t* d_idx2, float* d_dist2, double* d_d2)
+{
+    ERP_TRY(check_bin_args("erp_knn2_bin_dev", ctx, nq, nt, nbytes));
+    if (nq == 0) return ERP_OK;
+    ERP_ARG(d_q && d_t, ERP_E_ARG, "erp_knn2_bin_dev: null descriptors");
+    DeviceGuard g(ctx->device);
+    return knn2_bin(ctx, d_q, nq, d_t, nt, nbytes, bin_uses_tc(ctx, nq, nt), d_idx2, d_dist2, d_d2);
+}
+
+// cross-check: nearest query of every train row (roles swapped, lowest query index on ties), compacted to the first neighbour
+static int bin_reverse(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, int32_t* d_best_q)
+{
+    int st = ERP_OK;
+    int32_t* idx2 = ctx->scratch<int32_t>(S_RS_IDX, (size_t)nt * 2, &st);
+    ERP_TRY(st);
+    ERP_TRY(knn2_bin(ctx, d_t, nt, d_q, nq, nbytes, bin_uses_tc(ctx, nt, nq), idx2, nullptr, nullptr));
+    ERP_CUDA(cudaMemcpy2DAsync(d_best_q, sizeof(int32_t), idx2, 2 * sizeof(int32_t), sizeof(int32_t), nt,
+                               cudaMemcpyDeviceToDevice, ctx->stream));
+    return ERP_OK;
+}
+
+ERP_API int erp_knn2_match_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes,
+                                   float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
+{
+    ERP_TRY(check_bin_args("erp_knn2_match_bin_dev", ctx, nq, nt, nbytes));
+    ERP_ARG(d_n_out, ERP_E_ARG, "erp_knn2_match_bin_dev: d_n_out is null");
+    DeviceGuard g(ctx->device);
+    int st = ERP_OK;
+    int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
+    float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
+    ERP_TRY(st);
+    ERP_TRY(erp_knn2_bin_dev(ctx, d_q, nq, d_t, nt, nbytes, idx2, dist2, nullptr));
+    int32_t* rev = nullptr;
+    if (cross_check && nq > 0) {
+        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
+        ERP_TRY(st);
+        ERP_TRY(bin_reverse(ctx, d_q, nq, d_t, nt, nbytes, rev));
+    }
+    return erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n_out);
+}
+
+// host rows -> S_Q / S_T (dense) and the 2-NN, chunked like the float rows.  One engine for the whole call: the i8
+// operand of the train rows is prepared by the first query chunk only.
+static int knn2_bin_host(erp_ctx* ctx, const uint8_t* q, int nq, size_t qs, const uint8_t* t, int nt, size_t ts, int nbytes,
+                         int32_t* d_idx2, float* d_dist2)
+{
+    ERP_ARG((nq == 0 || q) && (nt == 0 || t), ERP_E_ARG, "null descriptor pointer");
+    ERP_ARG(qs >= (size_t)nbytes && ts >= (size_t)nbytes, ERP_E_ARG, "row stride smaller than a descriptor row (%zu < %d)",
+            qs < ts ? qs : ts, nbytes);
+    int st = ERP_OK;
+    uint8_t* dq = ctx->scratch<uint8_t>(S_Q, (size_t)nq * nbytes + 16, &st);
+    uint8_t* dt = ctx->scratch<uint8_t>(S_T, (size_t)nt * nbytes + 16, &st);
+    ERP_TRY(st);
+    const bool tc = bin_uses_tc(ctx, nq, nt);
+    return knn2_host_rows(ctx, q, nq, qs, t, nt, ts, (size_t)nbytes, dq, dt,
+                          [&](const void* cq, int n, int32_t* i2, float* d2) {
+                              return knn2_bin(ctx, static_cast<const uint8_t*>(cq), n, dt, nt, nbytes, tc, i2, d2, nullptr);
+                          }, d_idx2, d_dist2);
+}
+
+ERP_API int erp_knn2_match_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes,
+                               const uint8_t* t, int nt, size_t t_stride_bytes, int nbytes,
+                               float ratio, int cross_check, erp_dmatch* out, int* n_out)
+{
+    ERP_TRY(check_bin_args("erp_knn2_match_bin", ctx, nq, nt, nbytes));
+    ERP_ARG(n_out, ERP_E_ARG, "erp_knn2_match_bin: n_out is null");
+    *n_out = 0;
+    if (nq == 0) return ERP_OK;
+    ERP_ARG(out, ERP_E_ARG, "erp_knn2_match_bin: out is null");
+    DeviceGuard g(ctx->device);
+    int st = ERP_OK;
+    erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
+    int32_t* d_n = ctx->scratch<int32_t>(S_NOUT, 4, &st);
+    int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
+    float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
+    ERP_TRY(st);
+    ERP_TRY(knn2_bin_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, nbytes, idx2, dist2));
+    int32_t* rev = nullptr;
+    if (cross_check) {
+        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
+        ERP_TRY(st);
+        ERP_TRY(bin_reverse(ctx, ctx->dev[S_Q].as<uint8_t>(), nq, ctx->dev[S_T].as<uint8_t>(), nt, nbytes, rev));
+    }
+    ERP_TRY(erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n));
+    return download_matches(ctx, d_out, d_n, (size_t)nq, out, n_out);
+}
+
+ERP_API int erp_knn2_raw_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes,
+                             const uint8_t* t, int nt, size_t t_stride_bytes, int nbytes,
+                             int32_t* idx2, float* dist2)
+{
+    ERP_TRY(check_bin_args("erp_knn2_raw_bin", ctx, nq, nt, nbytes));
+    if (nq == 0) return ERP_OK;
+    DeviceGuard g(ctx->device);
+    int st = ERP_OK;
+    int32_t* d_idx = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
+    float* d_dist = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
+    ERP_TRY(st);
+    ERP_TRY(knn2_bin_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, nbytes, d_idx, d_dist));
+    if (idx2) ERP_CUDA(cudaMemcpyAsync(idx2, d_idx, sizeof(int32_t) * 2 * (size_t)nq, cudaMemcpyDeviceToHost, ctx->stream));
+    if (dist2) ERP_CUDA(cudaMemcpyAsync(dist2, d_dist, sizeof(float) * 2 * (size_t)nq, cudaMemcpyDeviceToHost, ctx->stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
     return ERP_OK;
 }
 
@@ -867,6 +1004,7 @@ struct GraphCache {
     cudaGraphExec_t exec = nullptr;
     uint64_t launches = 0;
     int64_t knn_stats[5] = {0, 0, 0, 0, 0};
+    bool knn_bin = false;
     int32_t *sc_misc_dev = nullptr, *tc_misc_dev = nullptr;
     int n_ev_score = 0;
     bool disabled = false;
@@ -894,6 +1032,7 @@ int graph_run(erp_ctx* ctx, const void* key, size_t key_bytes, const std::functi
         ERP_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
         ctx->launches += g.launches;
         memcpy(ctx->knn_stats, g.knn_stats, sizeof g.knn_stats);
+        ctx->knn_bin = g.knn_bin;
         ctx->sc_misc_dev = g.sc_misc_dev; ctx->tc_misc_dev = g.tc_misc_dev; ctx->n_ev_score = g.n_ev_score;
         return ERP_OK;
     }
@@ -927,6 +1066,7 @@ int graph_run(erp_ctx* ctx, const void* key, size_t key_bytes, const std::functi
         ctx->launches = l0;
         g.key = k; g.key_gen = ctx->scratch_gen;
         memcpy(g.knn_stats, ctx->knn_stats, sizeof g.knn_stats);
+        g.knn_bin = ctx->knn_bin;
         g.sc_misc_dev = ctx->sc_misc_dev; g.tc_misc_dev = ctx->tc_misc_dev; g.n_ev_score = ctx->n_ev_score;
         ERP_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
         ctx->launches += g.launches;
@@ -1070,6 +1210,28 @@ ERP_API int erp_pair_pose_dev(erp_ctx* ctx, const float* d_q, int nq, const floa
     });
 }
 
+// everything is enqueued: the host waits for the MATCH stage only (the pose chain keeps running), learns the match
+// count and brings the records back on the copy stream while the hypotheses are being scored
+static int pair_pose_download(erp_ctx* ctx, const char* who, const erp_dmatch* d_out, const int32_t* d_n, const PoseBuffers& b, int S,
+                              erp_dmatch* matches_out, int* n_matches, erp_ransac_result* result, uint8_t* mask)
+{
+    int32_t n = 0;
+    ERP_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_stage[1], 0));
+    ERP_CUDA(cudaMemcpyAsync(&n, d_n, sizeof n, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
+    *n_matches = n;
+    if (n > 0) ERP_CUDA(cudaMemcpyAsync(matches_out, d_out, sizeof(erp_dmatch) * (size_t)n, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    ERP_CUDA(cudaMemcpyAsync(result, b.res, sizeof *result, cudaMemcpyDeviceToHost, ctx->stream));
+    if (mask && n > 0) ERP_CUDA(cudaMemcpyAsync(mask, b.mask, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
+    if (n < S) {
+        set_error("%s: %d matches for sample size %d", who, n, S);
+        return ERP_E_TOO_FEW_POINTS;
+    }
+    return ERP_OK;
+}
+
 ERP_API int erp_pair_pose(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes, const float* t, int nt, size_t t_stride_bytes,
                           int dim, float ratio, int cross_check,
                           const void* left_xy, const void* right_xy, size_t kp_stride_bytes, int width, int height,
@@ -1129,23 +1291,62 @@ ERP_API int erp_pair_pose(erp_ctx* ctx, const float* q, int nq, size_t q_stride_
         ERP_TRY(erp_pair_pose_dev(ctx, dq, nq, dt, nt, dim, ratio, cross_check, d_xy, d_xy + (size_t)nq * 2, 8, width, height,
                                   seed, H, S, metric, tau, d_out, d_n, b.mask, b.res));
     }
-    // everything is enqueued: the host waits for the MATCH stage only (the pose chain keeps running), learns the match
-    // count and brings the records back on the copy stream while the hypotheses are being scored
-    int32_t n = 0;
-    ERP_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_stage[1], 0));
-    ERP_CUDA(cudaMemcpyAsync(&n, d_n, sizeof n, cudaMemcpyDeviceToHost, ctx->copy_stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
-    *n_matches = n;
-    if (n > 0) ERP_CUDA(cudaMemcpyAsync(matches_out, d_out, sizeof(erp_dmatch) * (size_t)n, cudaMemcpyDeviceToHost, ctx->copy_stream));
-    ERP_CUDA(cudaMemcpyAsync(result, b.res, sizeof *result, cudaMemcpyDeviceToHost, ctx->stream));
-    if (mask && n > 0) ERP_CUDA(cudaMemcpyAsync(mask, b.mask, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
-    if (n < S) {
-        set_error("erp_pair_pose: %d matches for sample size %d", n, S);
-        return ERP_E_TOO_FEW_POINTS;
-    }
-    return ERP_OK;
+    return pair_pose_download(ctx, "erp_pair_pose", d_out, d_n, b, S, matches_out, n_matches, result, mask);
+}
+
+ERP_API int erp_pair_pose_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, float ratio,
+                                  int cross_check, const void* d_left_xy, const void* d_right_xy, size_t kp_stride_bytes, int width,
+                                  int height, uint64_t seed, int H, int S, int metric, float tau,
+                                  erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result)
+{
+    ERP_TRY(check_bin_args("erp_pair_pose_bin_dev", ctx, nq, nt, nbytes));
+    ERP_TRY(check_ransac_args("erp_pair_pose_bin_dev", ctx, H, S, metric, 0));
+    ERP_ARG(d_matches && d_n_matches && d_result && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose_bin_dev: bad argument");
+    ERP_ARG(d_left_xy && d_right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose_bin_dev: bad keypoints");
+    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "erp_pair_pose_bin_dev: no query descriptors");
+    DeviceGuard g(ctx->device);
+    // the leading tag keeps the graph of this call apart from erp_pair_pose_dev's with the same pointers and sizes
+    const uint64_t key[] = {0x48414d4d494e47ull, (uint64_t)(uintptr_t)d_q, (uint64_t)(uintptr_t)d_t, (uint64_t)(uintptr_t)d_left_xy, (uint64_t)(uintptr_t)d_right_xy, (uint64_t)(uintptr_t)d_matches, (uint64_t)(uintptr_t)d_n_matches, (uint64_t)(uintptr_t)d_mask, (uint64_t)(uintptr_t)d_result, (uint64_t)nq, (uint64_t)nt, (uint64_t)nbytes, (uint64_t)cross_check, (uint64_t)width, (uint64_t)height, (uint64_t)H, (uint64_t)S, (uint64_t)metric, (uint64_t)__builtin_bit_cast(uint32_t, ratio), (uint64_t)__builtin_bit_cast(uint32_t, tau), (uint64_t)seed, (uint64_t)kp_stride_bytes};
+    return graph_run(ctx, key, sizeof key, [&]() -> int {
+    ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
+    ERP_TRY(erp_knn2_match_bin_dev(ctx, d_q, nq, d_t, nt, nbytes, ratio, cross_check, d_matches, d_n_matches));
+    ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
+    return pose_after_match(ctx, d_matches, nq, d_n_matches, d_left_xy, d_right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
+                            d_mask, d_result);
+    });
+}
+
+ERP_API int erp_pair_pose_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes, const uint8_t* t, int nt,
+                              size_t t_stride_bytes, int nbytes, float ratio, int cross_check,
+                              const void* left_xy, const void* right_xy, size_t kp_stride_bytes, int width, int height,
+                              uint64_t seed, int H, int S, int metric, float tau,
+                              erp_dmatch* matches_out, int* n_matches, erp_ransac_result* result, uint8_t* mask)
+{
+    ERP_TRY(check_bin_args("erp_pair_pose_bin", ctx, nq, nt, nbytes));
+    ERP_TRY(check_ransac_args("erp_pair_pose_bin", ctx, H, S, metric, 0));
+    ERP_ARG(n_matches && result && matches_out && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose_bin: bad argument");
+    ERP_ARG(left_xy && right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose_bin: bad keypoints");
+    *n_matches = 0;
+    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "erp_pair_pose_bin: no query descriptors");
+    ERP_ARG(q && t && q_stride_bytes >= (size_t)nbytes && t_stride_bytes >= (size_t)nbytes, ERP_E_ARG,
+            "erp_pair_pose_bin: bad descriptor buffers");
+    DeviceGuard g(ctx->device);
+    int st = ERP_OK;
+    erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
+    int32_t* d_n = ctx->scratch<int32_t>(S_NOUT, 4, &st);
+    float* d_xy = ctx->scratch<float>(S_XY, ((size_t)nq + nt) * 2, &st);           // left pairs, then right pairs
+    uint8_t* dq = ctx->scratch<uint8_t>(S_Q, (size_t)nq * nbytes + 16, &st);
+    uint8_t* dt = ctx->scratch<uint8_t>(S_T, (size_t)nt * nbytes + 16, &st);
+    PoseBuffers b;
+    ERP_TRY(pose_chain_buffers(ctx, nq, &b));
+    ERP_TRY(st);
+    ERP_TRY(upload_rows(ctx, dt, t, nt, (size_t)nbytes, t_stride_bytes));
+    ERP_TRY(upload_rows(ctx, dq, q, nq, (size_t)nbytes, q_stride_bytes));
+    ERP_TRY(upload_rows(ctx, d_xy, left_xy, nq, 8, kp_stride_bytes));
+    ERP_TRY(upload_rows(ctx, d_xy + (size_t)nq * 2, right_xy, nt, 8, kp_stride_bytes));
+    ERP_TRY(erp_pair_pose_bin_dev(ctx, dq, nq, dt, nt, nbytes, ratio, cross_check, d_xy, d_xy + (size_t)nq * 2, 8, width, height,
+                                  seed, H, S, metric, tau, d_out, d_n, b.mask, b.res));
+    return pair_pose_download(ctx, "erp_pair_pose_bin", d_out, d_n, b, S, matches_out, n_matches, result, mask);
 }
 
 // ======================================================================================

@@ -77,6 +77,7 @@ struct erp_ctx {
     int engine = ERP_ENGINE_AUTO;
     uint64_t launches = 0;
     int64_t knn_stats[5] = {0, 0, 0, 0, 0};
+    bool knn_bin = false;                           // the last erp_knn2* search was on binary descriptors (knn_bin.cu)
     int32_t* sc_misc_dev = nullptr;                 // device words of the last tensor-core best search: ., max c_lo, list length
     int32_t* tc_misc_dev = nullptr;                 // device words of the last tcgen05 call: re-scan count, ., deviation
     cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr;   // around the dominant distance kernel
@@ -191,6 +192,9 @@ bool knn2_tc1_preferred(int nq, int nt, int dim);
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2);
 bool tc1_f16_operands();
+bool knn2_bin_preferred(int nq, int nt);
+int knn2_bin(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, bool tc,
+             int32_t* d_idx2, float* d_dist2, double* d_d2);
 int near_ties(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim, const int32_t* d_idx2, const double* d_d2,
               double rel_tol, int32_t* d_third, uint8_t* d_flags);
 int tc_misc_begin(erp_ctx* ctx, int32_t* misc);

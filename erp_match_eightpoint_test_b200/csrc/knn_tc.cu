@@ -612,6 +612,7 @@ int knn2_tc(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, in
     ERP_TRY(tc_misc_end(ctx, misc));
 
     ctx->knn_stats[0] = ERP_ENGINE_TCGEN05;
+    ctx->knn_bin = false;
     ctx->knn_stats[1] = -1;                       // re-scan count lives on the device: see erp_ctx_last_knn_stats
     ctx->knn_stats[2] = n_seg;
     ctx->knn_stats[3] = upc;

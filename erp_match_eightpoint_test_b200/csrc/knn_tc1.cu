@@ -646,6 +646,7 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     ERP_TRY(tc_misc_end(ctx, misc));
 
     ctx->knn_stats[0] = ERP_ENGINE_TCGEN05_1X;
+    ctx->knn_bin = false;
     ctx->knn_stats[1] = -1;
     ctx->knn_stats[2] = n_seg;
     ctx->knn_stats[3] = (int)L;

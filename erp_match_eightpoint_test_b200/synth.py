@@ -87,3 +87,29 @@ def keypoint_pair(m: int, W: int, H: int, euler_deg=(5.0, 10.0, 15.0), t=(0.3, -
     inl = np.ones(m, bool)
     inl[out_idx] = False
     return dict(left_xy=lp.astype(np.float32), right_xy=rp.astype(np.float32), R=R, t=t, E=E, inlier=inl)
+
+
+def binary_pair(nq: int, nt: int, nbytes: int = 32, f_match: float = 0.5, seed: int = SEED_BASE + 200):
+    """Binary descriptors (ORB-like uint8 rows) for Hamming matching.  Returns (query, train, planted): a share f_match of
+    the queries are train rows with a few flipped bits (planted[i] = that row, -1 for fresh random rows), and the last
+    nt // 16 train rows duplicate earlier ones, so that exact distance ties are certain."""
+    rng = _rng(seed)
+    nbits = 8 * nbytes
+    train = rng.integers(0, 256, size=(nt, nbytes), dtype=np.uint8)
+    n_dup = nt // 16
+    if n_dup:
+        train[nt - n_dup:] = train[rng.integers(0, nt - n_dup, size=n_dup)]
+    n_pl = min(int(nq * f_match), nt)
+    src = rng.permutation(nt)[:n_pl]
+    bits = np.unpackbits(train[src], axis=1)
+    k_max = max(1, nbits // 16)
+    pos = rng.integers(0, nbits, size=(n_pl, k_max))
+    keep = np.arange(k_max)[None, :] < rng.integers(1, k_max + 1, size=(n_pl, 1))
+    rows = np.broadcast_to(np.arange(n_pl)[:, None], pos.shape)
+    bits[rows[keep], pos[keep]] ^= 1
+    noisy = np.packbits(bits, axis=1)
+    fresh = rng.integers(0, 256, size=(nq - n_pl, nbytes), dtype=np.uint8)
+    query = np.concatenate([noisy, fresh], axis=0)
+    planted = np.concatenate([src, -np.ones(nq - n_pl, dtype=np.int64)])
+    perm = rng.permutation(nq)
+    return np.ascontiguousarray(query[perm]), train, planted[perm]

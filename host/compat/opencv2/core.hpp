@@ -290,6 +290,7 @@ inline void vconcat(const Mat* src, size_t n, Mat& dst)
     dst = out;
 }
 
+enum NormTypes { NORM_L2 = 4, NORM_HAMMING = 6 };
 enum RotateFlags { ROTATE_90_CLOCKWISE = 0, ROTATE_180 = 1, ROTATE_90_COUNTERCLOCKWISE = 2 };
 inline void rotate(const Mat& src, Mat& dst, int code)
 {

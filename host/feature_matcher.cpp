@@ -54,6 +54,25 @@ Mat feature_matcher::comput_descriptor(const Mat &image, vector<KeyPoint> &key_p
 // instead of the reference's approximate FLANN trees (SURVEY D1).
 vector<DMatch> feature_matcher::match_two_image(const Mat &descriptor1, const Mat &descriptor2)
 {
+    static_assert(sizeof(DMatch) == sizeof(erp_dmatch), "cv::DMatch and erp_dmatch must share a layout");
+    if (norm_type == cv::NORM_HAMMING) {
+        // binary descriptors: cv::BFMatcher(NORM_HAMMING) semantics on the kind::i8 / popcount engines
+        if (descriptor1.type() != CV_8UC1 || descriptor2.type() != CV_8UC1)
+            CV_Error(cv::Error::StsBadArg, "match_two_image: NORM_HAMMING descriptors must be CV_8U single channel");
+        if (descriptor1.rows > 0 && descriptor1.cols != descriptor2.cols)
+            CV_Error(cv::Error::StsBadArg, "match_two_image: descriptor sizes differ");
+        vector<DMatch> good(descriptor1.rows > 0 ? descriptor1.rows : 0);
+        int n = 0, st;
+        {
+            erp_host::Lock lock;
+            st = erp_knn2_match_bin(erp_host::context(), descriptor1.ptr<uint8_t>(0), descriptor1.rows, descriptor1.step,
+                                    descriptor2.ptr<uint8_t>(0), descriptor2.rows, descriptor2.step, descriptor1.cols,
+                                    ratio_thresh, cross_check ? 1 : 0, reinterpret_cast<erp_dmatch*>(good.data()), &n);
+        }
+        if (st != ERP_OK) CV_Error(cv::Error::StsBadArg, string("match_two_image: ") + erp_last_error());
+        good.resize(n);
+        return good;
+    }
     if (descriptor1.type() != CV_32FC1 || descriptor2.type() != CV_32FC1)
         CV_Error(cv::Error::StsBadArg, "match_two_image: descriptors must be CV_32F single channel");
     if (descriptor1.rows > 0 && descriptor1.cols != descriptor2.cols)

@@ -42,6 +42,7 @@ public:
 
     // CV_32F descriptors, one per row (64 or 128 wide; any multiple of 4 works).  Returns DMatch{queryIdx, trainIdx,
     // imgIdx = 0, distance = L2} in ascending queryIdx for the rows that pass d0 < ratio_thresh * d1.
+    // With norm_type == cv::NORM_HAMMING: CV_8U rows of 1..64 bytes, distance = Hamming.
     std::vector<cv::DMatch> match_two_image(const cv::Mat &descriptor1,
                                             const cv::Mat &descriptor2);
 
@@ -63,6 +64,9 @@ public:
     // --- extensions (SURVEY D5) -----------------------------------------------------------------------------------
     float ratio_thresh = 0.3f;               // Lowe ratio; the reference hard-codes 0.3f
     bool cross_check = false;                // keep a match only if it is also the train row's nearest query
+    // cv::NORM_HAMMING: match_two_image takes CV_8U binary descriptors (ORB, AKAZE, BRISK, ...) and matches them by
+    // Hamming distance (erp_knn2_match_bin); the default keeps the CV_32F / L2 behaviour
+    int norm_type = cv::NORM_L2;
     // SURF-128: re-creates the detector / extractor with extended descriptors (SURF::create(100, 4, 3, true))
     void set_extended(bool extended_descriptors);
     bool extended() const { return extended_; }

@@ -72,7 +72,8 @@ typedef enum {
 typedef enum {
     ERP_OPERANDS_NONE = 0,     /* no tensor product: ERP_ENGINE_EXACT_SIMT */
     ERP_OPERANDS_TF32 = 1,
-    ERP_OPERANDS_F16 = 2
+    ERP_OPERANDS_F16 = 2,
+    ERP_OPERANDS_I8 = 3        /* binary descriptors: bits expanded to +-1 int8, tcgen05.mma.kind::i8, exact s32 */
 } erp_operands;
 
 /* pose record per hypothesis: XYZ-euler of R1, of R2 (rad), t, validity flags (1.0/0.0), 1 pad */
@@ -163,6 +164,31 @@ int erp_match_filter_dev(erp_ctx* ctx, const int32_t* d_idx2, const float* d_dis
 int erp_knn2_match_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
                        float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out);
 
+/* ---------------------------------------------------------------- binary descriptors
+ * replaces feature_matcher::match_two_image      src/feature_matcher.cpp:42-59
+ * with cv::BFMatcher(NORM_HAMMING) in place of the L2 matcher: ORB, AKAZE (MLDB), BRISK, FREAK, LATCH rows.
+ * Rows are nbytes uint8 (1 <= nbytes <= 64, else ERP_E_DIM), strides in bytes; distance = popcount(q XOR t) over the
+ * nbytes bytes, carried as a float in erp_dmatch.distance and dist2 (as NORM_HAMMING does).  2-NN order is (distance,
+ * trainIdx) ascending: exact ties go to the lowest trainIdx.  Ratio test, cross-check (reverse ties: lowest queryIdx)
+ * and output order are those of the float entry points.  Every engine returns the same bits:
+ *   ERP_ENGINE_EXACT_SIMT              __popc on 32-bit words
+ *   ERP_ENGINE_TCGEN05, _TCGEN05_1X    both select the tcgen05.mma.kind::i8 engine (bits as +-1 int8: dot = n - 2 H,
+ *                                      exact in the s32 accumulator, so there is nothing to certify or re-scan)
+ *   ERP_ENGINE_AUTO                    kind::i8 from 1e6 query x train pairs up, SIMT below
+ * erp_ctx_last_knn_stats: [0] engine, [1] 0 (never re-scanned); erp_ctx_last_knn_operands: ERP_OPERANDS_I8 or NONE.
+ * Not provided for binary rows: the multi-GPU forms (_dist, erp_group_*). */
+int erp_knn2_match_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes,
+                       const uint8_t* t, int nt, size_t t_stride_bytes, int nbytes,
+                       float ratio, int cross_check, erp_dmatch* out, int* n_out);
+int erp_knn2_raw_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes,
+                     const uint8_t* t, int nt, size_t t_stride_bytes, int nbytes,
+                     int32_t* idx2, float* dist2);
+/* device-resident forms (dense rows: stride == nbytes), enqueue only */
+int erp_knn2_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes,
+                     int32_t* d_idx2, float* d_dist2, double* d_d2 /* nq x 2 or NULL */);
+int erp_knn2_match_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes,
+                           float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out);
+
 /* ---------------------------------------------------------------- geometry
  * pixel -> unit-sphere bearing, replaces src/eight_point.cpp:157-186.
  * xy points at the first (x,y) float pair; stride 28 == sizeof(cv::KeyPoint). */
@@ -242,6 +268,17 @@ int erp_pair_pose_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, 
                       const void* d_left_xy, const void* d_right_xy, size_t kp_stride_bytes, int width, int height,
                       uint64_t seed, int H, int S, int metric, float tau,
                       erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result);
+/* erp_pair_pose / erp_pair_pose_dev on binary descriptors (nbytes per row, Hamming matching as erp_knn2_match_bin);
+ * same keypoint, RANSAC and output arguments */
+int erp_pair_pose_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes, const uint8_t* t, int nt,
+                      size_t t_stride_bytes, int nbytes, float ratio, int cross_check,
+                      const void* left_xy, const void* right_xy, size_t kp_stride_bytes, int width, int height,
+                      uint64_t seed, int H, int S, int metric, float tau,
+                      erp_dmatch* matches_out /* nq */, int* n_matches, erp_ransac_result* result, uint8_t* mask /* nq or NULL */);
+int erp_pair_pose_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, float ratio,
+                          int cross_check, const void* d_left_xy, const void* d_right_xy, size_t kp_stride_bytes, int width,
+                          int height, uint64_t seed, int H, int S, int metric, float tau,
+                          erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result);
 /* sharded form: every rank scores its hypothesis range and leaves its packed best in
  * d_packed (one uint64 on the device); the caller max-reduces it across ranks (one 8-byte
  * NCCL allreduce) and calls erp_ransac_finish_dev with the winning packed value. */
