@@ -393,7 +393,7 @@ ERP_API int erp_ctx_last_knn_operands(erp_ctx* ctx, int64_t out[3])
     ERP_ARG(ctx && out, ERP_E_ARG, "erp_ctx_last_knn_operands: bad argument");
     const int64_t engine = ctx->knn_stats[0];
     out[0] = engine == ERP_ENGINE_TCGEN05 ? ERP_OPERANDS_TF32
-           : engine == ERP_ENGINE_TCGEN05_1X ? (ctx->knn_bin ? ERP_OPERANDS_I8 : tc1_f16_operands() ? ERP_OPERANDS_F16 : ERP_OPERANDS_TF32)
+           : engine == ERP_ENGINE_TCGEN05_1X ? (ctx->knn_bin ? ERP_OPERANDS_I8 : ERP_OPERANDS_F16)
            : ERP_OPERANDS_NONE;
     out[1] = out[2] = 0;
     if (out[0] == ERP_OPERANDS_F16 && ctx->tc_misc_dev) {

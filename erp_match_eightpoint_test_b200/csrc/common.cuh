@@ -191,7 +191,6 @@ bool knn2_tc_preferred(int nq, int nt, int dim);
 bool knn2_tc1_preferred(int nq, int nt, int dim);
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2);
-bool tc1_f16_operands();
 bool knn2_bin_preferred(int nq, int nt);
 int knn2_bin(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, bool tc,
              int32_t* d_idx2, float* d_dist2, double* d_d2);

@@ -1,18 +1,16 @@
-// knn_tc1.cu -- the fast tcgen05 distance engine: ONE product of 11-bit operands per tile (f16 by default, tf32 on request),
+// knn_tc1.cu -- the fast tcgen05 distance engine: ONE product of IEEE f16 operands per tile (tcgen05.mma kind::f16),
 // a wider candidate list and the same exact certificate.
 //
 // knn_tc.cu reproduces fp32 ranking by arithmetic (3xTF32).  The certificate of refine_kernel makes
 // that unnecessary: any approximate score with a known error bound yields the exact 2-NN as long as
 //     d2_exact(second) < min_lists(s_kth) + |q|^2 - eps        (otherwise the query is re-scanned)
-// holds, and a single product of 11-bit operands (TF32 or IEEE FP16) has a worst-case error of 2^-10 (|q|^2 + |t|^2) (inputs rounded
-// to 11 significant bits, products exact, fp32 accumulation).  Only columns within twice that error
-// of the running second best are kept (up to 8 per list: near-ties overflow 4), which for SURF-like
-// data leaves almost nothing to re-scan, so the kernel issues a third of the tensor work:
-//     8 UMMA instructions per 128 x 256 tile instead of 24.
-// FP16 operands (the default) carry the same 11 significant bits at twice the tf32 rate and half the bytes: 5 UMMA
-// instructions per tile at D = 64 (4 + the norm step) instead of 9, and 32 KB of train operand per tile instead of 64 KB.
-// ERP_B200_TC1_OPERANDS=tf32 selects the tf32 operands (same results, the A/B baseline).
-// At the tf32 rate the L2 -> shared-memory feed becomes the limiter, so every 64 KB train tile that TMA
+// holds, and a single product of operands with 11 significant bits has a worst-case error of 2^-10 (|q|^2 + |t|^2) (inputs
+// rounded to 11 significant bits, products exact, fp32 accumulation).  f16 meets all three, as tf32 does, at twice the tf32
+// rate and half the bytes.  Only columns within twice that error of the running second best are kept (up to 8 per list:
+// near-ties overflow 4), which for SURF-like data leaves almost nothing to re-scan, so the kernel issues a fifth of the
+// tensor instructions of 3xTF32, each at twice the rate:
+//     5 UMMA instructions per 128 x 256 tile at D = 64 (4 + the norm step) instead of 24.
+// At that rate the L2 -> shared-memory feed becomes the limiter, so every train tile (32 KB per k chunk) that TMA
 // brings in is multiplied against TWO resident query tiles (256 queries), alternating between the
 // two TMEM accumulators.  Results are identical to the exact engine by construction.
 #include "tc_common.cuh"
@@ -22,10 +20,9 @@
 namespace erp {
 
 constexpr int F_BM = 128;                 // queries per sub-tile (UMMA M)
-constexpr int F_SUB_MAX = 2;              // resident query sub-tiles sharing every train tile (1 beyond three k chunks: smem)
+constexpr int F_SUB = 2;                  // resident query sub-tiles sharing every train tile
 constexpr int F_BN = 256;                 // train rows per tile (UMMA N)
-// a k chunk is one 128-byte swizzle row: 32 floats or 64 halves
-__host__ __device__ constexpr int f_kc(bool half) { return half ? 64 : 32; }
+constexpr int F_KC = 64;                  // halves per k chunk: one 128-byte swizzle row
 constexpr int F_QCH = F_BM * 128;         // 16 KB
 constexpr int F_TCH = F_BN * 128;         // 32 KB
 constexpr int F_EPI_GROUPS = 2;
@@ -34,7 +31,7 @@ constexpr int F_THREADS = 128 + F_EPI_THREADS;
 constexpr int F_EPI_COLS = F_BN / F_EPI_GROUPS;
 constexpr int F_TOPK = 8;
 constexpr int F_MAX_SEG = 128 / (F_TOPK * F_EPI_GROUPS);    // up to 8 segments per query pair (refine_kernel: 128 candidate slots)
-constexpr int F_AUG_T = F_BN * 32;        // 8 KB: one extra k step (8 floats or 16 halves) per train row, 32-byte swizzle rows
+constexpr int F_AUG_T = F_BN * 32;        // 8 KB: one extra k step (16 halves) per train row, 32-byte swizzle rows
 constexpr int F_AUG_Q = F_BM * 32;        // 4 KB: the constant query side of that k step
 constexpr int F_BARS = 256;               // mbarriers + TMEM slot
 // Instrumented builds (scripts/build_variant.sh N): -DERP_TC_COUNTERS=1 adds clock64 phase timers to the MMA issuer and the
@@ -55,8 +52,8 @@ static __device__ unsigned long long erp_clk[8];
 #define TCC_FLUSH()
 #endif
 // |s_tc - s_exact| <= 2^-10 (|q|^2 + max|t|^2) in the worst case: both operands are rounded to 11
-// significant bits (relative error 2^-11 each: tf32 rounds to nearest away, f16 to nearest even, the worst case is the same),
-// products are exact (11 x 11 bits fit fp32, and so do f16 subnormal products), and 2|q||t| <= |q|^2 + |t|^2.
+// significant bits (relative error 2^-11 each, f16 rounds to nearest even), products are exact (11 x 11 bits fit fp32,
+// and so do f16 subnormal products), and 2|q||t| <= |q|^2 + |t|^2.
 // On top of 2^-10: the second-order rounding term (2^-22 relative = 2^-12 of the budget), the column id packed into the
 // three low mantissa bits of a score (<= 7 ulp = 2^-21 relative), and the fp32 accumulation inside the tensor pipe,
 // whose rounding mode is not documented: with truncating adds over D + 3 <= 131 terms the worst case is 131 * 2^-24
@@ -72,35 +69,26 @@ static __device__ unsigned long long erp_clk[8];
 //     |q| or max|t| is above ~0.1 (SURF is unit-norm, SIFT far above), so real descriptors never take this path.
 constexpr double F_KAPPA = 1.05 / 1024.0;
 constexpr double F_F16_ABS = 0.02 / 1024.0;
-// instruction descriptors: D fp32, A/B tf32 (format 2) or f16 (format 0), both K-major, N = 256, M = 128
-constexpr uint32_t F_IDESC_TF32 = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(F_BN >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
-constexpr uint32_t F_IDESC_F16 = (1u << 4) | ((uint32_t)(F_BN >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
-// f16 norm step: train row (hi, mid, lo, 0 x 5 | 0 x 8), query row (2^8, 2^-3, 2^-14, 2^15 x 5) in both 16-byte halves, so
-// |t|^2 = 2^8 hi + 2^-3 mid + 2^-14 lo (a 33-bit split of the fp32 norm: exact while hi is normal, within 2^-39 below).  Padding
-// train rows put 65504 into the five 2^15 slots: 1.07e10, finite, and above any score the range guard lets through
-// (|2q| |t| <= 65504 sqrt(128) * 4096 = 3.0e9 plus |t|^2 < 1.7e7)
+// instruction descriptor: D fp32, A/B f16 (format 0), both K-major, N = 256, M = 128
+constexpr uint32_t F_IDESC = (1u << 4) | ((uint32_t)(F_BN >> 3) << 17) | ((uint32_t)(F_BM >> 4) << 24);
+// |t|^2 enters the accumulator through the tensor core, as an extra k step after the k chunks, so the epilogue neither
+// loads nor adds it.  Norm step: train row (hi, mid, lo, 0 x 5 | 0 x 8), query row (2^8, 2^-3, 2^-14, 2^15 x 5) in both
+// 16-byte halves, so |t|^2 = 2^8 hi + 2^-3 mid + 2^-14 lo (a 33-bit split of the fp32 norm: exact while hi is normal,
+// within 2^-39 below).  Padding train rows put 65504 into the five 2^15 slots: 1.07e10, finite, and above any score the
+// range guard lets through (|2q| |t| <= 65504 sqrt(128) * 4096 = 3.0e9 plus |t|^2 < 1.7e7)
 __host__ __device__ constexpr float f16_norm_scale(int i) { return i == 0 ? 256.0f : i == 1 ? 0.125f : i == 2 ? 1.0f / 16384.0f : 32768.0f; }
 
-__host__ __device__ constexpr int f_sub(int kch) { return kch <= 3 ? F_SUB_MAX : 1; }
-// D <= 64: |t|^2 enters the accumulator through the tensor core (an extra k step whose train side is the
-// norm split in three tf32 pieces and whose query side is 1,1,1), so the epilogue neither loads nor adds it.
-// Wider descriptors keep the norm add: the 20 KB of operand staging would cost them a ring slot they need.
-__host__ __device__ constexpr bool f_fold(int kch) { return kch <= 2; }
-__host__ __device__ constexpr int f_tail(int kch, bool share)
-{
-    return (f_fold(kch) ? 2 * F_AUG_T + F_AUG_Q : 2 * F_BN * 4) + F_BARS + (share ? f_sub(kch) * F_BM * 4 : 0);
-}
-__host__ __device__ constexpr int f_slots_for(int kch, bool share) { return (TC_SMEM_LIMIT - f_sub(kch) * kch * F_QCH - f_tail(kch, share)) / F_TCH; }
-// the per-row threshold exchange between the two column groups needs 512 B per sub-tile: on unless it costs the look-ahead slot
-__host__ __device__ constexpr bool f_share(int kch) { return f_slots_for(kch, true) >= kch + 1; }
-__host__ __device__ constexpr int f_slots(int kch) { return f_slots_for(kch, f_share(kch)); }
-__host__ __device__ constexpr int f_smem(int kch) { return f_sub(kch) * kch * F_QCH + f_slots(kch) * F_TCH + f_tail(kch, f_share(kch)); }
+// shared memory behind the query chunks and the T ring: the norm operand (two train tiles and the query side), the barriers,
+// and the per-row threshold exchange between the two column groups (512 B per sub-tile)
+constexpr int F_TAIL = 2 * F_AUG_T + F_AUG_Q + F_BARS + F_SUB * F_BM * 4;
+__host__ __device__ constexpr int f_slots(int kch) { return (TC_SMEM_LIMIT - F_SUB * kch * F_QCH - F_TAIL) / F_TCH; }
+__host__ __device__ constexpr int f_smem(int kch) { return F_SUB * kch * F_QCH + f_slots(kch) * F_TCH + F_TAIL; }
 
-// one operand of a prep launch: rows x, scaled, rounded to tf32 or f16 into out (dpad elements per row); norms (+inf padding up
-// to n_pad), their maximum, and the 32-byte norm operand rows when aug is given
+// one operand of a prep launch: rows x, scaled, rounded to f16 into out (dpad halves per row); norms (+inf padding up to n_pad),
+// their maximum, and the 32-byte norm operand rows when aug is given
 // LPR lanes own one row (4 elements per lane and pass); a warp covers 32 / LPR rows
 struct RoundJob {
-    const float* x; int n; float scale; void* out; float* norm; int n_pad; unsigned* max_bits; void* aug; int blocks;
+    const float* x; int n; float scale; __half* out; float* norm; int n_pad; unsigned* max_bits; __half* aug; int blocks;
 };
 
 // f16 of a scaled input; a finite input whose f16 is infinite marks the call for the exact re-scan
@@ -112,7 +100,7 @@ __device__ __forceinline__ __half f16_guarded(float x, float scaled, bool& wide)
 }
 
 // both operands of a search in ONE launch: blocks [0, a.blocks) round the queries, the rest the train rows
-template <int LPR, bool HALF>
+template <int LPR>
 __global__ void __launch_bounds__(256)
 round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad, unsigned* wide_flag)
 {
@@ -133,15 +121,9 @@ round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad, unsigned* wi
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
             if (k < dim) v = *reinterpret_cast<const float4*>(x + (size_t)row * dim + k);
             acc += (double)v.x * v.x + (double)v.y * v.y + (double)v.z * v.z + (double)v.w * v.w;
-            if (HALF) {
-                __half2* o = reinterpret_cast<__half2*>(static_cast<__half*>(j.out) + (size_t)row * dpad + k);
-                o[0] = __halves2half2(f16_guarded(v.x, __fmul_rn(v.x, scale), wide), f16_guarded(v.y, __fmul_rn(v.y, scale), wide));
-                o[1] = __halves2half2(f16_guarded(v.z, __fmul_rn(v.z, scale), wide), f16_guarded(v.w, __fmul_rn(v.w, scale), wide));
-            } else {
-                float4 hi = make_float4(tf32_rna(__fmul_rn(v.x, scale)), tf32_rna(__fmul_rn(v.y, scale)),
-                                        tf32_rna(__fmul_rn(v.z, scale)), tf32_rna(__fmul_rn(v.w, scale)));
-                *reinterpret_cast<float4*>(static_cast<float*>(j.out) + (size_t)row * dpad + k) = hi;
-            }
+            __half2* o = reinterpret_cast<__half2*>(j.out + (size_t)row * dpad + k);
+            o[0] = __halves2half2(f16_guarded(v.x, __fmul_rn(v.x, scale), wide), f16_guarded(v.y, __fmul_rn(v.y, scale), wide));
+            o[1] = __halves2half2(f16_guarded(v.z, __fmul_rn(v.z, scale), wide), f16_guarded(v.w, __fmul_rn(v.w, scale), wide));
         }
     }
     if (norm) {
@@ -150,7 +132,7 @@ round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad, unsigned* wi
         if (l == 0 && row < n_pad) {
             float f = row < n ? (float)acc : INFINITY;
             norm[row] = f;
-            if (j.aug && HALF) {
+            if (j.aug) {
                 // |t|^2 = 2^8 hi + 2^-3 mid + 2^-14 lo (f16_norm_scale); rows past the end fill the 2^15 slots
                 unsigned short h[8] = {0, 0, 0, 0, 0, 0, 0, 0};
                 if (row < n) {
@@ -163,111 +145,88 @@ round_kernel(const RoundJob a, const RoundJob b, int dim, int dpad, unsigned* wi
                 } else {
                     for (int i = 3; i < 8; i++) h[i] = 0x7bffu;   // 65504
                 }
-                uint4* o = reinterpret_cast<uint4*>(static_cast<__half*>(j.aug) + (size_t)row * 16);
+                uint4* o = reinterpret_cast<uint4*>(j.aug + (size_t)row * 16);
                 o[0] = make_uint4(h[0] | (uint32_t)h[1] << 16, h[2] | (uint32_t)h[3] << 16, h[4] | (uint32_t)h[5] << 16, h[6] | (uint32_t)h[7] << 16);
                 o[1] = make_uint4(0u, 0u, 0u, 0u);
-            } else if (j.aug) {
-                // |t|^2 = hi + mid + lo exactly, every piece a tf32 number; rows past the end score 1e30
-                const float g = row < n ? f : 1e30f;
-                const float hi = tf32_rna(g), r1 = __fsub_rn(g, hi), mid = tf32_rna(r1), lo = __fsub_rn(r1, mid);
-                float* aug = static_cast<float*>(j.aug);
-                *reinterpret_cast<float4*>(aug + (size_t)row * 8) = make_float4(hi, mid, lo, 0.f);
-                *reinterpret_cast<float4*>(aug + (size_t)row * 8 + 4) = make_float4(0.f, 0.f, 0.f, 0.f);
             }
             // non-negative floats (and +inf, NaN) order like their bit patterns
             // one hot word for the whole array: read it first, the atomic only fires while the maximum still grows
             if (row < n && __float_as_uint(f) > *reinterpret_cast<volatile unsigned*>(max_bits)) atomicMax(max_bits, __float_as_uint(f));
         }
     }
-    if (HALF && wide) *wide_flag = 1u;
+    if (wide) *wide_flag = 1u;
 }
 
-template <bool HALF>
-static void launch_round(erp_ctx* ctx, int lpr, int grid, const RoundJob& a, const RoundJob& b, int dim, int dpad, unsigned* wide_flag)
+static int launch_prep(erp_ctx* ctx, RoundJob a, RoundJob b, int dim, int dpad, unsigned* wide_flag)
 {
-    if (lpr == 8) round_kernel<8, HALF><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
-    else if (lpr == 16) round_kernel<16, HALF><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
-    else round_kernel<32, HALF><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
-}
-
-static int launch_prep(erp_ctx* ctx, RoundJob a, RoundJob b, int dim, int dpad, bool half, unsigned* wide_flag)
-{
-    // 8 / 16 / 32 lanes per row for dpad = 32 / 64 / (96, 128)
-    const int lpr = dpad <= 32 ? 8 : dpad <= 64 ? 16 : 32;
+    // 16 lanes per row for dpad = 64, 32 for dpad = 128
+    const int lpr = dpad <= 64 ? 16 : 32;
     const int rows_per_block = 8 * (32 / lpr);
     a.blocks = cdiv(a.n_pad, rows_per_block);
     b.blocks = b.x ? cdiv(b.n_pad, rows_per_block) : 0;
     const int grid = a.blocks + b.blocks;
-    if (half) launch_round<true>(ctx, lpr, grid, a, b, dim, dpad, wide_flag);
-    else launch_round<false>(ctx, lpr, grid, a, b, dim, dpad, wide_flag);
+    if (lpr == 16) round_kernel<16><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
+    else round_kernel<32><<<grid, 256, 0, ctx->stream>>>(a, b, dim, dpad, wide_flag);
     ERP_LAUNCH(ctx, "round_kernel");
     return ERP_OK;
 }
 
 struct Tc1Params {
-    int nq, nt;
-    int n_qpairs, n_ttiles;   // n_qpairs counts groups of f_sub(kch) query sub-tiles
-    int units_per_cta;        // CTA b owns units [b*L, (b+1)*L) of the n_qpairs x n_ttiles grid
-    int n_seg;                // candidate lists per query = n_seg x F_EPI_GROUPS
-    const float* tn;
     const float* qn;          // nq query norms |q|^2
     const unsigned* tn_max_bits;
     int32_t* cand_idx;        // nq x lists x F_TOPK, pre-set to -1
     float* cand_s;
     float* cand_thr;          // nq x lists: lower bound of the approximate score of every non-candidate
     int32_t* row_thr;         // nq ordered-int keys (or null): the lowest threshold any segment of the row has published
+    int nq, nt;
+    int n_qpairs, n_ttiles;   // n_qpairs counts groups of F_SUB query sub-tiles
+    int units_per_cta;        // CTA b owns units [b*L, (b+1)*L) of the n_qpairs x n_ttiles grid
+    int n_seg;                // candidate lists per query = n_seg x F_EPI_GROUPS
 };
 
 // monotone float <-> int key (scores may be negative), so that atomicMin orders thresholds
 __device__ __forceinline__ int32_t thr_key(float f) { const int32_t k = __float_as_int(f); return k >= 0 ? k : k ^ 0x7fffffff; }
 __device__ __forceinline__ float key_thr(int32_t k) { return __int_as_float(k >= 0 ? k : k ^ 0x7fffffff); }
 
-template <bool HALF>
-__device__ __forceinline__ void f_mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate)
-{
-    if (HALF) tc_mma_f16(d_tmem, a_desc, b_desc, F_IDESC_F16, accumulate);
-    else tc_mma_tf32(d_tmem, a_desc, b_desc, F_IDESC_TF32, accumulate);
-}
-
-template <int KCH, bool HALF>   // KCH k chunks of 128 bytes: dpad = KCH * f_kc(HALF) elements
+template <int KCH>   // KCH k chunks of 128 bytes: dpad = KCH * F_KC halves
 __global__ void __launch_bounds__(F_THREADS, 1)
 knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_t,
                 const __grid_constant__ CUtensorMap map_aug, const Tc1Params p)
 {
-    constexpr int NS = f_slots(KCH), F_SUB = f_sub(KCH);
-    constexpr bool FOLD = f_fold(KCH), SHARE = f_share(KCH);
+    constexpr int NS = f_slots(KCH);
     static_assert(NS >= KCH + 1, "T ring must hold one tile plus a chunk of look-ahead");
     extern __shared__ __align__(1024) uint8_t smem[];
     if ((smem_u32(smem) & 1023u) != 0) __trap();
     uint8_t* q_smem = smem;                                   // [F_SUB][KCH] chunks
     uint8_t* t_smem = smem + F_SUB * KCH * F_QCH;             // NS slots
-    uint8_t* aug_t = t_smem + NS * F_TCH;                     // FOLD: [2][F_AUG_T] by train-tile parity, then the query side
+    uint8_t* aug_t = t_smem + NS * F_TCH;                     // [2][F_AUG_T] norm operand by train-tile parity, then the query side
     uint8_t* aug_q = aug_t + 2 * F_AUG_T;
-    float* tn_smem = reinterpret_cast<float*>(t_smem + NS * F_TCH);   // !FOLD: [2][F_BN] |t|^2, by train-tile parity
-    uint64_t* bars = reinterpret_cast<uint64_t*>(t_smem + NS * F_TCH + (FOLD ? 2 * F_AUG_T + F_AUG_Q : 2 * F_BN * 4));
+    uint64_t* bars = reinterpret_cast<uint64_t*>(aug_q + F_AUG_Q);
     uint64_t* full = bars;              // [NS]  TMA -> MMA
     uint64_t* empty = bars + NS;        // [NS]  MMA -> TMA
     uint64_t* qfull = bars + 2 * NS;    // query pair landed
     uint64_t* qempty = qfull + 1;       // query pair no longer read
     uint64_t* tfull = qfull + 2;        // [2] accumulator ready
     uint64_t* tempty = qfull + 4;       // [2] accumulator drained
-    uint64_t* nfull = qfull + 6;        // [2] |t|^2 of a train tile landed
-    uint64_t* nempty = qfull + 8;       // [2] ... and consumed by both sub-tiles (FOLD: by their MMAs)
+    uint64_t* nfull = qfull + 6;        // [2] norm operand of a train tile landed
+    uint64_t* nempty = qfull + 8;       // [2] ... and read by the MMAs of both sub-tiles
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(qfull + 10);
     static_assert((2 * NS + 10) * 8 + 4 <= F_BARS, "barrier block");
-    float* thr_sh = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + F_BARS);   // SHARE: [F_SUB][F_BM] row thresholds
+    float* thr_sh = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + F_BARS);   // [F_SUB][F_BM] row thresholds
+    static_assert(F_SUB * KCH * F_QCH + NS * F_TCH + 2 * F_AUG_T + F_AUG_Q + F_BARS + F_SUB * F_BM * 4 <= f_smem(KCH),
+                  "threshold exchange area");
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     TCC_DECL;
     constexpr int W_ALLOC = F_EPI_THREADS / 32, W_NORM = W_ALLOC + 1, W_TMA = W_ALLOC + 2, W_MMA = W_ALLOC + 3;
 
-    if (warp == W_TMA && lane == 0) { tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_t); if (FOLD) tma_prefetch_desc(&map_aug); }
+    if (warp == W_TMA && lane == 0) { tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_t); tma_prefetch_desc(&map_aug); }
     if (warp == W_MMA && lane == 0) {
         for (int i = 0; i < NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
         mbar_init(qfull, 1); mbar_init(qempty, 1);
         for (int i = 0; i < 2; i++) {
             mbar_init(&tfull[i], 1); mbar_init(&tempty[i], F_EPI_THREADS / 32);
-            mbar_init(&nfull[i], 1); mbar_init(&nempty[i], FOLD ? 1 : F_EPI_THREADS / 32);
+            mbar_init(&nfull[i], 1); mbar_init(&nempty[i], 1);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -275,16 +234,10 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    if (FOLD && HALF) {
-        // query side of the norm step: the same 8 halves in both 16-byte halves of every row, which the swizzle cannot change
-        for (int i = threadIdx.x; i < F_AUG_Q / 2; i += F_THREADS)
-            reinterpret_cast<__half*>(aug_q)[i] = __float2half_rn(f16_norm_scale(i & 7));
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    } else if (FOLD) {
-        // query side of the norm step: (1,1,1,0) in both 16-byte halves of every row, which the swizzle cannot change
-        for (int i = threadIdx.x; i < F_AUG_Q / 4; i += F_THREADS) reinterpret_cast<float*>(aug_q)[i] = (i & 3) != 3 ? 1.0f : 0.0f;
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
+    // query side of the norm step: the same 8 halves in both 16-byte halves of every row, which the swizzle cannot change
+    for (int i = threadIdx.x; i < F_AUG_Q / 2; i += F_THREADS)
+        reinterpret_cast<__half*>(aug_q)[i] = __float2half_rn(f16_norm_scale(i & 7));
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -306,13 +259,13 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                 for (int sub = 0; sub < F_SUB; sub++)
 #pragma unroll
                     for (int c = 0; c < KCH; c++)
-                        tma_load_2d(&map_q, qfull, q_smem + (sub * KCH + c) * F_QCH, c * f_kc(HALF), (qp * F_SUB + sub) * F_BM);
+                        tma_load_2d(&map_q, qfull, q_smem + (sub * KCH + c) * F_QCH, c * F_KC, (qp * F_SUB + sub) * F_BM);
                 for (int tt = t0; tt < t1; tt++) {
 #pragma unroll
                     for (int c = 0; c < KCH; c++) {
                         mbar_wait(&empty[slot], ph ^ 1);
                         mbar_expect_tx(&full[slot], F_TCH);
-                        tma_load_2d(&map_t, &full[slot], t_smem + slot * F_TCH, c * f_kc(HALF), tt * F_BN);
+                        tma_load_2d(&map_t, &full[slot], t_smem + slot * F_TCH, c * F_KC, tt * F_BN);
                         if (++slot == NS) { slot = 0; ph ^= 1; }
                     }
                 }
@@ -347,20 +300,19 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                             TCC_ADD(5, clock64() - f0);
                             tc_fence_after();
                             const uint32_t a = q_base + (sub * KCH + c) * F_QCH, b = t_base + sl * F_TCH;
-                            // one instruction per 32 bytes of the 128-byte row: K = 8 tf32 or K = 16 f16
+                            // one instruction per 32 bytes of the 128-byte row: K = 16 halves
 #pragma unroll
                             for (int k = 0; k < 4; k++)
-                                f_mma<HALF>(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), (c | k) != 0);
+                                tc_mma_f16(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), F_IDESC, (c | k) != 0);
                             if (sub == F_SUB - 1) tc_commit(&empty[sl]);
                             if (++sl == NS) { sl = 0; pp ^= 1; }
                         }
-                        if (FOLD) {
-                            const uint32_t nb = tt_n & 1;
-                            if (sub == 0) mbar_wait(&nfull[nb], (tt_n >> 1) & 1);
-                            tc_fence_after();
-                            f_mma<HALF>(d_tmem, aq_desc, smem_desc_sw32(smem_u32(aug_t + nb * F_AUG_T)), 1);
-                            if (sub == F_SUB - 1) tc_commit(&nempty[nb]);
-                        }
+                        // the norm step
+                        const uint32_t nb = tt_n & 1;
+                        if (sub == 0) mbar_wait(&nfull[nb], (tt_n >> 1) & 1);
+                        tc_fence_after();
+                        tc_mma_f16(d_tmem, aq_desc, smem_desc_sw32(smem_u32(aug_t + nb * F_AUG_T)), F_IDESC, 1);
+                        if (sub == F_SUB - 1) tc_commit(&nempty[nb]);
                         tc_commit(&tfull[acc]);
                         if (sub == F_SUB - 1) { slot = sl; ph = pp; }
                     }
@@ -369,7 +321,7 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
             }
         }
     } else if (warp == W_NORM) {
-        // ================================================================ |t|^2 producer (one bulk copy per train tile)
+        // ================================================================ norm operand producer (one TMA load per train tile)
         if (lane == 0) {
             uint32_t tt_n = 0;
             SegIter it(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x);
@@ -378,15 +330,8 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                 for (int tt = t0; tt < t1; tt++, tt_n++) {
                     const uint32_t nb = tt_n & 1;
                     mbar_wait(&nempty[nb], ((tt_n >> 1) & 1) ^ 1);
-                    if (FOLD) {
-                        mbar_expect_tx(&nfull[nb], F_AUG_T);
-                        tma_load_2d(&map_aug, &nfull[nb], aug_t + nb * F_AUG_T, 0, tt * F_BN);
-                        continue;
-                    }
-                    mbar_expect_tx(&nfull[nb], F_BN * 4);
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                                 ::"r"(smem_u32(tn_smem + nb * F_BN)), "l"(p.tn + (size_t)tt * F_BN), "r"(F_BN * 4), "r"(smem_u32(&nfull[nb]))
-                                 : "memory");
+                    mbar_expect_tx(&nfull[nb], F_AUG_T);
+                    tma_load_2d(&map_aug, &nfull[nb], aug_t + nb * F_AUG_T, 0, tt * F_BN);
                 }
             }
         }
@@ -396,7 +341,7 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         // ================================================================ epilogue (2 column groups x 4 lane quarters)
         const int ew = warp & 3, cg = warp >> 2;
         const int row = ew * 32 + lane;
-        uint32_t tile_n = 0, tt_n = 0;
+        uint32_t tile_n = 0;
         SegIter it(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x);
         int qp, t0, t1, seg;
         while (it.next(qp, t0, t1, seg)) {
@@ -420,24 +365,21 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
             // the segments publish theirs (atomicMin on an ordered key) and fold the others' in every few tiles: the row
             // then warms up once, not once per segment.  Racy on purpose: every published value is a valid bound, and
             // floor_thr -- the lowest threshold ever in force -- is what the list's certificate bound is built from.
-            const bool seed = SHARE && p.row_thr != nullptr;
+            const bool seed = p.row_thr != nullptr;
             float published[F_SUB];
 #pragma unroll
             for (int sub = 0; sub < F_SUB; sub++) published[sub] = INFINITY;
-            if (SHARE) {
-                // every epilogue warp has left the previous query rows before their thresholds are replaced
-                asm volatile("bar.sync 1, %0;" ::"n"(F_EPI_THREADS) : "memory");
+            // every epilogue warp has left the previous query rows before their thresholds are replaced
+            asm volatile("bar.sync 1, %0;" ::"n"(F_EPI_THREADS) : "memory");
 #pragma unroll
-                for (int sub = 0; sub < F_SUB; sub++) {
-                    const int qrow = (qp * F_SUB + sub) * F_BM + row;
-                    float g = INFINITY;
-                    if (seed && qrow < p.nq) g = key_thr(*reinterpret_cast<volatile int32_t*>(p.row_thr + qrow));
-                    thr_sh[sub * F_BM + row] = g;
-                }
-                asm volatile("bar.sync 1, %0;" ::"n"(F_EPI_THREADS) : "memory");
+            for (int sub = 0; sub < F_SUB; sub++) {
+                const int qrow = (qp * F_SUB + sub) * F_BM + row;
+                float g = INFINITY;
+                if (seed && qrow < p.nq) g = key_thr(*reinterpret_cast<volatile int32_t*>(p.row_thr + qrow));
+                thr_sh[sub * F_BM + row] = g;
             }
-            for (int tt = t0; tt < t1; tt++, tt_n++) {
-                const uint32_t nb = tt_n & 1;
+            asm volatile("bar.sync 1, %0;" ::"n"(F_EPI_THREADS) : "memory");
+            for (int tt = t0; tt < t1; tt++) {
                 // every fourth tile: fetch the row's published bound now, use it after this tile's scan
                 const bool sync_thr = seed && ((tt - t0) & 3) == 3;
                 int32_t fetched[F_SUB];
@@ -448,8 +390,6 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                         fetched[sub] = qrow < p.nq ? *reinterpret_cast<volatile int32_t*>(p.row_thr + qrow) : 0x7f7f7f7f;
                     }
                 }
-                if (!FOLD) mbar_wait(&nfull[nb], (tt_n >> 1) & 1);
-                const float4* tn4 = reinterpret_cast<const float4*>(tn_smem + nb * F_BN + cg * F_EPI_COLS);
                 const int colbase = tt * F_BN + cg * F_EPI_COLS;
 #pragma unroll
                 for (int sub = 0; sub < F_SUB; sub++, tile_n++) {
@@ -472,25 +412,14 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                     tc_wait_ld32(vb);
                     tc_wait_ld32(vc);
                     tc_wait_ld32(vd);
-                    if (FOLD) {
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(&tempty[acc]);
-                    }
-                    scan_chunk_lean<SHARE, FOLD>(va, tn4, colbase, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
-                    scan_chunk_lean<SHARE, FOLD>(vb, tn4 + 8, colbase + 32, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
-                    scan_chunk_lean<SHARE, FOLD>(vc, tn4 + 16, colbase + 64, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
-                    scan_chunk_lean<SHARE, FOLD>(vd, tn4 + 24, colbase + 96, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
-                    if (!FOLD) {
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(&tempty[acc]);
-                    }
-                    TCC_ADD(0, c1 - c0); TCC_ADD(1, clock64() - c1); TCC_ADD(2, 1);
-                }
-                if (!FOLD) {
+                    tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) mbar_arrive(&nempty[nb]);
+                    if (lane == 0) mbar_arrive(&tempty[acc]);
+                    scan_chunk_lean(va, colbase, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
+                    scan_chunk_lean(vb, colbase + 32, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
+                    scan_chunk_lean(vc, colbase + 64, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
+                    scan_chunk_lean(vd, colbase + 96, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
+                    TCC_ADD(0, c1 - c0); TCC_ADD(1, clock64() - c1); TCC_ADD(2, 1);
                 }
                 if (sync_thr) {
 #pragma unroll
@@ -547,14 +476,14 @@ __global__ void dbg_print_kernel()
     for (int i = 0; i < 8; i++) erp_clk[i] = 0;
 }
 #endif
-template <int KCH, bool HALF>
+template <int KCH>
 static int launch_tc1(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt, const CUtensorMap& ma, const Tc1Params& p, int grid)
 {
     constexpr int smem = f_smem(KCH);
     static_assert(smem <= TC_SMEM_LIMIT, "shared memory budget");
     static std::atomic<uint64_t> configured{0};
-    ERP_TRY(ensure_dynamic_smem(ctx, knn2_tc1_kernel<KCH, HALF>, smem, configured));
-    knn2_tc1_kernel<KCH, HALF><<<grid, F_THREADS, smem, ctx->stream>>>(mq, mt, ma, p);
+    ERP_TRY(ensure_dynamic_smem(ctx, knn2_tc1_kernel<KCH>, smem, configured));
+    knn2_tc1_kernel<KCH><<<grid, F_THREADS, smem, ctx->stream>>>(mq, mt, ma, p);
     ERP_LAUNCH(ctx, "knn2_tc1_kernel");
 #if ERP_TC_COUNTERS
     dbg_print_kernel<<<1, 1, 0, ctx->stream>>>();
@@ -563,20 +492,12 @@ static int launch_tc1(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt
     return ERP_OK;
 }
 
-// operands of the one-product engine: f16 unless ERP_B200_TC1_OPERANDS=tf32 (read once)
-bool tc1_f16_operands()
-{
-    static const bool f16 = [] { const char* e = getenv("ERP_B200_TC1_OPERANDS"); return !(e && strcmp(e, "tf32") == 0); }();
-    return f16;
-}
-
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2)
 {
     if (!knn2_tc_supported(nq, nt, dim)) { set_error("tcgen05 engine: unsupported shape nq=%d nt=%d dim=%d", nq, nt, dim); return ERP_E_DIM; }
-    const bool half = tc1_f16_operands();
-    const int kc = f_kc(half), kch = (dim + kc - 1) / kc, dpad = kch * kc, esize = half ? 2 : 4;
-    const int n_qpairs = cdiv(nq, F_BM * f_sub(kch)), n_ttiles = cdiv(nt, F_BN);
+    const int kch = cdiv(dim, F_KC), dpad = kch * F_KC;     // dim <= 128: one or two k chunks
+    const int n_qpairs = cdiv(nq, F_BM * F_SUB), n_ttiles = cdiv(nt, F_BN);
     // stream-K plan: equal contiguous unit ranges, a query pair cut in at most F_MAX_SEG segments
     long total = (long)n_qpairs * n_ttiles;
     long L = (total + ctx->sm_count - 1) / ctx->sm_count;
@@ -589,8 +510,8 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     const int n_lists = n_seg * F_EPI_GROUPS;
 
     int st = ERP_OK;
-    uint8_t* qs = ctx->scratch<uint8_t>(S_TC_Q, (size_t)nq * dpad * esize, &st);
-    uint8_t* ts = ctx->scratch<uint8_t>(S_TC_T, (size_t)nt * dpad * esize, &st);
+    __half* qs = ctx->scratch<__half>(S_TC_Q, (size_t)nq * dpad, &st);
+    __half* ts = ctx->scratch<__half>(S_TC_T, (size_t)nt * dpad, &st);
     float* tn = ctx->scratch<float>(S_TC_TN, (size_t)n_ttiles * F_BN * 9, &st);      // norms, then the 32-byte norm operand rows
     int32_t* cand = ctx->scratch<int32_t>(S_TC_CAND, (size_t)nq * n_lists * (F_TOPK * 2 + 1), &st);
     float* qn = ctx->scratch<float>(S_TC_QN, (size_t)nq + 8, &st);
@@ -608,38 +529,27 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     ERP_TRY(tc_misc_begin(ctx, misc));
     ERP_CUDA(cudaMemsetAsync(cand, 0xFF, (size_t)nq * n_lists * F_TOPK * sizeof(int32_t), ctx->stream));
 
-    float* aug = tn + (size_t)n_ttiles * F_BN;
+    __half* aug = reinterpret_cast<__half*>(tn + (size_t)n_ttiles * F_BN);
     RoundJob jq = {d_q, nq, -2.0f, qs, qn, nq, reinterpret_cast<unsigned*>(misc + 3), nullptr, 0};
-    RoundJob jt = {ctx->tc_chunk == 0 ? d_t : nullptr, nt, 1.0f, ts, tn, n_ttiles * F_BN, reinterpret_cast<unsigned*>(misc + 1),
-                   f_fold(kch) ? aug : nullptr, 0};
-    ERP_TRY(launch_prep(ctx, jq, jt, dim, dpad, half, reinterpret_cast<unsigned*>(misc + 5)));
+    RoundJob jt = {ctx->tc_chunk == 0 ? d_t : nullptr, nt, 1.0f, ts, tn, n_ttiles * F_BN, reinterpret_cast<unsigned*>(misc + 1), aug, 0};
+    ERP_TRY(launch_prep(ctx, jq, jt, dim, dpad, reinterpret_cast<unsigned*>(misc + 5)));
 
-    CUtensorMap mq, mt;
-    ERP_TRY(make_map(&mq, qs, nq, dpad, F_BM, false, half));
-    ERP_TRY(make_map(&mt, ts, nt, dpad, F_BN, false, half));
-    CUtensorMap ma = mt;
-    if (f_fold(kch)) ERP_TRY(make_map(&ma, aug, n_ttiles * F_BN, 32 / esize, F_BN, true, half));
+    CUtensorMap mq, mt, ma;
+    ERP_TRY(make_map(&mq, qs, nq, dpad, F_BM, false, true));
+    ERP_TRY(make_map(&mt, ts, nt, dpad, F_BN, false, true));
+    ERP_TRY(make_map(&ma, aug, n_ttiles * F_BN, 16, F_BN, true, true));     // 16 halves: one 32-byte row per train row
     Tc1Params p;
     p.nq = nq; p.nt = nt; p.n_qpairs = n_qpairs; p.n_ttiles = n_ttiles; p.units_per_cta = (int)L; p.n_seg = n_seg;
-    p.tn = tn; p.cand_idx = cand; p.cand_s = cand_s; p.cand_thr = cand_thr; p.qn = qn;
+    p.cand_idx = cand; p.cand_s = cand_s; p.cand_thr = cand_thr; p.qn = qn;
     p.tn_max_bits = reinterpret_cast<const unsigned*>(misc + 1);
     p.row_thr = row_thr;
 
     if (ctx->tc_chunk == 0) ERP_CUDA(record_timing(ctx, ctx->ev_k0));
-    if (half) {
-        if (kch == 1) ERP_TRY((launch_tc1<1, true>(ctx, mq, mt, ma, p, grid)));
-        else ERP_TRY((launch_tc1<2, true>(ctx, mq, mt, ma, p, grid)));
-    } else {
-        switch (kch) {
-        case 1: ERP_TRY((launch_tc1<1, false>(ctx, mq, mt, ma, p, grid))); break;
-        case 2: ERP_TRY((launch_tc1<2, false>(ctx, mq, mt, ma, p, grid))); break;
-        case 3: ERP_TRY((launch_tc1<3, false>(ctx, mq, mt, ma, p, grid))); break;
-        default: ERP_TRY((launch_tc1<4, false>(ctx, mq, mt, ma, p, grid))); break;
-        }
-    }
+    if (kch == 1) ERP_TRY(launch_tc1<1>(ctx, mq, mt, ma, p, grid));
+    else ERP_TRY(launch_tc1<2>(ctx, mq, mt, ma, p, grid));
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
 
-    ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, F_TOPK, F_KAPPA, half ? F_F16_ABS : -1.0, cand, cand_s, cand_thr,
+    ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, F_TOPK, F_KAPPA, F_F16_ABS, cand, cand_s, cand_thr,
                           reinterpret_cast<unsigned*>(misc),
                           d_idx2, d_dist2, d_d2, list));
     ERP_TRY(knn2_exact_rescan(ctx, d_q, nq, d_t, nt, dim, list, misc, nq, d_idx2, d_dist2, d_d2));

@@ -304,7 +304,7 @@ __device__ __forceinline__ void scan_chunk(const uint32_t (&v)[32], uint32_t tad
     }
 }
 
-// Candidate list of the 1xTF32 engine, 8 entries per (query row, list): [0], [1] = the two best scores so far in
+// Candidate list of the one-product engine (knn_tc1.cu), 8 entries per (query row, list): [0], [1] = the two best scores so far in
 // order (all the threshold needs), [2..7] = a FIFO of the other columns that were within the slack of the runner-up when
 // they arrived (newest first).  An entry pushed out of the FIFO lowers floor_thr to its score (and with it the threshold),
 // every other dropped column scored >= the threshold in force, so min(floor_thr, final threshold) bounds all
@@ -316,36 +316,28 @@ __device__ __forceinline__ void scan_chunk(const uint32_t (&v)[32], uint32_t tad
 // scan_chunk_lean: 32 accumulator columns of one query row, all in registers.  Common case: a min tree and ONE compare.
 // Rare case (per lane, no TMEM access, no warp-wide vote): the groups of 8 columns whose minimum is below the threshold are
 // selected out of the registers behind an opaque group id (so the compiler cannot specialise the code per group), packed,
-// and inserted smallest first.  With SHARE the threshold is also exchanged through shared memory with the thread that scans
-// the other column range of the same row; any published value is a valid bound, so a lost race only costs pruning.
-// With FOLD the accumulator already holds |t|^2 - 2 q.t (the norm entered the MMA as an extra k step).
+// and inserted smallest first.  The threshold is also exchanged through shared memory with the thread that scans the other
+// column range of the same row; any published value is a valid bound, so a lost race only costs pruning.
+// The accumulator already holds |t|^2 - 2 q.t (the norm entered the MMA as an extra k step).
 #if defined(ERP_TC_COUNTERS) && ERP_TC_COUNTERS == 2
 static __device__ unsigned long long erp_evt[8];
 #endif
-template <bool SHARE, bool FOLD>
-__device__ __forceinline__ void scan_chunk_lean(const uint32_t (&v)[32], const float4* __restrict__ tn4, int col0, float slack,
-                                                float (&bs)[8], int (&bi)[8], float* row_thr, float& floor_thr)
+__device__ __forceinline__ void scan_chunk_lean(const uint32_t (&v)[32], int col0, float slack, float (&bs)[8], int (&bi)[8],
+                                                float* row_thr, float& floor_thr)
 {
-    const float other = SHARE ? *reinterpret_cast<volatile float*>(row_thr) : INFINITY;
+    const float other = *reinterpret_cast<volatile float*>(row_thr);
     float gm[4];
 #pragma unroll
     for (int g = 0; g < 4; g++) {
         float s[8];
-        if (FOLD) {
 #pragma unroll
-            for (int j = 0; j < 8; j++) s[j] = __uint_as_float(v[g * 8 + j]);
-        } else {
-            const float4 na = tn4[g * 2], nb = tn4[g * 2 + 1];
-            const float nrm[8] = {na.x, na.y, na.z, na.w, nb.x, nb.y, nb.z, nb.w};
-#pragma unroll
-            for (int j = 0; j < 8; j++) s[j] = __fadd_rn(__uint_as_float(v[g * 8 + j]), nrm[j]);
-        }
+        for (int j = 0; j < 8; j++) s[j] = __uint_as_float(v[g * 8 + j]);
         gm[g] = fminf(fminf(fminf(s[0], s[1]), fminf(s[2], s[3])), fminf(fminf(s[4], s[5]), fminf(s[6], s[7])));
     }
     // floor_thr in the threshold is the capacity rule: once an entry has been pushed out, columns at or above its score
     // cannot improve the list's bound any more (all-equal scores would otherwise insert at every column)
     float thr = fminf(fminf(__fadd_rn(bs[1], slack), other), floor_thr);
-    if (SHARE) floor_thr = thr;
+    floor_thr = thr;
     if (fminf(fminf(gm[0], gm[1]), fminf(gm[2], gm[3])) < thr) {                                     // rare, per lane
         unsigned mine = (gm[0] < thr ? 1u : 0u) | (gm[1] < thr ? 2u : 0u) | (gm[2] < thr ? 4u : 0u) | (gm[3] < thr ? 8u : 0u);
 #if defined(ERP_TC_COUNTERS) && ERP_TC_COUNTERS == 2
@@ -357,11 +349,6 @@ __device__ __forceinline__ void scan_chunk_lean(const uint32_t (&v)[32], const f
             mine &= mine - 1;
             asm volatile("" : "+r"(g));
             const bool pl = (g & 1) != 0, ph = (g & 2) != 0;
-            float nrm[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-            if (!FOLD) {
-                const float4 na = tn4[g * 2], nb = tn4[g * 2 + 1];
-                nrm[0] = na.x; nrm[1] = na.y; nrm[2] = na.z; nrm[3] = na.w; nrm[4] = nb.x; nrm[5] = nb.y; nrm[6] = nb.z; nrm[7] = nb.w;
-            }
 #if defined(ERP_TC_COUNTERS) && ERP_TC_COUNTERS == 2
             atomicAdd(&erp_evt[5], 1ull);
 #endif
@@ -369,9 +356,8 @@ __device__ __forceinline__ void scan_chunk_lean(const uint32_t (&v)[32], const f
 #pragma unroll
             for (int j = 0; j < 8; j++) {
                 const uint32_t lo = pl ? v[8 + j] : v[j], hi = pl ? v[24 + j] : v[16 + j];
-                const float raw = __uint_as_float(ph ? hi : lo);
-                const float e = FOLD ? raw : __fadd_rn(raw, nrm[j]);
-                k[j] = __uint_as_float((__float_as_uint(e) & ~7u) | (uint32_t)j);
+                const uint32_t e = ph ? hi : lo;
+                k[j] = __uint_as_float((e & ~7u) | (uint32_t)j);
             }
             const int cbase = col0 + g * 8;
             for (;;) {
@@ -401,9 +387,7 @@ __device__ __forceinline__ void scan_chunk_lean(const uint32_t (&v)[32], const f
                 for (int j = 0; j < 8; j++) k[j] = k[j] == km ? INFINITY : k[j];
             }
         } while (mine);
-        if (SHARE) {
-            if (thr < *reinterpret_cast<volatile float*>(row_thr)) *reinterpret_cast<volatile float*>(row_thr) = thr;
-        }
+        if (thr < *reinterpret_cast<volatile float*>(row_thr)) *reinterpret_cast<volatile float*>(row_thr) = thr;
 #if defined(ERP_TC_COUNTERS) && ERP_TC_COUNTERS == 2
         const long long e1 = clock64();
         {

@@ -64,8 +64,8 @@ typedef enum {
     ERP_ENGINE_AUTO = 0,       /* the fastest exact engine for the shape: TCGEN05_1X for large problems, else SIMT */
     ERP_ENGINE_EXACT_SIMT = 1, /* fp64 direct-form brute force (also the rescan path)            */
     ERP_ENGINE_TCGEN05 = 2,    /* 3xTF32 GEMM-form tiles + fused top-4, exact fp64 refine + certificate  */
-    ERP_ENGINE_TCGEN05_1X = 3  /* one product of 11-bit operands (f16, or tf32 with ERP_B200_TC1_OPERANDS=tf32), top-8, same
-                                  certificate: 5 tensor instructions per tile at D = 64 where 3xTF32 issues 24 */
+    ERP_ENGINE_TCGEN05_1X = 3  /* one product of f16 operands (11 significant bits), top-8, same certificate:
+                                  5 tensor instructions per tile at D = 64 where 3xTF32 issues 24 */
 } erp_engine;
 
 /* operand format of the tensor products of a distance search (erp_ctx_last_knn_operands) */

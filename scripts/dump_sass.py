@@ -21,7 +21,7 @@ for line in txt.splitlines():
         continue
     if cur and re.match(r"\s+/\*[0-9a-f]{4,}\*/", line):
         kernels[cur].append(re.sub(r"\s*/\* 0x[0-9a-f]+ \*/\s*$", "", line).rstrip())
-FULL = {"knn2_tc_kernelILi2": "knn2_tc_kernel_D64.sass", "knn2_tc1_kernelILi2": "knn2_tc1_kernel_D64.sass", "knn2_tc1_kernelILi4": "knn2_tc1_kernel_D128.sass",
+FULL = {"knn2_tc_kernelILi2": "knn2_tc_kernel_D64.sass", "knn2_tc1_kernelILi1E": "knn2_tc1_kernel_D64.sass", "knn2_tc1_kernelILi2E": "knn2_tc1_kernel_D128.sass",
         "score_tc_kernel": "score_tc_kernel.sass", "min8_kernelILb0": "min8_kernel.sass", "refine_kernelILi2": "refine_kernel.sass",
         "score_list_kernel": "score_list_kernel.sass", "finish_kernelILi0": "finish_kernel.sass", "push_slots_kernel": "push_slots_kernel.sass",
         "xchg_best_kernel": "xchg_best_kernel.sass", "gather_slots_kernel": "gather_slots_kernel.sass", "argmax_plan_kernel": "argmax_plan_kernel.sass"}

@@ -161,7 +161,7 @@ def test_diagnostics(ctx):
     fq, ft, _ = synth.descriptor_pair(3000, 3000, 64, seed=1)
     ctx.set_engine(binding.ENGINE_TCGEN05_1X)
     ctx.knn2_raw(fq, ft)
-    assert ctx.last_knn_operands()["operands"] in (binding.OPERANDS_F16, binding.OPERANDS_TF32)
+    assert ctx.last_knn_operands()["operands"] == binding.OPERANDS_F16
     ctx.set_engine(binding.ENGINE_AUTO)
 
 
