@@ -430,13 +430,9 @@ ERP_API int erp_knn2_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_
     const bool forced = ctx->engine == ERP_ENGINE_TCGEN05 || ctx->engine == ERP_ENGINE_TCGEN05_1X;
     if (forced) ERP_ARG(knn2_tc_supported(nq, nt, dim), ERP_E_DIM, "tcgen05 engine does not support nq=%d nt=%d dim=%d", nq, nt, dim);
     if (ctx->engine == ERP_ENGINE_TCGEN05) return knn2_tc(ctx, d_q, nq, d_t, nt, dim, d_idx2, d_dist2, d_d2);
-    if (ctx->engine == ERP_ENGINE_TCGEN05_1X || (ctx->engine == ERP_ENGINE_AUTO && knn2_tc1_preferred(nq, nt, dim)))
+    if (ctx->engine == ERP_ENGINE_TCGEN05_1X || (ctx->engine == ERP_ENGINE_AUTO && knn2_tc_preferred(nq, nt, dim)))
         return knn2_tc1(ctx, d_q, nq, d_t, nt, dim, d_idx2, d_dist2, d_d2);
-    if (ctx->engine == ERP_ENGINE_AUTO && knn2_tc_preferred(nq, nt, dim))
-        return knn2_tc(ctx, d_q, nq, d_t, nt, dim, d_idx2, d_dist2, d_d2);
-    ctx->knn_stats[0] = ERP_ENGINE_EXACT_SIMT; ctx->knn_stats[1] = 0; ctx->knn_stats[2] = 1; ctx->knn_stats[3] = cdiv(nq, 64);
-    ctx->knn_stats[4] = 0;
-    ctx->knn_bin = false;
+    set_knn_stats(ctx, ERP_ENGINE_EXACT_SIMT, false, 1, cdiv(nq, 64), 0, nullptr);
     ERP_CUDA(record_timing(ctx, ctx->ev_k0));
     ERP_TRY(knn2_exact(ctx, d_q, nq, d_t, nt, dim, nullptr, 0, 0, d_idx2, d_dist2, d_d2));
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
@@ -474,8 +470,7 @@ ERP_API int erp_nn1_reverse_dev(erp_ctx* ctx, const float* d_q, int nq, const fl
     bool tc = nq >= 2 && (forced ? knn2_tc_supported(nt, nq, dim) : (ctx->engine == ERP_ENGINE_AUTO && knn2_tc_preferred(nt, nq, dim)));
     if (tc) {
         // (the tensor-core paths have no index offset: it is added while compacting)
-        if (ctx->engine == ERP_ENGINE_TCGEN05 || (ctx->engine == ERP_ENGINE_AUTO && !knn2_tc1_preferred(nt, nq, dim)))
-            ERP_TRY(knn2_tc(ctx, d_t, nt, d_q, nq, dim, idx2, nullptr, d2));
+        if (ctx->engine == ERP_ENGINE_TCGEN05) ERP_TRY(knn2_tc(ctx, d_t, nt, d_q, nq, dim, idx2, nullptr, d2));
         else ERP_TRY(knn2_tc1(ctx, d_t, nt, d_q, nq, dim, idx2, nullptr, d2));
     } else {
         ERP_TRY(knn2_exact(ctx, d_t, nt, d_q, nq, dim, nullptr, 0, 0, idx2, nullptr, d2));

@@ -160,6 +160,20 @@ inline int ensure_dynamic_smem(erp_ctx* ctx, Kernel kernel, int bytes, std::atom
     return ERP_OK;
 }
 
+// what erp_ctx_last_knn_stats and erp_ctx_last_knn_operands report about the last search: engine, binary rows, segments per
+// query row, units per CTA, grid; misc = the device words of a tcgen05 search that has a re-scan (its count is read from
+// there: knn_stats[1] = -1), null otherwise (nothing re-scanned: 0)
+inline void set_knn_stats(erp_ctx* ctx, int engine, bool bin, int n_seg, int units_per_cta, int grid, int32_t* misc)
+{
+    ctx->knn_stats[0] = engine;
+    ctx->knn_stats[1] = misc ? -1 : 0;
+    ctx->knn_stats[2] = n_seg;
+    ctx->knn_stats[3] = units_per_cta;
+    ctx->knn_stats[4] = grid;
+    ctx->knn_bin = bin;
+    ctx->tc_misc_dev = misc;
+}
+
 // timing events are recorded by the library on its own stream; inside a stream capture they become external event-record
 // nodes, so a replayed graph refreshes them like a direct call does
 inline cudaError_t record_timing(erp_ctx* ctx, cudaEvent_t ev)
@@ -188,7 +202,6 @@ int knn2_tc(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, in
             int32_t* d_idx2, float* d_dist2, double* d_d2);
 bool knn2_tc_supported(int nq, int nt, int dim);
 bool knn2_tc_preferred(int nq, int nt, int dim);
-bool knn2_tc1_preferred(int nq, int nt, int dim);
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2);
 bool knn2_bin_preferred(int nq, int nt);

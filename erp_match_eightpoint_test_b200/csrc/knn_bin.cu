@@ -4,8 +4,8 @@
 //     dot = n - 2 * Hamming
 // and one tcgen05.mma.kind::i8 GEMM (s8 x s8 -> s32) yields the EXACT distance in its accumulator: no norm step, no
 // rounding certificate, no refine or re-scan pass.  A kind::i8 instruction (K = 32) reads the same 32 bytes per operand
-// row as a kind::f16 K = 16 step, so the tile shape, smem descriptors, 128-byte swizzle, TMA ring and stream-K plan of
-// knn_tc1.cu carry over.  K padding is 0 on both sides and contributes nothing.
+// row as a kind::f16 K = 16 step, so the tile shape and the query-pair pipeline of knn_tc1.cu (tc_common.cuh: PairPipe)
+// carry over.  K padding is 0 on both sides and contributes nothing.
 //
 // Ties are the normal case for Hamming distances (a third of the queries of random 256-bit rows tie at the second
 // position), so every list is kept exactly in (H, trainIdx) order: the lowest index wins a tie everywhere.
@@ -60,17 +60,6 @@ bin_prep_kernel(const BinJob a, const BinJob b, int nbytes, int kpad)
     *reinterpret_cast<uint2*>(j.out + (size_t)row * kpad + 8 * k) = o;
 }
 
-// D[tmem] (+)= A[smem] * B[smem]^T, 128 x 256 x 32, s8 inputs, s32 accumulate
-__device__ __forceinline__ void tc_mma_i8(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
 struct BinParams {
     int nq, nt, nbits;
     int n_qpairs, n_ttiles;
@@ -113,6 +102,8 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     uint64_t* tempty = qfull + 4;       // [2] accumulator drained
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(qfull + 6);
     static_assert((2 * NS + 6) * 8 + 4 <= B_BARS, "barrier block");
+    static_assert(b_smem(KCH) <= TC_SMEM_LIMIT, "shared memory budget");
+    const PairPipe<SUB, KCH, NS, B_BM, B_BN, 128> pipe{q_smem, t_smem, full, empty, qfull, qempty, tfull, tempty};
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int W_ALLOC = B_EPI_THREADS / 32, W_TMA = W_ALLOC + 2, W_MMA = W_ALLOC + 3;   // W_ALLOC + 1 idles
@@ -124,80 +115,20 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         for (int i = 0; i < 2; i++) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], B_EPI_THREADS / 32); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == W_ALLOC) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     // the feeder warpgroup needs few registers; the eight epilogue warps take them over (128 accumulator columns in flight)
     if (warp >= W_ALLOC) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 56;" ::: "memory");
     if (warp == W_TMA) {
         // ================================================================ TMA producer
-        if (lane == 0) {
-            uint32_t slot = 0, ph = 0, seg_n = 0;
-            SegIter it(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x);
-            int qp, t0, t1, seg;
-            for (; it.next(qp, t0, t1, seg); seg_n++) {
-                mbar_wait(qempty, (seg_n & 1) ^ 1);
-                mbar_expect_tx(qfull, SUB * KCH * B_QCH);
-#pragma unroll
-                for (int sub = 0; sub < SUB; sub++)
-#pragma unroll
-                    for (int c = 0; c < KCH; c++)
-                        tma_load_2d(&map_q, qfull, q_smem + (sub * KCH + c) * B_QCH, c * 128, (qp * SUB + sub) * B_BM);
-                for (int tt = t0; tt < t1; tt++) {
-#pragma unroll
-                    for (int c = 0; c < KCH; c++) {
-                        mbar_wait(&empty[slot], ph ^ 1);
-                        mbar_expect_tx(&full[slot], B_TCH);
-                        tma_load_2d(&map_t, &full[slot], t_smem + slot * B_TCH, c * 128, tt * B_BN);
-                        if (++slot == NS) { slot = 0; ph ^= 1; }
-                    }
-                }
-            }
-        }
+        if (lane == 0) pipe.produce(&map_q, &map_t, SegIter(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x));
     } else if (warp == W_MMA) {
         // ================================================================ MMA issuer
-        if (lane == 0) {
-            uint32_t slot = 0, ph = 0, seg_n = 0, tile_n = 0;
-            const uint32_t q_base = smem_u32(q_smem), t_base = smem_u32(t_smem);
-            SegIter it(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x);
-            int qp, t0, t1, seg;
-            for (; it.next(qp, t0, t1, seg); seg_n++) {
-                mbar_wait(qfull, seg_n & 1);
-                for (int tt = t0; tt < t1; tt++) {
-                    // the KCH chunks of this train tile occupy KCH consecutive ring slots
-                    const uint32_t s0 = slot, p0 = ph;
-#pragma unroll
-                    for (int sub = 0; sub < SUB; sub++, tile_n++) {
-                        const uint32_t acc = tile_n & 1;
-                        mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
-                        const uint32_t d_tmem = tmem_base + acc * B_BN;
-                        uint32_t sl = s0, pp = p0;
-#pragma unroll
-                        for (int c = 0; c < KCH; c++) {
-                            if (sub == 0) mbar_wait(&full[sl], pp);
-                            tc_fence_after();
-                            const uint32_t a = q_base + (sub * KCH + c) * B_QCH, b = t_base + sl * B_TCH;
-                            // one instruction per 32 bytes of the 128-byte row: K = 32 int8
-#pragma unroll
-                            for (int k = 0; k < 4; k++)
-                                tc_mma_i8(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), B_IDESC_I8, (c | k) != 0);
-                            if (sub == SUB - 1) tc_commit(&empty[sl]);
-                            if (++sl == NS) { sl = 0; pp ^= 1; }
-                        }
-                        tc_commit(&tfull[acc]);
-                        if (sub == SUB - 1) { slot = sl; ph = pp; }
-                    }
-                }
-                tc_commit(qempty);
-            }
-        }
+        if (lane == 0)
+            pipe.issue(tmem_base, SegIter(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x),
+                       [](uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t accumulate) { tc_mma_i8(d_tmem, a, b, B_IDESC_I8, accumulate); },
+                       [](int, uint32_t, uint32_t) {});
     }
     } else {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 224;" ::: "memory");
@@ -220,20 +151,8 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                     mbar_wait(&tfull[acc], (tile_n >> 1) & 1);
                     tc_fence_after();
                     const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * B_BN + cg * B_EPI_COLS;
-                    // the warp's 128 columns go to registers at once and the accumulator is handed back before they are
-                    // examined: a slow insert path delays this warp's next read, not the next MMA
                     uint32_t va[32], vb[32], vc[32], vd[32];
-                    tc_ld32(taddr, va);
-                    tc_ld32(taddr + 32, vb);
-                    tc_ld32(taddr + 64, vc);
-                    tc_ld32(taddr + 96, vd);
-                    tc_wait_ld32(va);
-                    tc_wait_ld32(vb);
-                    tc_wait_ld32(vc);
-                    tc_wait_ld32(vd);
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&tempty[acc]);
+                    pipe.drain(taddr, acc, va, vb, vc, vd);
                     int m;
                     if (lim >= B_EPI_COLS) {
                         m = best_of32<false>(va, 0, 0, -1, INT_MIN);
@@ -275,12 +194,7 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         }
     }
 
-    tc_fence_before();
-    __syncthreads();
-    if (warp == W_ALLOC) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    tmem_free(warp == W_ALLOC, tmem_base);
 }
 
 // the n_lists x 2 keys of a query -> its two nearest in (distance, index) order
@@ -361,34 +275,6 @@ knn2_bin_exact_kernel(const uint8_t* __restrict__ q, int nq, const uint8_t* __re
     }
 }
 
-// rows x row_bytes uint8, box = one 128-byte swizzle row x box_rows, zero fill out of bounds
-static int make_map_u8(CUtensorMap* map, const void* base, int rows, int row_bytes, int box_rows)
-{
-    EncodeTiledFn fn = encode_fn();
-    if (!fn) { set_error("cuTensorMapEncodeTiled is not available from this driver"); return ERP_E_CUDA; }
-    cuuint64_t dims[2] = {(cuuint64_t)row_bytes, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
-    cuuint32_t box[2] = {128u, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d", (int)r); return ERP_E_CUDA; }
-    return ERP_OK;
-}
-
-template <int KCH>
-static int launch_bin(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt, const BinParams& p, int grid)
-{
-    constexpr int smem = b_smem(KCH);
-    static_assert(smem <= TC_SMEM_LIMIT, "shared memory budget");
-    static std::atomic<uint64_t> configured{0};
-    ERP_TRY(ensure_dynamic_smem(ctx, knn2_bin_kernel<KCH>, smem, configured));
-    knn2_bin_kernel<KCH><<<grid, B_THREADS, smem, ctx->stream>>>(mq, mt, p);
-    ERP_LAUNCH(ctx, "knn2_bin_kernel");
-    return ERP_OK;
-}
-
 // The kind::i8 engine is already 2.5x faster than SIMT at 1000 x 1000 x 32 B (DESIGN.md 4.8: 0.042 vs 0.103 ms per call,
 // B200); below 1e6 pairs, where nothing was measured, SIMT's single launch is kept.
 bool knn2_bin_preferred(int nq, int nt) { return (double)nq * (double)nt >= 1.0e6; }
@@ -396,12 +282,8 @@ bool knn2_bin_preferred(int nq, int nt) { return (double)nq * (double)nt >= 1.0e
 int knn2_bin(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, bool tc,
              int32_t* d_idx2, float* d_dist2, double* d_d2)
 {
-    ctx->knn_bin = true;
-    ctx->tc_misc_dev = nullptr;
-    ctx->knn_stats[1] = 0;
     if (!tc) {
-        ctx->knn_stats[0] = ERP_ENGINE_EXACT_SIMT; ctx->knn_stats[2] = 1; ctx->knn_stats[3] = cdiv(nq, BX_THREADS);
-        ctx->knn_stats[4] = 0;
+        set_knn_stats(ctx, ERP_ENGINE_EXACT_SIMT, true, 1, cdiv(nq, BX_THREADS), 0, nullptr);
         const int W = nbytes <= 8 ? 2 : nbytes <= 16 ? 4 : nbytes <= 32 ? 8 : 16;
         const int grid = cdiv(nq, BX_THREADS);
         if (ctx->tc_chunk == 0) ERP_CUDA(record_timing(ctx, ctx->ev_k0));
@@ -417,15 +299,8 @@ int knn2_bin(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     }
     const int kch = (nbytes + 15) / 16, kpad = kch * 128;
     const int n_qpairs = cdiv(nq, B_BM * b_sub(kch)), n_ttiles = cdiv(nt, B_BN);
-    // stream-K plan as knn2_tc1: equal contiguous unit ranges, a query pair cut in at most B_MAX_SEG segments
-    const long total = (long)n_qpairs * n_ttiles;
-    long L = (total + ctx->sm_count - 1) / ctx->sm_count;
-    const long lmin = (n_ttiles + (B_MAX_SEG - 2) - 1) / (B_MAX_SEG - 2);
-    if (L < lmin) L = lmin;
-    if (L < 1) L = 1;
-    const int grid = (int)((total + L - 1) / L);
-    const long segs = (n_ttiles + L - 1) / L + 1;
-    const int n_seg = (int)(segs > B_MAX_SEG ? B_MAX_SEG : segs);
+    const StreamK plan = stream_k_plan(n_qpairs, n_ttiles, ctx->sm_count, B_MAX_SEG);
+    const int n_seg = plan.n_seg;
     const int n_keys = n_seg * B_EPI_GROUPS * 2;
 
     int st = ERP_OK;
@@ -444,27 +319,24 @@ int knn2_bin(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int n
     ERP_LAUNCH(ctx, "bin_prep_kernel");
 
     CUtensorMap mq, mt;
-    ERP_TRY(make_map_u8(&mq, qs, nq, kpad, B_BM));
-    ERP_TRY(make_map_u8(&mt, ts, nt, kpad, B_BN));
+    ERP_TRY(make_map(&mq, qs, nq, kpad, B_BM, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1));
+    ERP_TRY(make_map(&mt, ts, nt, kpad, B_BN, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1));
     BinParams p;
-    p.nq = nq; p.nt = nt; p.nbits = 8 * nbytes; p.n_qpairs = n_qpairs; p.n_ttiles = n_ttiles; p.units_per_cta = (int)L;
+    p.nq = nq; p.nt = nt; p.nbits = 8 * nbytes; p.n_qpairs = n_qpairs; p.n_ttiles = n_ttiles; p.units_per_cta = plan.units_per_cta;
     p.n_seg = n_seg; p.cand = cand;
 
     if (ctx->tc_chunk == 0) ERP_CUDA(record_timing(ctx, ctx->ev_k0));
     switch (kch) {
-    case 1: ERP_TRY(launch_bin<1>(ctx, mq, mt, p, grid)); break;
-    case 2: ERP_TRY(launch_bin<2>(ctx, mq, mt, p, grid)); break;
-    case 3: ERP_TRY(launch_bin<3>(ctx, mq, mt, p, grid)); break;
-    default: ERP_TRY(launch_bin<4>(ctx, mq, mt, p, grid)); break;
+    case 1: ERP_TRY(launch_tc_kernel<knn2_bin_kernel<1>>(ctx, "knn2_bin_kernel", plan.grid, B_THREADS, b_smem(1), mq, mt, p)); break;
+    case 2: ERP_TRY(launch_tc_kernel<knn2_bin_kernel<2>>(ctx, "knn2_bin_kernel", plan.grid, B_THREADS, b_smem(2), mq, mt, p)); break;
+    case 3: ERP_TRY(launch_tc_kernel<knn2_bin_kernel<3>>(ctx, "knn2_bin_kernel", plan.grid, B_THREADS, b_smem(3), mq, mt, p)); break;
+    default: ERP_TRY(launch_tc_kernel<knn2_bin_kernel<4>>(ctx, "knn2_bin_kernel", plan.grid, B_THREADS, b_smem(4), mq, mt, p)); break;
     }
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
     bin_merge_kernel<<<cdiv(nq, 256), 256, 0, ctx->stream>>>(cand, nq, n_keys, d_idx2, d_dist2, d_d2);
     ERP_LAUNCH(ctx, "bin_merge_kernel");
 
-    ctx->knn_stats[0] = ERP_ENGINE_TCGEN05_1X;
-    ctx->knn_stats[2] = n_seg;
-    ctx->knn_stats[3] = (int)L;
-    ctx->knn_stats[4] = grid;
+    set_knn_stats(ctx, ERP_ENGINE_TCGEN05_1X, true, n_seg, plan.units_per_cta, plan.grid, nullptr);
     return ERP_OK;
 }
 

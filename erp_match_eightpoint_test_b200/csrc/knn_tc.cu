@@ -49,6 +49,7 @@ constexpr int SMEM_TAIL = 2 * BN * 4 + 256;     // |t|^2 of two tiles + mbarrier
 constexpr double KAPPA = 1.0 / 16384.0;
 
 __host__ __device__ constexpr int n_slots(int kch) { return (SMEM_LIMIT - 2 * kch * Q_CHUNK_BYTES - SMEM_TAIL) / T_CHUNK_BYTES; }
+__host__ __device__ constexpr int tc_smem(int kch) { return 2 * kch * Q_CHUNK_BYTES + n_slots(kch) * T_CHUNK_BYTES + SMEM_TAIL; }
 
 constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 
@@ -130,6 +131,7 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
 {
     constexpr int NS = n_slots(KCH);
     static_assert(NS >= 2, "T ring too small");
+    static_assert(tc_smem(KCH) <= SMEM_LIMIT, "shared memory budget");
     extern __shared__ __align__(1024) uint8_t smem[];
     // the 128B swizzle atoms need a 1024-byte aligned base; the budget has no room for a round-up
     if ((smem_u32(smem) & 1023u) != 0) __trap();
@@ -161,14 +163,7 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
         for (int i = 0; i < 2; i++) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], EPI_THREADS / 32); mbar_init(&nfull[i], 1); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == W_ALLOC) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     if (warp == W_TMA) {
         // ================================================================ TMA producer
@@ -310,13 +305,7 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
         }
     }
 
-    // ---- teardown
-    tc_fence_before();
-    __syncthreads();
-    if (warp == W_ALLOC) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    tmem_free(warp == W_ALLOC, tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -514,47 +503,12 @@ int refine_launch(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int 
 
 bool knn2_tc_supported(int nq, int nt, int dim) { return nq >= 1 && nt >= 2 && dim >= 4 && dim % 4 == 0 && dim <= 128; }
 
-// AUTO policy: tensor cores once the problem is large enough to amortise the extra passes; the
-// one-product engine (knn_tc1.cu) from 2e9 dist-evals (below that its paired tiles leave SMs idle)
+// AUTO policy: tensor cores once the problem is large enough to amortise the extra passes, and then the one-product
+// engine (knn_tc1.cu), measured faster than 3xTF32 at every size where a tensor engine pays at all
+// (20k x 20k x 64: 0.14 vs 0.27 ms, 50k x 50k: 0.54 vs 1.20 ms, 100k x 100k: 1.7 vs 4.2 ms)
 bool knn2_tc_preferred(int nq, int nt, int dim)
 {
     return knn2_tc_supported(nq, nt, dim) && (double)nq * (double)nt >= 4.0e6;
-}
-// the 1xTF32 engine: measured faster than 3xTF32 at every size where a tensor engine pays at all
-// (20k x 20k x 64: 0.14 vs 0.27 ms, 50k x 50k: 0.54 vs 1.20 ms, 100k x 100k: 1.7 vs 4.2 ms)
-bool knn2_tc1_preferred(int nq, int nt, int dim)
-{
-    return knn2_tc_supported(nq, nt, dim) && (double)nq * (double)nt >= 4.0e6;
-}
-
-// Stream-K style plan: the n_qtiles x n_ttiles unit grid (query tile major) is cut into equal
-// contiguous ranges, one per CTA.  A query tile may be cut into at most MAX_SEG segments (each
-// writes its own candidate lists), which bounds the range length from below for small nq.
-static void plan(int n_qtiles, int n_ttiles, int sms, int* units_per_cta, int* n_seg, int* grid)
-{
-    long total = (long)n_qtiles * n_ttiles;
-    long L = (total + sms - 1) / sms;
-    long lmin = MAX_SEG > 2 ? (n_ttiles + (MAX_SEG - 2) - 1) / (MAX_SEG - 2) : n_ttiles;   // <= MAX_SEG-2 interior cuts + 1
-    if (L < lmin) L = lmin;
-    if (L < 1) L = 1;
-    *units_per_cta = (int)L;
-    *grid = (int)((total + L - 1) / L);
-    long cuts = (n_ttiles + L - 1) / L;            // multiples of L strictly inside one row: at most this many
-    long segs = cuts + 1;
-    *n_seg = (int)(segs > MAX_SEG ? MAX_SEG : segs);
-}
-
-template <int KCH>
-static int launch_tc(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt, const TcParams& p, int grid)
-{
-    constexpr int NS = n_slots(KCH);
-    constexpr int smem = 2 * KCH * Q_CHUNK_BYTES + NS * T_CHUNK_BYTES + SMEM_TAIL;
-    static_assert(smem <= SMEM_LIMIT, "shared memory budget");
-    static std::atomic<uint64_t> configured{0};
-    ERP_TRY(ensure_dynamic_smem(ctx, knn2_tc_kernel<KCH>, smem, configured));
-    knn2_tc_kernel<KCH><<<grid, TC_THREADS, smem, ctx->stream>>>(mq, mt, p);
-    ERP_LAUNCH(ctx, "knn2_tc_kernel");
-    return ERP_OK;
 }
 
 int knn2_exact_rescan(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
@@ -567,9 +521,8 @@ int knn2_tc(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, in
     if (!knn2_tc_supported(nq, nt, dim)) { set_error("tcgen05 engine: unsupported shape nq=%d nt=%d dim=%d", nq, nt, dim); return ERP_E_DIM; }
     const int kch = (dim + KC - 1) / KC, dpad = kch * KC;
     const int n_qtiles = cdiv(nq, BM), n_ttiles = cdiv(nt, BN);
-    int upc, n_seg, grid;
-    plan(n_qtiles, n_ttiles, ctx->sm_count, &upc, &n_seg, &grid);
-    const int n_lists = n_seg * EPI_GROUPS;
+    const StreamK plan = stream_k_plan(n_qtiles, n_ttiles, ctx->sm_count, MAX_SEG);
+    const int n_seg = plan.n_seg, n_lists = n_seg * EPI_GROUPS;
 
     int st = ERP_OK;
     float* qs = ctx->scratch<float>(S_TC_Q, (size_t)nq * 2 * dpad, &st);
@@ -590,19 +543,19 @@ int knn2_tc(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, in
     if (ctx->tc_chunk == 0) ERP_TRY(launch_prep(ctx, d_t, nt, dim, dpad, 1.0f, ts, tn, n_ttiles * BN, reinterpret_cast<unsigned*>(misc + 1)));
 
     CUtensorMap mq, mt;
-    ERP_TRY(make_map(&mq, qs, nq, 2 * dpad, BM));
-    ERP_TRY(make_map(&mt, ts, nt, 2 * dpad, BN));
+    ERP_TRY(make_map(&mq, qs, nq, 2 * dpad, BM, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4));
+    ERP_TRY(make_map(&mt, ts, nt, 2 * dpad, BN, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4));
     TcParams p;
-    p.nq = nq; p.nt = nt; p.n_qtiles = n_qtiles; p.n_ttiles = n_ttiles; p.units_per_cta = upc; p.n_seg = n_seg;
+    p.nq = nq; p.nt = nt; p.n_qtiles = n_qtiles; p.n_ttiles = n_ttiles; p.units_per_cta = plan.units_per_cta; p.n_seg = n_seg;
     p.tn = tn; p.cand_idx = cand; p.cand_s = cand_s; p.cand_thr = cand_thr; p.qn = qn;
     p.tn_max_bits = reinterpret_cast<const unsigned*>(misc + 1);
 
     if (ctx->tc_chunk == 0) ERP_CUDA(record_timing(ctx, ctx->ev_k0));
     switch (kch) {
-    case 1: ERP_TRY(launch_tc<1>(ctx, mq, mt, p, grid)); break;
-    case 2: ERP_TRY(launch_tc<2>(ctx, mq, mt, p, grid)); break;
-    case 3: ERP_TRY(launch_tc<3>(ctx, mq, mt, p, grid)); break;
-    default: ERP_TRY(launch_tc<4>(ctx, mq, mt, p, grid)); break;
+    case 1: ERP_TRY(launch_tc_kernel<knn2_tc_kernel<1>>(ctx, "knn2_tc_kernel", plan.grid, TC_THREADS, tc_smem(1), mq, mt, p)); break;
+    case 2: ERP_TRY(launch_tc_kernel<knn2_tc_kernel<2>>(ctx, "knn2_tc_kernel", plan.grid, TC_THREADS, tc_smem(2), mq, mt, p)); break;
+    case 3: ERP_TRY(launch_tc_kernel<knn2_tc_kernel<3>>(ctx, "knn2_tc_kernel", plan.grid, TC_THREADS, tc_smem(3), mq, mt, p)); break;
+    default: ERP_TRY(launch_tc_kernel<knn2_tc_kernel<4>>(ctx, "knn2_tc_kernel", plan.grid, TC_THREADS, tc_smem(4), mq, mt, p)); break;
     }
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
 
@@ -611,13 +564,7 @@ int knn2_tc(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, in
     ERP_TRY(knn2_exact_rescan(ctx, d_q, nq, d_t, nt, dim, list, misc, nq, d_idx2, d_dist2, d_d2));
     ERP_TRY(tc_misc_end(ctx, misc));
 
-    ctx->knn_stats[0] = ERP_ENGINE_TCGEN05;
-    ctx->knn_bin = false;
-    ctx->knn_stats[1] = -1;                       // re-scan count lives on the device: see erp_ctx_last_knn_stats
-    ctx->knn_stats[2] = n_seg;
-    ctx->knn_stats[3] = upc;
-    ctx->knn_stats[4] = grid;
-    ctx->tc_misc_dev = misc;
+    set_knn_stats(ctx, ERP_ENGINE_TCGEN05, false, n_seg, plan.units_per_cta, plan.grid, misc);
     return ERP_OK;
 }
 

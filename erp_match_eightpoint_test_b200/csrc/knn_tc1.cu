@@ -34,23 +34,6 @@ constexpr int F_MAX_SEG = 128 / (F_TOPK * F_EPI_GROUPS);    // up to 8 segments 
 constexpr int F_AUG_T = F_BN * 32;        // 8 KB: one extra k step (16 halves) per train row, 32-byte swizzle rows
 constexpr int F_AUG_Q = F_BM * 32;        // 4 KB: the constant query side of that k step
 constexpr int F_BARS = 256;               // mbarriers + TMEM slot
-// Instrumented builds (scripts/build_variant.sh N): -DERP_TC_COUNTERS=1 adds clock64 phase timers to the MMA issuer and the
-// epilogue warps, =2 counts and times the insert path (tc_common.cuh); both print after every launch.  Off by default.
-#ifndef ERP_TC_COUNTERS
-#define ERP_TC_COUNTERS 0
-#endif
-#if ERP_TC_COUNTERS == 1
-static __device__ unsigned long long erp_clk[8];
-#define TCC_DECL unsigned long long lclk[6] = {0, 0, 0, 0, 0, 0}
-#define TCC_CLOCK(name) const long long name = clock64()
-#define TCC_ADD(i, v) (lclk[i] += (unsigned long long)(v))
-#define TCC_FLUSH() do { if ((threadIdx.x & 31) == 0) for (int i_ = 0; i_ < 6; i_++) if (lclk[i_]) atomicAdd(&erp_clk[i_], lclk[i_]); } while (0)
-#else
-#define TCC_DECL
-#define TCC_CLOCK(name)
-#define TCC_ADD(i, v)
-#define TCC_FLUSH()
-#endif
 // |s_tc - s_exact| <= 2^-10 (|q|^2 + max|t|^2) in the worst case: both operands are rounded to 11
 // significant bits (relative error 2^-11 each, f16 rounds to nearest even), products are exact (11 x 11 bits fit fp32,
 // and so do f16 subnormal products), and 2|q||t| <= |q|^2 + |t|^2.
@@ -215,6 +198,8 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     float* thr_sh = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + F_BARS);   // [F_SUB][F_BM] row thresholds
     static_assert(F_SUB * KCH * F_QCH + NS * F_TCH + 2 * F_AUG_T + F_AUG_Q + F_BARS + F_SUB * F_BM * 4 <= f_smem(KCH),
                   "threshold exchange area");
+    static_assert(f_smem(KCH) <= TC_SMEM_LIMIT, "shared memory budget");
+    const PairPipe<F_SUB, KCH, NS, F_BM, F_BN, F_KC> pipe{q_smem, t_smem, full, empty, qfull, qempty, tfull, tempty};
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     TCC_DECL;
@@ -230,95 +215,32 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == W_ALLOC) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
     // query side of the norm step: the same 8 halves in both 16-byte halves of every row, which the swizzle cannot change
     for (int i = threadIdx.x; i < F_AUG_Q / 2; i += F_THREADS)
         reinterpret_cast<__half*>(aug_q)[i] = __float2half_rn(f16_norm_scale(i & 7));
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     // the four feeder warps need few registers; the eight epilogue warps take them over (4 chunks of 32 accumulator columns in flight)
     if (warp >= W_ALLOC) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 56;" ::: "memory");
     if (warp == W_TMA) {
         // ================================================================ TMA producer
-        if (lane == 0) {
-            uint32_t slot = 0, ph = 0, seg_n = 0;
-            SegIter it(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x);
-            int qp, t0, t1, seg;
-            for (; it.next(qp, t0, t1, seg); seg_n++) {
-                mbar_wait(qempty, (seg_n & 1) ^ 1);
-                mbar_expect_tx(qfull, F_SUB * KCH * F_QCH);
-#pragma unroll
-                for (int sub = 0; sub < F_SUB; sub++)
-#pragma unroll
-                    for (int c = 0; c < KCH; c++)
-                        tma_load_2d(&map_q, qfull, q_smem + (sub * KCH + c) * F_QCH, c * F_KC, (qp * F_SUB + sub) * F_BM);
-                for (int tt = t0; tt < t1; tt++) {
-#pragma unroll
-                    for (int c = 0; c < KCH; c++) {
-                        mbar_wait(&empty[slot], ph ^ 1);
-                        mbar_expect_tx(&full[slot], F_TCH);
-                        tma_load_2d(&map_t, &full[slot], t_smem + slot * F_TCH, c * F_KC, tt * F_BN);
-                        if (++slot == NS) { slot = 0; ph ^= 1; }
-                    }
-                }
-            }
-        }
+        if (lane == 0) pipe.produce(&map_q, &map_t, SegIter(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x));
     } else if (warp == W_MMA) {
         // ================================================================ MMA issuer
         if (lane == 0) {
-            uint32_t slot = 0, ph = 0, seg_n = 0, tile_n = 0;
-            const uint32_t q_base = smem_u32(q_smem), t_base = smem_u32(t_smem);
             const uint64_t aq_desc = smem_desc_sw32(smem_u32(aug_q));
-            uint32_t tt_n = 0;
-            SegIter it(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x);
-            int qp, t0, t1, seg;
-            for (; it.next(qp, t0, t1, seg); seg_n++) {
-                mbar_wait(qfull, seg_n & 1);
-                for (int tt = t0; tt < t1; tt++, tt_n++) {
-                    // the KCH chunks of this train tile occupy KCH consecutive ring slots
-                    uint32_t s0 = slot, p0 = ph;
-#pragma unroll
-                    for (int sub = 0; sub < F_SUB; sub++, tile_n++) {
-                        const uint32_t acc = tile_n & 1;
-                        TCC_CLOCK(m0);
-                        mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
-                        TCC_ADD(3, clock64() - m0); TCC_ADD(4, 1);
-                        const uint32_t d_tmem = tmem_base + acc * F_BN;
-                        uint32_t sl = s0, pp = p0;
-#pragma unroll
-                        for (int c = 0; c < KCH; c++) {
-                            TCC_CLOCK(f0);
-                            if (sub == 0) mbar_wait(&full[sl], pp);
-                            TCC_ADD(5, clock64() - f0);
-                            tc_fence_after();
-                            const uint32_t a = q_base + (sub * KCH + c) * F_QCH, b = t_base + sl * F_TCH;
-                            // one instruction per 32 bytes of the 128-byte row: K = 16 halves
-#pragma unroll
-                            for (int k = 0; k < 4; k++)
-                                tc_mma_f16(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), F_IDESC, (c | k) != 0);
-                            if (sub == F_SUB - 1) tc_commit(&empty[sl]);
-                            if (++sl == NS) { sl = 0; pp ^= 1; }
-                        }
-                        // the norm step
-                        const uint32_t nb = tt_n & 1;
-                        if (sub == 0) mbar_wait(&nfull[nb], (tt_n >> 1) & 1);
-                        tc_fence_after();
-                        tc_mma_f16(d_tmem, aq_desc, smem_desc_sw32(smem_u32(aug_t + nb * F_AUG_T)), F_IDESC, 1);
-                        if (sub == F_SUB - 1) tc_commit(&nempty[nb]);
-                        tc_commit(&tfull[acc]);
-                        if (sub == F_SUB - 1) { slot = sl; ph = pp; }
-                    }
-                }
-                tc_commit(qempty);
-            }
+            pipe.issue(tmem_base, SegIter(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x),
+                       [](uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t accumulate) { tc_mma_f16(d_tmem, a, b, F_IDESC, accumulate); },
+                       [&](int sub, uint32_t tt_n, uint32_t d_tmem) {
+                           // the norm step
+                           const uint32_t nb = tt_n & 1;
+                           if (sub == 0) mbar_wait(&nfull[nb], (tt_n >> 1) & 1);
+                           tc_fence_after();
+                           tc_mma_f16(d_tmem, aq_desc, smem_desc_sw32(smem_u32(aug_t + nb * F_AUG_T)), F_IDESC, 1);
+                           if (sub == F_SUB - 1) tc_commit(&nempty[nb]);
+                       });
         }
     } else if (warp == W_NORM) {
         // ================================================================ norm operand producer (one TMA load per train tile)
@@ -399,22 +321,10 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                     TCC_CLOCK(c1);
                     tc_fence_after();
                     const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * F_BN + cg * F_EPI_COLS;
-                    // all four chunks of this warp's share go to registers at once (the epilogue warps hold 224 registers, see
-                    // setmaxnreg above), the accumulator is handed back, and only then are the columns examined: a slow insert
-                    // path delays this warp's next read, not the next MMA
+                    // all four chunks of this warp's share in registers at once: the epilogue warps hold 224 (setmaxnreg above)
                     static_assert(F_EPI_COLS == 128, "four chunks of 32 columns per warp and tile");
                     uint32_t va[32], vb[32], vc[32], vd[32];
-                    tc_ld32(taddr, va);
-                    tc_ld32(taddr + 32, vb);
-                    tc_ld32(taddr + 64, vc);
-                    tc_ld32(taddr + 96, vd);
-                    tc_wait_ld32(va);
-                    tc_wait_ld32(vb);
-                    tc_wait_ld32(vc);
-                    tc_wait_ld32(vd);
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&tempty[acc]);
+                    pipe.drain(taddr, acc, va, vb, vc, vd);
                     scan_chunk_lean(va, colbase, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
                     scan_chunk_lean(vb, colbase + 32, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
                     scan_chunk_lean(vc, colbase + 64, slack[sub], bs[sub], bi[sub], thr_sh + sub * F_BM + row, floor_thr[sub]);
@@ -452,12 +362,7 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     }
 
     TCC_FLUSH();
-    tc_fence_before();
-    __syncthreads();
-    if (warp == W_ALLOC) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    tmem_free(warp == W_ALLOC, tmem_base);
 }
 
 #if ERP_TC_COUNTERS == 2
@@ -476,38 +381,14 @@ __global__ void dbg_print_kernel()
     for (int i = 0; i < 8; i++) erp_clk[i] = 0;
 }
 #endif
-template <int KCH>
-static int launch_tc1(erp_ctx* ctx, const CUtensorMap& mq, const CUtensorMap& mt, const CUtensorMap& ma, const Tc1Params& p, int grid)
-{
-    constexpr int smem = f_smem(KCH);
-    static_assert(smem <= TC_SMEM_LIMIT, "shared memory budget");
-    static std::atomic<uint64_t> configured{0};
-    ERP_TRY(ensure_dynamic_smem(ctx, knn2_tc1_kernel<KCH>, smem, configured));
-    knn2_tc1_kernel<KCH><<<grid, F_THREADS, smem, ctx->stream>>>(mq, mt, ma, p);
-    ERP_LAUNCH(ctx, "knn2_tc1_kernel");
-#if ERP_TC_COUNTERS
-    dbg_print_kernel<<<1, 1, 0, ctx->stream>>>();
-    cudaStreamSynchronize(ctx->stream);
-#endif
-    return ERP_OK;
-}
-
 int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
              int32_t* d_idx2, float* d_dist2, double* d_d2)
 {
     if (!knn2_tc_supported(nq, nt, dim)) { set_error("tcgen05 engine: unsupported shape nq=%d nt=%d dim=%d", nq, nt, dim); return ERP_E_DIM; }
     const int kch = cdiv(dim, F_KC), dpad = kch * F_KC;     // dim <= 128: one or two k chunks
     const int n_qpairs = cdiv(nq, F_BM * F_SUB), n_ttiles = cdiv(nt, F_BN);
-    // stream-K plan: equal contiguous unit ranges, a query pair cut in at most F_MAX_SEG segments
-    long total = (long)n_qpairs * n_ttiles;
-    long L = (total + ctx->sm_count - 1) / ctx->sm_count;
-    long lmin = (n_ttiles + (F_MAX_SEG - 2) - 1) / (F_MAX_SEG - 2);
-    if (L < lmin) L = lmin;
-    if (L < 1) L = 1;
-    const int grid = (int)((total + L - 1) / L);
-    long segs = (n_ttiles + L - 1) / L + 1;
-    const int n_seg = (int)(segs > F_MAX_SEG ? F_MAX_SEG : segs);
-    const int n_lists = n_seg * F_EPI_GROUPS;
+    const StreamK plan = stream_k_plan(n_qpairs, n_ttiles, ctx->sm_count, F_MAX_SEG);
+    const int n_seg = plan.n_seg, n_lists = n_seg * F_EPI_GROUPS;
 
     int st = ERP_OK;
     __half* qs = ctx->scratch<__half>(S_TC_Q, (size_t)nq * dpad, &st);
@@ -535,18 +416,22 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     ERP_TRY(launch_prep(ctx, jq, jt, dim, dpad, reinterpret_cast<unsigned*>(misc + 5)));
 
     CUtensorMap mq, mt, ma;
-    ERP_TRY(make_map(&mq, qs, nq, dpad, F_BM, false, true));
-    ERP_TRY(make_map(&mt, ts, nt, dpad, F_BN, false, true));
-    ERP_TRY(make_map(&ma, aug, n_ttiles * F_BN, 16, F_BN, true, true));     // 16 halves: one 32-byte row per train row
+    ERP_TRY(make_map(&mq, qs, nq, dpad, F_BM, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2));
+    ERP_TRY(make_map(&mt, ts, nt, dpad, F_BN, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2));
+    ERP_TRY(make_map(&ma, aug, n_ttiles * F_BN, 16, F_BN, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, true));     // 16 halves: one 32-byte row per train row
     Tc1Params p;
-    p.nq = nq; p.nt = nt; p.n_qpairs = n_qpairs; p.n_ttiles = n_ttiles; p.units_per_cta = (int)L; p.n_seg = n_seg;
+    p.nq = nq; p.nt = nt; p.n_qpairs = n_qpairs; p.n_ttiles = n_ttiles; p.units_per_cta = plan.units_per_cta; p.n_seg = n_seg;
     p.cand_idx = cand; p.cand_s = cand_s; p.cand_thr = cand_thr; p.qn = qn;
     p.tn_max_bits = reinterpret_cast<const unsigned*>(misc + 1);
     p.row_thr = row_thr;
 
     if (ctx->tc_chunk == 0) ERP_CUDA(record_timing(ctx, ctx->ev_k0));
-    if (kch == 1) ERP_TRY(launch_tc1<1>(ctx, mq, mt, ma, p, grid));
-    else ERP_TRY(launch_tc1<2>(ctx, mq, mt, ma, p, grid));
+    if (kch == 1) ERP_TRY(launch_tc_kernel<knn2_tc1_kernel<1>>(ctx, "knn2_tc1_kernel", plan.grid, F_THREADS, f_smem(1), mq, mt, ma, p));
+    else ERP_TRY(launch_tc_kernel<knn2_tc1_kernel<2>>(ctx, "knn2_tc1_kernel", plan.grid, F_THREADS, f_smem(2), mq, mt, ma, p));
+#if ERP_TC_COUNTERS
+    dbg_print_kernel<<<1, 1, 0, ctx->stream>>>();
+    cudaStreamSynchronize(ctx->stream);
+#endif
     ERP_CUDA(record_timing(ctx, ctx->ev_k1));
 
     ERP_TRY(refine_launch(ctx, d_q, nq, d_t, nt, dim, n_lists, F_TOPK, F_KAPPA, F_F16_ABS, cand, cand_s, cand_thr,
@@ -555,13 +440,7 @@ int knn2_tc1(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, i
     ERP_TRY(knn2_exact_rescan(ctx, d_q, nq, d_t, nt, dim, list, misc, nq, d_idx2, d_dist2, d_d2));
     ERP_TRY(tc_misc_end(ctx, misc));
 
-    ctx->knn_stats[0] = ERP_ENGINE_TCGEN05_1X;
-    ctx->knn_bin = false;
-    ctx->knn_stats[1] = -1;
-    ctx->knn_stats[2] = n_seg;
-    ctx->knn_stats[3] = (int)L;
-    ctx->knn_stats[4] = grid;
-    ctx->tc_misc_dev = misc;
+    set_knn_stats(ctx, ERP_ENGINE_TCGEN05_1X, false, n_seg, plan.units_per_cta, plan.grid, misc);
     return ERP_OK;
 }
 

@@ -165,14 +165,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == W_ALLOC) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     // the four feeder warps need few registers; the eight epilogue warps take them over (128 accumulator columns in flight)
     if (warp >= W_ALLOC) {
@@ -318,12 +311,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
         }
     }
 
-    tc_fence_before();
-    __syncthreads();
-    if (warp == W_ALLOC) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    tmem_free(warp == W_ALLOC, tmem_base);
 }
 
 // ---- the small kernels between the passes ------------------------------------------------------
@@ -464,12 +452,9 @@ bool score_tc_preferred(int H, int m) { return (double)H * (double)m >= 3.0e7 &&
 
 static int launch_score_tc(erp_ctx* ctx, const CUtensorMap& me, const CUtensorMap& mk, const ScoreTcParams& p)
 {
-    static std::atomic<uint64_t> configured{0};
-    ERP_TRY(ensure_dynamic_smem(ctx, score_tc_kernel, S_SMEM, configured));
     cudaEvent_t e0, e1;
     ERP_TRY(score_event(ctx, &e0));
-    score_tc_kernel<<<ctx->sm_count, S_THREADS, S_SMEM, ctx->stream>>>(me, mk, p);
-    ERP_LAUNCH(ctx, "score_tc_kernel");
+    ERP_TRY(launch_tc_kernel<score_tc_kernel>(ctx, "score_tc_kernel", ctx->sm_count, S_THREADS, S_SMEM, me, mk, p));
     ERP_TRY(score_event(ctx, &e1));
     return ERP_OK;
 }
@@ -524,9 +509,9 @@ int score_tc_search(erp_ctx* ctx, const ScoreTcBuffers& b, const double* d_E, in
         ERP_LAUNCH(ctx, "prep_e_kernel");
     }
     CUtensorMap me, me2, mk;
-    ERP_TRY(make_map(&me, b.Es, H, 32, SM_ROWS));
-    ERP_TRY(make_map(&me2, b.Es2, H, 32, SM_ROWS));
-    ERP_TRY(make_map(&mk, b.Ks, m_cap, 32, SN_ROWS));
+    ERP_TRY(make_map(&me, b.Es, H, 32, SM_ROWS, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4));
+    ERP_TRY(make_map(&me2, b.Es2, H, 32, SM_ROWS, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4));
+    ERP_TRY(make_map(&mk, b.Ks, m_cap, 32, SN_ROWS, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4));
     ScoreTcParams p;
     p.tau = tau; p.big = big; p.kmax_bits = (const unsigned*)(w + W_KMAX);
 

@@ -1,5 +1,7 @@
-// tc_common.cuh -- inline-PTX wrappers (mbarrier, TMA, tcgen05 / TMEM) and the tensor-map encoder
-// shared by the two tcgen05 kernels (knn_tc.cu: distances, score_tc.cu: residuals).
+// tc_common.cuh -- what the tcgen05 kernels share (knn_tc.cu and knn_tc1.cu: distances, knn_bin.cu: Hamming distances,
+// score_tc.cu: residuals): inline-PTX wrappers (mbarrier, TMA, tcgen05 / TMEM), TMEM allocation, the tensor-map encoder,
+// the stream-K planner and the launcher; and the query-pair pipeline (TMA producer, MMA ring walk, accumulator drain) of
+// knn_tc1.cu and knn_bin.cu.
 #pragma once
 
 #include "common.cuh"
@@ -83,6 +85,16 @@ __device__ __forceinline__ void tc_mma_f16(uint32_t d_tmem, uint64_t a_desc, uin
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// D[tmem] (+)= A[smem] * B[smem]^T, 128 x 256 x 32, s8 inputs, s32 accumulate
+__device__ __forceinline__ void tc_mma_i8(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
         ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
@@ -173,6 +185,30 @@ __device__ __forceinline__ void tc_wait_ld8(uint32_t (&v)[8])
                  : "memory");
 }
 
+// all 512 TMEM columns (two accumulators of 256) for the CTA: the allocating warp writes their base address to *slot, and
+// after the CTA barrier every thread returns it
+__device__ __forceinline__ uint32_t tmem_alloc(bool alloc_warp, uint32_t* slot)
+{
+    if (alloc_warp) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(512) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    return *slot;
+}
+// teardown: once every warp of the CTA is done with tensor memory, the allocating warp frees it
+__device__ __forceinline__ void tmem_free(bool alloc_warp, uint32_t base)
+{
+    tc_fence_before();
+    __syncthreads();
+    if (alloc_warp) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(512) : "memory");
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
@@ -196,21 +232,48 @@ inline EncodeTiledFn encode_fn()
     return fn;
 }
 
-// rows x row_elems, row major, fp32 (or f16 with half = true); box = one 128-byte swizzle row (32 floats or 64 halves) x box_rows,
-// zero fill out of bounds; narrow = true: box = one 32-byte swizzle row x box_rows for the single-k-step operands
-inline int make_map(CUtensorMap* map, const void* base, int rows, int row_elems, int box_rows, bool narrow = false, bool half = false)
+// rows x row_elems, row major, elements of type (esize bytes each); box = one 128-byte swizzle row (32 floats, 64 halves or
+// 128 bytes) x box_rows, zero fill out of bounds; narrow = true: box = one 32-byte swizzle row x box_rows for the
+// single-k-step operands
+inline int make_map(CUtensorMap* map, const void* base, int rows, int row_elems, int box_rows, CUtensorMapDataType type, int esize,
+                    bool narrow = false)
 {
     EncodeTiledFn fn = encode_fn();
     if (!fn) { set_error("cuTensorMapEncodeTiled is not available from this driver"); return ERP_E_CUDA; }
-    const cuuint32_t esize = half ? 2 : 4;
     cuuint64_t dims[2] = {(cuuint64_t)row_elems, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)row_elems * esize};
     cuuint32_t box[2] = {(narrow ? 32u : 128u) / esize, (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(map, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides,
+    CUresult r = fn(map, type, 2, const_cast<void*>(base), dims, strides,
                     box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, narrow ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_128B,
                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d", (int)r); return ERP_E_CUDA; }
+    return ERP_OK;
+}
+
+// Stream-K plan: the n_rows x n_ttiles unit grid (row of query tiles major) is cut into equal contiguous ranges, one per
+// CTA.  A row may be cut into at most max_seg segments (each writes its own candidate lists), which bounds the range
+// length from below for small n_rows.
+struct StreamK { int units_per_cta, n_seg, grid; };
+inline StreamK stream_k_plan(int n_rows, int n_ttiles, int sms, int max_seg)
+{
+    const long total = (long)n_rows * n_ttiles;
+    long L = (total + sms - 1) / sms;
+    const long lmin = max_seg > 2 ? (n_ttiles + (max_seg - 2) - 1) / (max_seg - 2) : n_ttiles;   // <= max_seg-2 interior cuts + 1
+    if (L < lmin) L = lmin;
+    if (L < 1) L = 1;
+    const long segs = (n_ttiles + L - 1) / L + 1;    // multiples of L strictly inside one row: at most (n_ttiles + L - 1) / L
+    return {(int)L, (int)(segs > max_seg ? max_seg : segs), (int)((total + L - 1) / L)};
+}
+
+// sets the dynamic shared memory of Kernel once per device, launches it on the context's stream and checks the launch
+template <auto Kernel, class... Args>
+inline int launch_tc_kernel(erp_ctx* ctx, const char* name, int grid, int block, int smem, const Args&... args)
+{
+    static std::atomic<uint64_t> configured{0};
+    ERP_TRY(ensure_dynamic_smem(ctx, Kernel, smem, configured));
+    Kernel<<<grid, block, smem, ctx->stream>>>(args...);
+    ERP_LAUNCH(ctx, name);
     return ERP_OK;
 }
 
@@ -425,6 +488,128 @@ struct SegIter {
         seg = (int)(u / L - row0 / L);      // CTA boundaries (multiples of L) in (row0, u]
         u += t1 - t0;
         return true;
+    }
+};
+
+// Instrumented builds (scripts/build_variant.sh N): -DERP_TC_COUNTERS=1 adds clock64 phase timers to the MMA issuer and the
+// epilogue warps of knn_tc1.cu, =2 counts and times the insert path (scan_chunk_lean); both print after every launch.  Off
+// by default.
+#ifndef ERP_TC_COUNTERS
+#define ERP_TC_COUNTERS 0
+#endif
+#if ERP_TC_COUNTERS == 1
+static __device__ unsigned long long erp_clk[8];
+#define TCC_DECL unsigned long long lclk[6] = {0, 0, 0, 0, 0, 0}
+#define TCC_CLOCK(name) const long long name = clock64()
+#define TCC_ADD(i, v) (lclk[i] += (unsigned long long)(v))
+#define TCC_FLUSH() do { if ((threadIdx.x & 31) == 0) for (int i_ = 0; i_ < 6; i_++) if (lclk[i_]) atomicAdd(&erp_clk[i_], lclk[i_]); } while (0)
+#else
+#define TCC_DECL
+#define TCC_CLOCK(name)
+#define TCC_ADD(i, v)
+#define TCC_FLUSH()
+#endif
+
+// ---- the query-pair pipeline of knn_tc1.cu and knn_bin.cu --------------------------------------------------------------
+// SUB resident query sub-tiles of BM rows share every train tile of BN rows.  A row is KCH k chunks of one 128-byte swizzle
+// row (CK elements of the tensor maps).  The query sub-tiles sit in q_smem as [SUB][KCH] chunks, loaded once per segment;
+// the train chunks pass through a ring of NS slots in t_smem, the KCH chunks of a train tile in consecutive slots.  The
+// product of a sub-tile and a train tile goes to one of the two TMEM accumulators of BN columns, alternately.
+// Barriers: full / empty [NS] (chunk landed / read by the MMAs of the last sub-tile), qfull / qempty (query sub-tiles
+// landed / no longer read), tfull / tempty [2] (accumulator ready / drained, one arrival per epilogue warp).
+template <int SUB, int KCH, int NS, int BM, int BN, int CK>
+struct PairPipe {
+    static constexpr int QCH = BM * 128, TCH = BN * 128;    // bytes of a k chunk of a query sub-tile and of a train tile
+    uint8_t* q_smem;
+    uint8_t* t_smem;
+    uint64_t *full, *empty, *qfull, *qempty, *tfull, *tempty;
+
+    // TMA producer (one thread)
+    __device__ __forceinline__ void produce(const CUtensorMap* map_q, const CUtensorMap* map_t, SegIter it) const
+    {
+        uint32_t slot = 0, ph = 0, seg_n = 0;
+        int qp, t0, t1, seg;
+        for (; it.next(qp, t0, t1, seg); seg_n++) {
+            mbar_wait(qempty, (seg_n & 1) ^ 1);
+            mbar_expect_tx(qfull, SUB * KCH * QCH);
+#pragma unroll
+            for (int sub = 0; sub < SUB; sub++)
+#pragma unroll
+                for (int c = 0; c < KCH; c++)
+                    tma_load_2d(map_q, qfull, q_smem + (sub * KCH + c) * QCH, c * CK, (qp * SUB + sub) * BM);
+            for (int tt = t0; tt < t1; tt++) {
+#pragma unroll
+                for (int c = 0; c < KCH; c++) {
+                    mbar_wait(&empty[slot], ph ^ 1);
+                    mbar_expect_tx(&full[slot], TCH);
+                    tma_load_2d(map_t, &full[slot], t_smem + slot * TCH, c * CK, tt * BN);
+                    if (++slot == NS) { slot = 0; ph ^= 1; }
+                }
+            }
+        }
+    }
+
+    // MMA issuer (one thread).  mma(d_tmem, a_desc, b_desc, accumulate) is one instruction over 32 bytes of every row.
+    // After the k chunks of a (sub-tile, train tile), hook(sub, tt_n, d_tmem) may add to the accumulator before it is
+    // committed to the epilogue; tt_n counts the train tiles of the CTA.
+    template <class Mma, class Hook>
+    __device__ __forceinline__ void issue(uint32_t tmem_base, SegIter it, Mma mma, Hook hook) const
+    {
+        TCC_DECL;
+        uint32_t slot = 0, ph = 0, seg_n = 0, tile_n = 0;
+        const uint32_t q_base = smem_u32(q_smem), t_base = smem_u32(t_smem);
+        uint32_t tt_n = 0;
+        int qp, t0, t1, seg;
+        for (; it.next(qp, t0, t1, seg); seg_n++) {
+            mbar_wait(qfull, seg_n & 1);
+            for (int tt = t0; tt < t1; tt++, tt_n++) {
+                const uint32_t s0 = slot, p0 = ph;
+#pragma unroll
+                for (int sub = 0; sub < SUB; sub++, tile_n++) {
+                    const uint32_t acc = tile_n & 1;
+                    TCC_CLOCK(m0);
+                    mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
+                    TCC_ADD(3, clock64() - m0); TCC_ADD(4, 1);
+                    const uint32_t d_tmem = tmem_base + acc * BN;
+                    uint32_t sl = s0, pp = p0;
+#pragma unroll
+                    for (int c = 0; c < KCH; c++) {
+                        TCC_CLOCK(f0);
+                        if (sub == 0) mbar_wait(&full[sl], pp);
+                        TCC_ADD(5, clock64() - f0);
+                        tc_fence_after();
+                        const uint32_t a = q_base + (sub * KCH + c) * QCH, b = t_base + sl * TCH;
+#pragma unroll
+                        for (int k = 0; k < 4; k++) mma(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), (c | k) != 0);
+                        if (sub == SUB - 1) tc_commit(&empty[sl]);
+                        if (++sl == NS) { sl = 0; pp ^= 1; }
+                    }
+                    hook(sub, tt_n, d_tmem);
+                    tc_commit(&tfull[acc]);
+                    if (sub == SUB - 1) { slot = sl; ph = pp; }
+                }
+            }
+            tc_commit(qempty);
+        }
+        TCC_FLUSH();
+    }
+
+    // epilogue warp: its 128 columns of accumulator acc at taddr go to registers, and the accumulator is handed back before
+    // they are examined, so a slow insert path delays this warp's next read, not the next MMA
+    __device__ __forceinline__ void drain(uint32_t taddr, uint32_t acc, uint32_t (&va)[32], uint32_t (&vb)[32], uint32_t (&vc)[32],
+                                          uint32_t (&vd)[32]) const
+    {
+        tc_ld32(taddr, va);
+        tc_ld32(taddr + 32, vb);
+        tc_ld32(taddr + 64, vc);
+        tc_ld32(taddr + 96, vd);
+        tc_wait_ld32(va);
+        tc_wait_ld32(vb);
+        tc_wait_ld32(vc);
+        tc_wait_ld32(vd);
+        tc_fence_before();
+        __syncwarp();
+        if ((threadIdx.x & 31) == 0) mbar_arrive(&tempty[acc]);
     }
 };
 
