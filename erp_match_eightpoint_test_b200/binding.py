@@ -269,9 +269,14 @@ class Context:
         return int(lib().erp_ctx_launch_count(self._h))
 
     def last_knn_stats(self):
+        """engine, rescanned, the stream-K plan of the distance kernel (segments per query row, units per CTA, grid) and, for
+        float rows on a tensor engine, the largest observed |approximate - exact| / (|q|^2 + max|t|^2).  That deviation takes
+        the slot of the grid in the C record, so grid is None there.  chunks / items: older names of segments / units_per_cta."""
         out = (C.c_int64 * 5)()
         _check(lib().erp_ctx_last_knn_stats(self._h, out))
-        return dict(engine=out[0], rescanned=out[1], chunks=out[2], items=out[3], deviation=out[4] * 1e-12)
+        dev = self.last_knn_operands()["operands"] in (OPERANDS_TF32, OPERANDS_F16)
+        return dict(engine=out[0], rescanned=out[1], segments=out[2], units_per_cta=out[3], grid=None if dev else out[4],
+                    deviation=out[4] * 1e-12 if dev else 0.0, chunks=out[2], items=out[3])
 
     def last_knn_operands(self):
         """Operand format of the last search's tensor products (OPERANDS_*), whether the f16 range guard fired, and how many

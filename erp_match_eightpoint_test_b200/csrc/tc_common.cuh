@@ -465,11 +465,12 @@ __device__ __forceinline__ void scan_chunk_lean(const uint32_t (&v)[32], int col
     }
 }
 
-// A CTA's unit range cut into segments: consecutive train tiles of one query tile.
+// A CTA's unit range cut into segments: consecutive train tiles of one query tile.  Host-callable so that
+// tests/test_plan_host.py can check the plan's coverage and list slots without a GPU.
 struct SegIter {
     long u, end;
     int n_ttiles, L;
-    __device__ SegIter(int n_qtiles, int n_ttiles_, int units_per_cta, int cta)
+    __host__ __device__ SegIter(int n_qtiles, int n_ttiles_, int units_per_cta, int cta)
     {
         L = units_per_cta; n_ttiles = n_ttiles_;
         u = (long)cta * L;
@@ -477,7 +478,7 @@ struct SegIter {
         end = u + L < total ? u + L : total;
     }
     // next segment: query tile, train tiles [t0, t1), list slot of the segment within its query tile
-    __device__ bool next(int& qtile, int& t0, int& t1, int& seg)
+    __host__ __device__ bool next(int& qtile, int& t0, int& t1, int& seg)
     {
         if (u >= end) return false;
         qtile = (int)(u / n_ttiles);

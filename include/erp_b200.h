@@ -101,8 +101,10 @@ int  erp_ctx_set_engine(erp_ctx* ctx, int engine);  /* erp_engine */
 int  erp_ctx_device(erp_ctx* ctx);
 /* number of kernels this context has launched since creation (bench "gpu_launches") */
 uint64_t erp_ctx_launch_count(erp_ctx* ctx);
-/* diagnostics of the last erp_knn2* call: [0] engine used, [1] queries re-scanned exactly,
- * [2] train chunks, [3] work items, [4] reserved */
+/* diagnostics of the last erp_knn2* call: [0] engine used, [1] queries re-scanned exactly, and the plan of the distance
+ * kernel: [2] segments per query row (each writes its own candidate lists), [3] units (query tile x train tile) per CTA,
+ * [4] CTAs.  The SIMT engines report 1, their query blocks and 0.  After a tensor-core search of float rows, [4] is
+ * instead the largest observed |approximate - exact| / (|q|^2 + max|t|^2) of a candidate score, in 1e-12 units. */
 int  erp_ctx_last_knn_stats(erp_ctx* ctx, int64_t out[5]);
 /* operands of the last erp_knn2* call: [0] erp_operands, and for f16 operands [1] 1 if the range guard fired (a finite input
  * f16 cannot hold: every query of the call was re-scanned exactly), [2] queries re-scanned because f16 could not represent
