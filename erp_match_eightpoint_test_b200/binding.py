@@ -200,6 +200,12 @@ def _f64(a):
     return np.ascontiguousarray(a, dtype=np.float64)
 
 
+def _f32_rows(a):
+    """(n, dim) float32 descriptor rows: (array, row stride)."""
+    a = _f32(a)
+    return a, (a.strides[0] if a.shape[0] > 1 else 4 * a.shape[1])
+
+
 def _u8_rows(a):
     """(n, nbytes) uint8 rows whose bytes within a row are contiguous (strided row views stay views): (array, row stride)."""
     a = np.asarray(a)
@@ -309,30 +315,33 @@ class Context:
     # ---- matching (host buffers)
     def knn2_match(self, q, t, ratio: float = 0.3, cross_check: bool = False) -> np.ndarray:
         """feature_matcher::match_two_image (src/feature_matcher.cpp:42-59). Returns DMatch records."""
-        q, t = _f32(q), _f32(t)
-        out = np.empty(max(q.shape[0], 1), DMATCH)
-        n = C.c_int(0)
-        _check(lib().erp_knn2_match(self._h, _ptr(q), q.shape[0], q.strides[0] if q.shape[0] else 4 * q.shape[1],
-                                    _ptr(t), t.shape[0], t.strides[0] if t.shape[0] else 4 * t.shape[1], q.shape[1],
-                                    ratio, int(cross_check), _ptr(out), C.byref(n)))
-        return out[: n.value]          # a view of this call's own array: only the pages the records touched are resident
+        return self._knn2_match(lib().erp_knn2_match, self._h, _f32_rows, q, t, ratio, cross_check)
 
     def knn2_raw(self, q, t):
-        q, t = _f32(q), _f32(t)
+        return self._knn2_raw(lib().erp_knn2_raw, _f32_rows, q, t)
+
+    @staticmethod
+    def _knn2_match(fn, handle, rows, q, t, ratio, cross_check) -> np.ndarray:
+        (q, qs), (t, ts) = rows(q), rows(t)
+        out = np.empty(max(q.shape[0], 1), DMATCH)
+        n = C.c_int(0)
+        _check(fn(handle, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], ratio, int(cross_check), _ptr(out), C.byref(n)))
+        return out[: n.value]          # a view of this call's own array: only the pages the records touched are resident
+
+    def _knn2_raw(self, fn, rows, q, t):
+        (q, qs), (t, ts) = rows(q), rows(t)
         idx = np.empty((q.shape[0], 2), np.int32)
         dist = np.empty((q.shape[0], 2), np.float32)
-        _check(lib().erp_knn2_raw(self._h, _ptr(q), q.shape[0], 4 * q.shape[1], _ptr(t), t.shape[0], 4 * t.shape[1],
-                                  q.shape[1], _ptr(idx), _ptr(dist)))
+        _check(fn(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], _ptr(idx), _ptr(dist)))
         return idx, dist
 
     def knn2_near_ties(self, q, t, rel_tol: float = 1e-6) -> np.ndarray:
         """Per-query flags of erp_knn2_near_ties: bit 0 order of the two nearest, bit 1 identity of the second."""
-        q, t = _f32(q), _f32(t)
+        (q, qs), (t, ts) = _f32_rows(q), _f32_rows(t)
         flags = np.zeros(max(q.shape[0], 1), np.uint8)
         n = C.c_int(0)
-        _check(lib().erp_knn2_near_ties(self._h, _ptr(q), q.shape[0], q.strides[0] if q.shape[0] else 4 * q.shape[1],
-                                        _ptr(t), t.shape[0], t.strides[0] if t.shape[0] else 4 * t.shape[1], q.shape[1],
-                                        rel_tol, _ptr(flags), C.byref(n)))
+        _check(lib().erp_knn2_near_ties(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], rel_tol, _ptr(flags),
+                                        C.byref(n)))
         flags = flags[: q.shape[0]]
         assert int((flags != 0).sum()) == n.value
         return flags
@@ -355,19 +364,10 @@ class Context:
     # ---- binary descriptors (Hamming distance; include/erp_b200.h "binary descriptors")
     def knn2_match_bin(self, q, t, ratio: float = 0.3, cross_check: bool = False) -> np.ndarray:
         """match_two_image with cv::BFMatcher(NORM_HAMMING): (n, nbytes) uint8 rows -> DMatch records."""
-        (q, qs), (t, ts) = _u8_rows(q), _u8_rows(t)
-        out = np.empty(max(q.shape[0], 1), DMATCH)
-        n = C.c_int(0)
-        _check(lib().erp_knn2_match_bin(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1],
-                                        ratio, int(cross_check), _ptr(out), C.byref(n)))
-        return out[: n.value]
+        return self._knn2_match(lib().erp_knn2_match_bin, self._h, _u8_rows, q, t, ratio, cross_check)
 
     def knn2_raw_bin(self, q, t):
-        (q, qs), (t, ts) = _u8_rows(q), _u8_rows(t)
-        idx = np.empty((q.shape[0], 2), np.int32)
-        dist = np.empty((q.shape[0], 2), np.float32)
-        _check(lib().erp_knn2_raw_bin(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], _ptr(idx), _ptr(dist)))
-        return idx, dist
+        return self._knn2_raw(lib().erp_knn2_raw_bin, _u8_rows, q, t)
 
     def knn2_bin_dev(self, d_q, nq, d_t, nt, nbytes, d_idx2, d_dist2, d_d2=None):
         _check(lib().erp_knn2_bin_dev(self._h, _ptr(d_q), nq, _ptr(d_t), nt, nbytes, _ptr(d_idx2), _ptr(d_dist2), _ptr(d_d2)))
@@ -379,18 +379,8 @@ class Context:
     def pair_pose_bin(self, q, t, left_xy, right_xy, W, H_img, ratio=0.8, cross_check=False, seed=1, H=10000, S=8,
                       metric=METRIC_ALGEBRAIC, tau=0.002):
         """erp_pair_pose_bin: binary descriptors + all keypoints of both views -> (match records, RANSAC result with mask)."""
-        (q, qs), (t, ts) = _u8_rows(q), _u8_rows(t)
-        left_xy, right_xy = _f32(left_xy), _f32(right_xy)
-        out = np.empty(q.shape[0], DMATCH)
-        n = C.c_int(0)
-        res = RansacResult()
-        mask = np.empty(q.shape[0], np.uint8)
-        _check(lib().erp_pair_pose_bin(self._h, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1], ratio, int(cross_check),
-                                       _ptr(left_xy), _ptr(right_xy), left_xy.strides[0], W, H_img, seed, H, S, metric, tau,
-                                       _ptr(out), C.byref(n), C.byref(res), _ptr(mask)))
-        r = self._result(res)
-        r["mask"] = mask[:n.value]
-        return out[:n.value], r
+        return self._pair_pose(lib().erp_pair_pose_bin, self._h, _u8_rows, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed,
+                               H, S, metric, tau)
 
     def pair_pose_bin_dev(self, d_q, nq, d_t, nt, nbytes, ratio, cross_check, d_left_xy, d_right_xy, kp_stride, W, H_img, seed, H,
                           S, metric, tau, d_matches, d_n, d_mask, d_result):
@@ -502,7 +492,7 @@ class Context:
     def pair_pose(self, q, t, left_xy, right_xy, W, H_img, ratio=0.3, cross_check=False, seed=1, H=10000, S=8,
                   metric=METRIC_ALGEBRAIC, tau=0.002):
         """erp_pair_pose: descriptors + all keypoints of both views -> (match records, RANSAC result with mask)."""
-        return self._pair_pose(lib().erp_pair_pose, self._h, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed, H, S,
+        return self._pair_pose(lib().erp_pair_pose, self._h, _f32_rows, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed, H, S,
                                metric, tau)
 
     def pair_pose_dev(self, d_q, nq, d_t, nt, dim, ratio, cross_check, d_left_xy, d_right_xy, kp_stride, W, H_img, seed, H, S,
@@ -537,31 +527,26 @@ class Context:
     def pair_pose_dist(self, q, t, left_xy, right_xy, W, H_img, ratio=0.3, cross_check=False, seed=1, H=10000, S=8,
                        metric=METRIC_ALGEBRAIC, tau=0.002):
         """erp_pair_pose_dist: collective over the context's clique, host buffers (every rank passes the same arrays)."""
-        return self._pair_pose(lib().erp_pair_pose_dist, self._h, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed, H, S,
+        return self._pair_pose(lib().erp_pair_pose_dist, self._h, _f32_rows, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed, H, S,
                                metric, tau)
 
     def knn2_match_dist(self, q, t, ratio: float = 0.3, cross_check: bool = False) -> np.ndarray:
         """This rank's part of the query-sharded match list (global query ids)."""
-        q, t = _f32(q), _f32(t)
-        out = np.empty(max(q.shape[0], 1), DMATCH)
-        n = C.c_int(0)
-        _check(lib().erp_knn2_match_dist(self._h, _ptr(q), q.shape[0], q.strides[0] if q.shape[0] else 4 * q.shape[1],
-                                         _ptr(t), t.shape[0], t.strides[0] if t.shape[0] else 4 * t.shape[1], q.shape[1],
-                                         ratio, int(cross_check), _ptr(out), C.byref(n)))
-        return out[: n.value]
+        return self._knn2_match(lib().erp_knn2_match_dist, self._h, _f32_rows, q, t, ratio, cross_check)
 
     def knn2_match_dist_dev(self, d_q_shard, nq_total, d_t, nt, dim, ratio, cross_check, d_out, d_n_out):
         _check(lib().erp_knn2_match_dist_dev(self._h, _ptr(d_q_shard), nq_total, _ptr(d_t), nt, dim, ratio, int(cross_check),
                                              _ptr(d_out), _ptr(d_n_out)))
 
     @classmethod
-    def _pair_pose(cls, fn, handle, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed, H, S, metric, tau):
-        q, t, left_xy, right_xy = _f32(q), _f32(t), _f32(left_xy), _f32(right_xy)
+    def _pair_pose(cls, fn, handle, rows, q, t, left_xy, right_xy, W, H_img, ratio, cross_check, seed, H, S, metric, tau):
+        (q, qs), (t, ts) = rows(q), rows(t)
+        left_xy, right_xy = _f32(left_xy), _f32(right_xy)
         out = np.empty(q.shape[0], DMATCH)
         n = C.c_int(0)
         res = RansacResult()
         mask = np.empty(q.shape[0], np.uint8)
-        _check(fn(handle, _ptr(q), q.shape[0], q.strides[0], _ptr(t), t.shape[0], t.strides[0], q.shape[1],
+        _check(fn(handle, _ptr(q), q.shape[0], qs, _ptr(t), t.shape[0], ts, q.shape[1],
                   ratio, int(cross_check), _ptr(left_xy), _ptr(right_xy), left_xy.strides[0], W, H_img,
                   seed, H, S, metric, tau, _ptr(out), C.byref(n), C.byref(res), _ptr(mask)))
         r = cls._result(res)
@@ -703,14 +688,8 @@ class Group:
 
     def pair_pose(self, q, t, left_xy, right_xy, W, H_img, ratio=0.3, cross_check=False, seed=1, H=10000, S=8,
                   metric=METRIC_ALGEBRAIC, tau=0.002):
-        return Context._pair_pose(lib().erp_group_pair_pose, self._h, q, t, left_xy, right_xy, W, H_img, ratio, cross_check,
+        return Context._pair_pose(lib().erp_group_pair_pose, self._h, _f32_rows, q, t, left_xy, right_xy, W, H_img, ratio, cross_check,
                                   seed, H, S, metric, tau)
 
     def knn2_match(self, q, t, ratio: float = 0.3, cross_check: bool = False) -> np.ndarray:
-        q, t = _f32(q), _f32(t)
-        out = np.empty(max(q.shape[0], 1), DMATCH)
-        n = C.c_int(0)
-        _check(lib().erp_group_knn2_match(self._h, _ptr(q), q.shape[0], q.strides[0] if q.shape[0] else 4 * q.shape[1],
-                                          _ptr(t), t.shape[0], t.strides[0] if t.shape[0] else 4 * t.shape[1], q.shape[1],
-                                          ratio, int(cross_check), _ptr(out), C.byref(n)))
-        return out[: n.value]
+        return Context._knn2_match(lib().erp_group_knn2_match, self._h, _f32_rows, q, t, ratio, cross_check)

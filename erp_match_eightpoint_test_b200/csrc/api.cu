@@ -153,19 +153,19 @@ static bool is_pageable(const void* p)
     return a.type == cudaMemoryTypeUnregistered;
 }
 
-int upload_rows(erp_ctx* ctx, void* d_dst, const void* src, int rows, size_t row_bytes, size_t stride)
+int upload_rows(erp_ctx* ctx, cudaStream_t stream, void* d_dst, const void* src, int rows, size_t row_bytes, size_t stride)
 {
     if (rows == 0) return ERP_OK;
     const size_t total = row_bytes * (size_t)rows;
     StagePool* pool = (total >= STAGE_MIN_BYTES && row_bytes <= STAGE_CHUNK && is_pageable(src)) ? stage_pool(ctx) : nullptr;
     if (!pool) {
-        if (stride == row_bytes) ERP_CUDA(cudaMemcpyAsync(d_dst, src, total, cudaMemcpyHostToDevice, ctx->stream));
-        else ERP_CUDA(cudaMemcpy2DAsync(d_dst, row_bytes, src, stride, row_bytes, rows, cudaMemcpyHostToDevice, ctx->stream));
+        if (stride == row_bytes) ERP_CUDA(cudaMemcpyAsync(d_dst, src, total, cudaMemcpyHostToDevice, stream));
+        else ERP_CUDA(cudaMemcpy2DAsync(d_dst, row_bytes, src, stride, row_bytes, rows, cudaMemcpyHostToDevice, stream));
         return ERP_OK;
     }
     // the staged copies must not overtake work already queued on the target buffer
     const double t_begin = now_s();
-    ERP_CUDA(cudaEventRecord(ctx->ev_copy[8], ctx->stream));
+    ERP_CUDA(cudaEventRecord(ctx->ev_copy[8], stream));
     const int T = pool->threads;
     const int rows_per_chunk = (int)(STAGE_CHUNK / row_bytes);
     std::atomic<int> failed{0};
@@ -187,9 +187,9 @@ int upload_rows(erp_ctx* ctx, void* d_dst, const void* src, int rows, size_t row
     };
     pool->run(work);
     if (failed) { set_error("staged upload failed: %s", cudaGetErrorString(cudaGetLastError())); return ERP_E_CUDA; }
-    // the context stream continues after the last DMA of every helper stream
+    // `stream` continues after the last DMA of every helper stream
     for (int t = 0; t < T; t++)
-        for (int s = 0; s < StagePool::SLOTS; s++) ERP_CUDA(cudaStreamWaitEvent(ctx->stream, pool->ev[t][s], 0));
+        for (int s = 0; s < StagePool::SLOTS; s++) ERP_CUDA(cudaStreamWaitEvent(stream, pool->ev[t][s], 0));
     if (getenv("ERP_B200_STAGE_TRACE")) fprintf(stderr, "[stage] %zu bytes staged by %d threads, host %.3f ms\n", total, T, 1e3 * (now_s() - t_begin));
     return ERP_OK;
 }
@@ -408,100 +408,127 @@ ERP_API int erp_ctx_last_knn_operands(erp_ctx* ctx, int64_t out[3])
 }
 
 // ======================================================================================
-// matching
+// matching: float rows (knn_exact.cu, knn_tc.cu, knn_tc1.cu) and binary rows (knn_bin.cu: feature_matcher::match_two_image
+// with NORM_HAMMING) through the same entry points
 // ======================================================================================
-static int check_knn_args(const char* who, erp_ctx* ctx, int nq, int nt, int dim)
+namespace erp {
+
+int RowKind::check_dim(const char* who) const
+{
+    if (bin) ERP_ARG(dim >= 1 && dim <= 64, ERP_E_DIM, "%s: binary descriptor size %d must be in [1,64] bytes", who, dim);
+    else ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "%s: descriptor dimension %d must be a multiple of 4 in [4,512]", who, dim);
+    return ERP_OK;
+}
+
+// Both tensor engine settings select the kind::i8 engine for binary rows, which serves every shape.  AUTO takes a tensor
+// engine where it is faster than SIMT: the one-product engine for float rows, the i8 engine for binary rows.
+int RowKind::engine(erp_ctx* ctx, int nq, int nt, bool fallback, int* out) const
+{
+    const bool forced = ctx->engine == ERP_ENGINE_TCGEN05 || ctx->engine == ERP_ENGINE_TCGEN05_1X;
+    const bool tc = bin ? forced || (ctx->engine == ERP_ENGINE_AUTO && knn2_bin_preferred(nq, nt))
+                        : forced ? knn2_tc_supported(nq, nt, dim) : ctx->engine == ERP_ENGINE_AUTO && knn2_tc_preferred(nq, nt, dim);
+    ERP_ARG(tc || !forced || fallback, ERP_E_DIM, "tcgen05 engine does not support nq=%d nt=%d dim=%d", nq, nt, dim);
+    *out = !tc ? ERP_ENGINE_EXACT_SIMT : ctx->engine == ERP_ENGINE_TCGEN05 ? ERP_ENGINE_TCGEN05 : ERP_ENGINE_TCGEN05_1X;
+    return ERP_OK;
+}
+
+int RowKind::knn2(erp_ctx* ctx, int engine, bool forward, const void* d_q, int nq, const void* d_t, int nt,
+                  int32_t* d_idx2, float* d_dist2, double* d_d2) const
+{
+    if (bin)
+        return knn2_bin(ctx, static_cast<const uint8_t*>(d_q), nq, static_cast<const uint8_t*>(d_t), nt, dim, engine != ERP_ENGINE_EXACT_SIMT,
+                        d_idx2, d_dist2, d_d2);
+    const float *q = static_cast<const float*>(d_q), *t = static_cast<const float*>(d_t);
+    if (engine == ERP_ENGINE_TCGEN05) return knn2_tc(ctx, q, nq, t, nt, dim, d_idx2, d_dist2, d_d2);
+    if (engine == ERP_ENGINE_TCGEN05_1X) return knn2_tc1(ctx, q, nq, t, nt, dim, d_idx2, d_dist2, d_d2);
+    if (!forward) return knn2_exact(ctx, q, nq, t, nt, dim, nullptr, 0, 0, d_idx2, d_dist2, d_d2);
+    set_knn_stats(ctx, ERP_ENGINE_EXACT_SIMT, false, 1, cdiv(nq, 64), 0, nullptr);
+    ERP_CUDA(record_timing(ctx, ctx->ev_k0));
+    ERP_TRY(knn2_exact(ctx, q, nq, t, nt, dim, nullptr, 0, 0, d_idx2, d_dist2, d_d2));
+    ERP_CUDA(record_timing(ctx, ctx->ev_k1));
+    return ERP_OK;
+}
+
+int check_knn_args(const char* who, erp_ctx* ctx, int nq, int nt, RowKind k)
 {
     ERP_ARG(ctx, ERP_E_ARG, "%s: null context", who);
     ERP_ARG(nq >= 0 && nt >= 0, ERP_E_ARG, "%s: negative size", who);
-    ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "%s: descriptor dimension %d must be a multiple of 4 in [4,512]", who, dim);
+    ERP_TRY(k.check_dim(who));
     // knnMatch(k=2) on fewer than 2 train rows throws in the reference (FLANN: knn <= index size)
     ERP_ARG(nq == 0 || nt >= 2, ERP_E_TOO_FEW_TRAIN, "%s: k=2 needs at least 2 train descriptors, got %d", who, nt);
     return ERP_OK;
 }
 
-ERP_API int erp_knn2_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
-                         int32_t* d_idx2, float* d_dist2, double* d_d2)
-{
-    ERP_TRY(check_knn_args("erp_knn2_dev", ctx, nq, nt, dim));
-    if (nq == 0) return ERP_OK;
-    ERP_ARG(d_q && d_t, ERP_E_ARG, "erp_knn2_dev: null descriptors");
-    DeviceGuard g(ctx->device);
-    const bool forced = ctx->engine == ERP_ENGINE_TCGEN05 || ctx->engine == ERP_ENGINE_TCGEN05_1X;
-    if (forced) ERP_ARG(knn2_tc_supported(nq, nt, dim), ERP_E_DIM, "tcgen05 engine does not support nq=%d nt=%d dim=%d", nq, nt, dim);
-    if (ctx->engine == ERP_ENGINE_TCGEN05) return knn2_tc(ctx, d_q, nq, d_t, nt, dim, d_idx2, d_dist2, d_d2);
-    if (ctx->engine == ERP_ENGINE_TCGEN05_1X || (ctx->engine == ERP_ENGINE_AUTO && knn2_tc_preferred(nq, nt, dim)))
-        return knn2_tc1(ctx, d_q, nq, d_t, nt, dim, d_idx2, d_dist2, d_d2);
-    set_knn_stats(ctx, ERP_ENGINE_EXACT_SIMT, false, 1, cdiv(nq, 64), 0, nullptr);
-    ERP_CUDA(record_timing(ctx, ctx->ev_k0));
-    ERP_TRY(knn2_exact(ctx, d_q, nq, d_t, nt, dim, nullptr, 0, 0, d_idx2, d_dist2, d_d2));
-    ERP_CUDA(record_timing(ctx, ctx->ev_k1));
-    return ERP_OK;
-}
-
-namespace erp {
 __global__ void add_offset_kernel(int32_t* v, int n, int off)
 {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n && v[i] >= 0) v[i] += off;
 }
-}
-static int add_offset(erp_ctx* ctx, int32_t* v, int n, int off)
+
+} // namespace erp
+
+static int knn2_dev(const char* who, erp_ctx* ctx, RowKind k, const void* d_q, int nq, const void* d_t, int nt,
+                    int32_t* d_idx2, float* d_dist2, double* d_d2)
 {
-    erp::add_offset_kernel<<<cdiv(n, 256), 256, 0, ctx->stream>>>(v, n, off);
-    ERP_LAUNCH(ctx, "add_offset_kernel");
-    return ERP_OK;
+    ERP_TRY(check_knn_args(who, ctx, nq, nt, k));
+    if (nq == 0) return ERP_OK;
+    ERP_ARG(d_q && d_t, ERP_E_ARG, "%s: null descriptors", who);
+    DeviceGuard g(ctx->device);
+    int engine;
+    ERP_TRY(k.engine(ctx, nq, nt, false, &engine));
+    return k.knn2(ctx, engine, true, d_q, nq, d_t, nt, d_idx2, d_dist2, d_d2);
 }
 
-ERP_API int erp_nn1_reverse_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
-                                int q_offset, int32_t* d_best_q, double* d_best_d2)
+// cross-check: the nearest query of every train row (roles swapped, lowest query index on ties), compacted to the first
+// neighbour; the query index is offset by q_offset, d_best_d2 (float rows) receives the squared distance
+static int knn1_reverse(erp_ctx* ctx, RowKind k, const void* d_q, int nq, const void* d_t, int nt, int q_offset,
+                        int32_t* d_best_q, double* d_best_d2)
 {
-    ERP_ARG(ctx && nq >= 1 && nt >= 0 && d_best_q, ERP_E_ARG, "erp_nn1_reverse_dev: bad argument");
-    ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "erp_nn1_reverse_dev: bad dimension %d", dim);
-    if (nt == 0) return ERP_OK;
-    DeviceGuard g(ctx->device);
-    // roles swapped: every train row looks for its nearest query.  Results land interleaved
-    // (x2) in scratch and are compacted to the first neighbour.
     int st = ERP_OK;
     int32_t* idx2 = ctx->scratch<int32_t>(S_RS_IDX, (size_t)nt * 2, &st);
-    double* d2 = ctx->scratch<double>(S_RS_D2, (size_t)nt * 2, &st);
+    double* d2 = k.bin ? nullptr : ctx->scratch<double>(S_RS_D2, (size_t)nt * 2, &st);
     ERP_TRY(st);
-    const bool forced = ctx->engine == ERP_ENGINE_TCGEN05 || ctx->engine == ERP_ENGINE_TCGEN05_1X;
-    bool tc = nq >= 2 && (forced ? knn2_tc_supported(nt, nq, dim) : (ctx->engine == ERP_ENGINE_AUTO && knn2_tc_preferred(nt, nq, dim)));
-    if (tc) {
-        // (the tensor-core paths have no index offset: it is added while compacting)
-        if (ctx->engine == ERP_ENGINE_TCGEN05) ERP_TRY(knn2_tc(ctx, d_t, nt, d_q, nq, dim, idx2, nullptr, d2));
-        else ERP_TRY(knn2_tc1(ctx, d_t, nt, d_q, nq, dim, idx2, nullptr, d2));
-    } else {
-        ERP_TRY(knn2_exact(ctx, d_t, nt, d_q, nq, dim, nullptr, 0, 0, idx2, nullptr, d2));
-    }
+    int engine;
+    ERP_TRY(k.engine(ctx, nt, nq, true, &engine));
+    ERP_TRY(k.knn2(ctx, engine, false, d_t, nt, d_q, nq, idx2, nullptr, d2));      // (no index offset: it is added below)
     ERP_CUDA(cudaMemcpy2DAsync(d_best_q, sizeof(int32_t), idx2, 2 * sizeof(int32_t), sizeof(int32_t), nt,
                                cudaMemcpyDeviceToDevice, ctx->stream));
     if (d_best_d2)
         ERP_CUDA(cudaMemcpy2DAsync(d_best_d2, sizeof(double), d2, 2 * sizeof(double), sizeof(double), nt,
                                    cudaMemcpyDeviceToDevice, ctx->stream));
-    if (q_offset != 0) ERP_TRY(add_offset(ctx, d_best_q, nt, q_offset));
+    if (q_offset != 0) {
+        erp::add_offset_kernel<<<cdiv(nt, 256), 256, 0, ctx->stream>>>(d_best_q, nt, q_offset);
+        ERP_LAUNCH(ctx, "add_offset_kernel");
+    }
     return ERP_OK;
 }
 
-ERP_API int erp_knn2_match_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
-                               float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
+// the cross-check (when asked) and the ratio filter of the 2-NN of a pair: match records and their count on the device
+static int filter_matches(erp_ctx* ctx, RowKind k, const void* d_q, int nq, const void* d_t, int nt, const int32_t* idx2,
+                          const float* dist2, float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
 {
-    ERP_TRY(check_knn_args("erp_knn2_match_dev", ctx, nq, nt, dim));
-    ERP_ARG(d_n_out, ERP_E_ARG, "erp_knn2_match_dev: d_n_out is null");
+    int32_t* rev = nullptr;
+    if (cross_check && nq > 0) {
+        int st = ERP_OK;
+        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
+        ERP_TRY(st);
+        ERP_TRY(knn1_reverse(ctx, k, d_q, nq, d_t, nt, 0, rev, nullptr));
+    }
+    return erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n_out);
+}
+
+static int knn2_match_dev(const char* who, erp_ctx* ctx, RowKind k, const void* d_q, int nq, const void* d_t, int nt,
+                          float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
+{
+    ERP_TRY(check_knn_args(who, ctx, nq, nt, k));
+    ERP_ARG(d_n_out, ERP_E_ARG, "%s: d_n_out is null", who);
     DeviceGuard g(ctx->device);
     int st = ERP_OK;
     int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
     float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
     ERP_TRY(st);
-    ERP_TRY(erp_knn2_dev(ctx, d_q, nq, d_t, nt, dim, idx2, dist2, nullptr));
-    int32_t* rev = nullptr;
-    if (cross_check && nq > 0) {
-        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
-        ERP_TRY(st);
-        ERP_TRY(erp_nn1_reverse_dev(ctx, d_q, nq, d_t, nt, dim, 0, rev, nullptr));
-    }
-    return erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n_out);
+    ERP_TRY(knn2_dev(who, ctx, k, d_q, nq, d_t, nt, idx2, dist2, nullptr));
+    return filter_matches(ctx, k, d_q, nq, d_t, nt, idx2, dist2, ratio, cross_check, d_out, d_n_out);
 }
 
 // Host-buffer 2-NN: the train set and the first query chunk are uploaded, then every further query chunk travels
@@ -538,24 +565,26 @@ static int chunk_bounds(int nq, int nt, bool pageable, int (&bounds)[9])
     bounds[++n] = nq;
     return n;
 }
-// search(d_q_chunk, rows, idx2, dist2): the 2-NN of one uploaded query chunk against the uploaded train rows
-using ChunkSearch = std::function<int(const void*, int, int32_t*, float*)>;
-static int knn2_host_rows(erp_ctx* ctx, const void* q, int nq, size_t qs, const void* t, int nt, size_t ts, size_t row,
-                          uint8_t* dq, uint8_t* dt, const ChunkSearch& search, int32_t* d_idx2, float* d_dist2)
+
+// host rows -> S_Q / S_T (dense, 16 bytes of padding) and their 2-NN
+static int knn2_host(erp_ctx* ctx, RowKind k, const void* q, int nq, size_t qs, const void* t, int nt, size_t ts,
+                     int32_t* d_idx2, float* d_dist2)
 {
+    const size_t row = k.row_bytes();
+    ERP_ARG((nq == 0 || q) && (nt == 0 || t), ERP_E_ARG, "null descriptor pointer");
+    ERP_ARG(qs >= row && ts >= row, ERP_E_ARG, "row stride smaller than a descriptor row (%zu < %zu)", qs < ts ? qs : ts, row);
+    int st = ERP_OK;
+    uint8_t* dq = ctx->scratch<uint8_t>(S_Q, (size_t)nq * row + 16, &st);
+    uint8_t* dt = ctx->scratch<uint8_t>(S_T, (size_t)nt * row + 16, &st);
+    ERP_TRY(st);
+    // one engine for the whole call: the tensor engines prepare the train operand with the first query chunk only
+    int engine;
+    ERP_TRY(k.engine(ctx, nq, nt, false, &engine));
     int bounds[9];
     const int chunks = chunk_bounds(nq, nt, is_pageable(q), bounds);
     // fork: the copy stream starts after whatever the context stream still has queued
     ERP_CUDA(cudaEventRecord(ctx->ev_copy[7], ctx->stream));
     ERP_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[7], 0));
-    cudaStream_t main_stream = ctx->stream;
-    // upload_rows enqueues on ctx->stream; it must point at the context's own stream again on EVERY exit path
-    struct StreamSwap {
-        erp_ctx* c; cudaStream_t main;
-        void to_copy() { c->stream = c->copy_stream; }
-        void to_main() { c->stream = main; }
-        ~StreamSwap() { c->stream = main; }
-    } sw{ctx, main_stream};
     // tc_chunk > 0 tells the tensor engines that the train operand of this call is already prepared: it must not
     // survive this function on ANY exit path (a stale value would make the next call reuse old train data)
     struct ChunkReset { erp_ctx* c; ~ChunkReset() { c->tc_chunk = 0; } } reset{ctx};
@@ -565,24 +594,21 @@ static int knn2_host_rows(erp_ctx* ctx, const void* q, int nq, size_t qs, const 
     int n_tr = 0;
     auto mark = [&](cudaStream_t s) { if (trace && n_tr < 20 && cudaEventCreate(&tr[n_tr]) == cudaSuccess) cudaEventRecord(tr[n_tr++], s); };
     mark(ctx->copy_stream);
-    sw.to_copy();
-    int rc = upload_rows(ctx, dt, t, nt, row, ts);
+    int rc = upload_rows(ctx, ctx->copy_stream, dt, t, nt, row, ts);
     mark(ctx->copy_stream);
     // chunk c's search is enqueued as soon as chunk c is on its way: a pageable source blocks this thread while the
     // staging threads copy chunk c + 1, and the device searches chunk c meanwhile (pinned sources never block here)
     for (int c = 0; c < chunks && rc == ERP_OK; c++) {
         const int r0 = bounds[c], n = bounds[c + 1] - r0;
-        sw.to_copy();
-        rc = upload_rows(ctx, dq + (size_t)r0 * row, reinterpret_cast<const char*>(q) + (size_t)r0 * qs, n, row, qs);
+        rc = upload_rows(ctx, ctx->copy_stream, dq + (size_t)r0 * row, static_cast<const char*>(q) + (size_t)r0 * qs, n, row, qs);
         if (rc == ERP_OK && cudaEventRecord(ctx->ev_copy[c], ctx->copy_stream) != cudaSuccess) rc = ERP_E_CUDA;
         mark(ctx->copy_stream);
-        sw.to_main();
         if (rc != ERP_OK) break;
         ERP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy[c], 0));
         mark(ctx->stream);
         ctx->tc_chunk = c;
         const double t_enq = now_s();
-        rc = search(dq + (size_t)r0 * row, n, d_idx2 + 2 * (size_t)r0, d_dist2 + 2 * (size_t)r0);
+        rc = k.knn2(ctx, engine, true, dq + (size_t)r0 * row, n, dt, nt, d_idx2 + 2 * (size_t)r0, d_dist2 + 2 * (size_t)r0, nullptr);
         mark(ctx->stream);
         if (trace) fprintf(stderr, "[stage] chunk %d: search of %d rows enqueued in %.3f ms (host)\n", c, n, 1e3 * (now_s() - t_enq));
     }
@@ -597,31 +623,15 @@ static int knn2_host_rows(erp_ctx* ctx, const void* q, int nq, size_t qs, const 
     }
     return rc;
 }
-static int knn2_host(erp_ctx* ctx, const float* q, int nq, size_t qs, const float* t, int nt, size_t ts, int dim,
-                     int32_t* d_idx2, float* d_dist2)
-{
-    size_t row = (size_t)dim * sizeof(float);
-    ERP_ARG((nq == 0 || q) && (nt == 0 || t), ERP_E_ARG, "null descriptor pointer");
-    ERP_ARG(qs >= row && ts >= row, ERP_E_ARG, "row stride smaller than a descriptor row (%zu < %zu)", qs < ts ? qs : ts, row);
-    int st = ERP_OK;
-    float* dq = ctx->scratch<float>(S_Q, (size_t)nq * dim + 4, &st);
-    float* dt = ctx->scratch<float>(S_T, (size_t)nt * dim + 4, &st);
-    ERP_TRY(st);
-    return knn2_host_rows(ctx, q, nq, qs, t, nt, ts, row, reinterpret_cast<uint8_t*>(dq), reinterpret_cast<uint8_t*>(dt),
-                          [&](const void* cq, int n, int32_t* i2, float* d2) {
-                              return erp_knn2_dev(ctx, static_cast<const float*>(cq), n, dt, nt, dim, i2, d2, nullptr);
-                          }, d_idx2, d_dist2);
-}
 
-ERP_API int erp_knn2_match(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes,
-                           const float* t, int nt, size_t t_stride_bytes, int dim,
-                           float ratio, int cross_check, erp_dmatch* out, int* n_out)
+static int knn2_match_host(const char* who, erp_ctx* ctx, RowKind k, const void* q, int nq, size_t qs, const void* t, int nt,
+                           size_t ts, float ratio, int cross_check, erp_dmatch* out, int* n_out)
 {
-    ERP_TRY(check_knn_args("erp_knn2_match", ctx, nq, nt, dim));
-    ERP_ARG(n_out, ERP_E_ARG, "erp_knn2_match: n_out is null");
+    ERP_TRY(check_knn_args(who, ctx, nq, nt, k));
+    ERP_ARG(n_out, ERP_E_ARG, "%s: n_out is null", who);
     *n_out = 0;
     if (nq == 0) return ERP_OK;
-    ERP_ARG(out, ERP_E_ARG, "erp_knn2_match: out is null");
+    ERP_ARG(out, ERP_E_ARG, "%s: out is null", who);
     DeviceGuard g(ctx->device);
     int st = ERP_OK;
     erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
@@ -629,40 +639,70 @@ ERP_API int erp_knn2_match(erp_ctx* ctx, const float* q, int nq, size_t q_stride
     int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
     float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
     ERP_TRY(st);
-    ERP_TRY(knn2_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, dim, idx2, dist2));
-    int32_t* rev = nullptr;
-    if (cross_check) {
-        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
-        ERP_TRY(st);
-        ERP_TRY(erp_nn1_reverse_dev(ctx, ctx->dev[S_Q].as<float>(), nq, ctx->dev[S_T].as<float>(), nt, dim, 0, rev, nullptr));
-    }
-    ERP_TRY(erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n));
+    ERP_TRY(knn2_host(ctx, k, q, nq, qs, t, nt, ts, idx2, dist2));
+    ERP_TRY(filter_matches(ctx, k, ctx->dev[S_Q].p, nq, ctx->dev[S_T].p, nt, idx2, dist2, ratio, cross_check, d_out, d_n));
     return download_matches(ctx, d_out, d_n, (size_t)nq, out, n_out);
 }
 
-ERP_API int erp_knn2_raw(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes,
-                         const float* t, int nt, size_t t_stride_bytes, int dim,
-                         int32_t* idx2, float* dist2)
+static int knn2_raw_host(const char* who, erp_ctx* ctx, RowKind k, const void* q, int nq, size_t qs, const void* t, int nt,
+                         size_t ts, int32_t* idx2, float* dist2)
 {
-    ERP_TRY(check_knn_args("erp_knn2_raw", ctx, nq, nt, dim));
+    ERP_TRY(check_knn_args(who, ctx, nq, nt, k));
     if (nq == 0) return ERP_OK;
     DeviceGuard g(ctx->device);
     int st = ERP_OK;
     int32_t* d_idx = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
     float* d_dist = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
     ERP_TRY(st);
-    ERP_TRY(knn2_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, dim, d_idx, d_dist));
+    ERP_TRY(knn2_host(ctx, k, q, nq, qs, t, nt, ts, d_idx, d_dist));
     if (idx2) ERP_CUDA(cudaMemcpyAsync(idx2, d_idx, sizeof(int32_t) * 2 * (size_t)nq, cudaMemcpyDeviceToHost, ctx->stream));
     if (dist2) ERP_CUDA(cudaMemcpyAsync(dist2, d_dist, sizeof(float) * 2 * (size_t)nq, cudaMemcpyDeviceToHost, ctx->stream));
     ERP_CUDA(cudaStreamSynchronize(ctx->stream));
     return ERP_OK;
 }
 
+ERP_API int erp_knn2_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
+                         int32_t* d_idx2, float* d_dist2, double* d_d2)
+{
+    return knn2_dev("erp_knn2_dev", ctx, RowKind::f32(dim), d_q, nq, d_t, nt, d_idx2, d_dist2, d_d2);
+}
+
+ERP_API int erp_nn1_reverse_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
+                                int q_offset, int32_t* d_best_q, double* d_best_d2)
+{
+    ERP_ARG(ctx && nq >= 1 && nt >= 0 && d_best_q, ERP_E_ARG, "erp_nn1_reverse_dev: bad argument");
+    ERP_TRY(RowKind::f32(dim).check_dim("erp_nn1_reverse_dev"));
+    if (nt == 0) return ERP_OK;
+    DeviceGuard g(ctx->device);
+    return knn1_reverse(ctx, RowKind::f32(dim), d_q, nq, d_t, nt, q_offset, d_best_q, d_best_d2);
+}
+
+ERP_API int erp_knn2_match_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim,
+                               float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
+{
+    return knn2_match_dev("erp_knn2_match_dev", ctx, RowKind::f32(dim), d_q, nq, d_t, nt, ratio, cross_check, d_out, d_n_out);
+}
+
+ERP_API int erp_knn2_match(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes,
+                           const float* t, int nt, size_t t_stride_bytes, int dim,
+                           float ratio, int cross_check, erp_dmatch* out, int* n_out)
+{
+    return knn2_match_host("erp_knn2_match", ctx, RowKind::f32(dim), q, nq, q_stride_bytes, t, nt, t_stride_bytes, ratio, cross_check,
+                           out, n_out);
+}
+
+ERP_API int erp_knn2_raw(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes,
+                         const float* t, int nt, size_t t_stride_bytes, int dim,
+                         int32_t* idx2, float* dist2)
+{
+    return knn2_raw_host("erp_knn2_raw", ctx, RowKind::f32(dim), q, nq, q_stride_bytes, t, nt, t_stride_bytes, idx2, dist2);
+}
+
 ERP_API int erp_knn2_near_ties(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes,
                                const float* t, int nt, size_t t_stride_bytes, int dim, float rel_tol,
                                uint8_t* flags, int* n_flagged)
 {
-    ERP_TRY(check_knn_args("erp_knn2_near_ties", ctx, nq, nt, dim));
+    ERP_TRY(check_knn_args("erp_knn2_near_ties", ctx, nq, nt, RowKind::f32(dim)));
     ERP_ARG(n_flagged && rel_tol >= 0.f, ERP_E_ARG, "erp_knn2_near_ties: bad argument");
     *n_flagged = 0;
     if (nq == 0) return ERP_OK;
@@ -681,8 +721,8 @@ ERP_API int erp_knn2_near_ties(erp_ctx* ctx, const float* q, int nq, size_t q_st
     float* dq = ctx->scratch<float>(S_Q, (size_t)nq * dim + 4, &st);
     float* dt = ctx->scratch<float>(S_T, (size_t)nt * dim + 4, &st);
     ERP_TRY(st);
-    ERP_TRY(upload_rows(ctx, dt, t, nt, row, t_stride_bytes));
-    ERP_TRY(upload_rows(ctx, dq, q, nq, row, q_stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, dt, t, nt, row, t_stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, dq, q, nq, row, q_stride_bytes));
     ERP_TRY(erp_knn2_dev(ctx, dq, nq, dt, nt, dim, d_idx, d_dist, d_d2));
     ERP_TRY(near_ties(ctx, dq, nq, dt, nt, dim, d_idx, d_d2, (double)rel_tol, d_third, d_flags));
     int32_t n = 0;
@@ -693,129 +733,31 @@ ERP_API int erp_knn2_near_ties(erp_ctx* ctx, const float* q, int nq, size_t q_st
     return ERP_OK;
 }
 
-// ======================================================================================
-// binary descriptors (knn_bin.cu): feature_matcher::match_two_image with NORM_HAMMING
-// ======================================================================================
-static int check_bin_args(const char* who, erp_ctx* ctx, int nq, int nt, int nbytes)
-{
-    ERP_ARG(ctx, ERP_E_ARG, "%s: null context", who);
-    ERP_ARG(nq >= 0 && nt >= 0, ERP_E_ARG, "%s: negative size", who);
-    ERP_ARG(nbytes >= 1 && nbytes <= 64, ERP_E_DIM, "%s: binary descriptor size %d must be in [1,64] bytes", who, nbytes);
-    ERP_ARG(nq == 0 || nt >= 2, ERP_E_TOO_FEW_TRAIN, "%s: k=2 needs at least 2 train descriptors, got %d", who, nt);
-    return ERP_OK;
-}
-
-// both tensor engine settings select the kind::i8 engine; AUTO takes it where it is faster than SIMT
-static bool bin_uses_tc(erp_ctx* ctx, int nq, int nt)
-{
-    return ctx->engine == ERP_ENGINE_TCGEN05 || ctx->engine == ERP_ENGINE_TCGEN05_1X ||
-           (ctx->engine == ERP_ENGINE_AUTO && knn2_bin_preferred(nq, nt));
-}
-
 ERP_API int erp_knn2_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes,
                              int32_t* d_idx2, float* d_dist2, double* d_d2)
 {
-    ERP_TRY(check_bin_args("erp_knn2_bin_dev", ctx, nq, nt, nbytes));
-    if (nq == 0) return ERP_OK;
-    ERP_ARG(d_q && d_t, ERP_E_ARG, "erp_knn2_bin_dev: null descriptors");
-    DeviceGuard g(ctx->device);
-    return knn2_bin(ctx, d_q, nq, d_t, nt, nbytes, bin_uses_tc(ctx, nq, nt), d_idx2, d_dist2, d_d2);
-}
-
-// cross-check: nearest query of every train row (roles swapped, lowest query index on ties), compacted to the first neighbour
-static int bin_reverse(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, int32_t* d_best_q)
-{
-    int st = ERP_OK;
-    int32_t* idx2 = ctx->scratch<int32_t>(S_RS_IDX, (size_t)nt * 2, &st);
-    ERP_TRY(st);
-    ERP_TRY(knn2_bin(ctx, d_t, nt, d_q, nq, nbytes, bin_uses_tc(ctx, nt, nq), idx2, nullptr, nullptr));
-    ERP_CUDA(cudaMemcpy2DAsync(d_best_q, sizeof(int32_t), idx2, 2 * sizeof(int32_t), sizeof(int32_t), nt,
-                               cudaMemcpyDeviceToDevice, ctx->stream));
-    return ERP_OK;
+    return knn2_dev("erp_knn2_bin_dev", ctx, RowKind::binary(nbytes), d_q, nq, d_t, nt, d_idx2, d_dist2, d_d2);
 }
 
 ERP_API int erp_knn2_match_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes,
                                    float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
 {
-    ERP_TRY(check_bin_args("erp_knn2_match_bin_dev", ctx, nq, nt, nbytes));
-    ERP_ARG(d_n_out, ERP_E_ARG, "erp_knn2_match_bin_dev: d_n_out is null");
-    DeviceGuard g(ctx->device);
-    int st = ERP_OK;
-    int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
-    float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
-    ERP_TRY(st);
-    ERP_TRY(erp_knn2_bin_dev(ctx, d_q, nq, d_t, nt, nbytes, idx2, dist2, nullptr));
-    int32_t* rev = nullptr;
-    if (cross_check && nq > 0) {
-        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
-        ERP_TRY(st);
-        ERP_TRY(bin_reverse(ctx, d_q, nq, d_t, nt, nbytes, rev));
-    }
-    return erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n_out);
-}
-
-// host rows -> S_Q / S_T (dense) and the 2-NN, chunked like the float rows.  One engine for the whole call: the i8
-// operand of the train rows is prepared by the first query chunk only.
-static int knn2_bin_host(erp_ctx* ctx, const uint8_t* q, int nq, size_t qs, const uint8_t* t, int nt, size_t ts, int nbytes,
-                         int32_t* d_idx2, float* d_dist2)
-{
-    ERP_ARG((nq == 0 || q) && (nt == 0 || t), ERP_E_ARG, "null descriptor pointer");
-    ERP_ARG(qs >= (size_t)nbytes && ts >= (size_t)nbytes, ERP_E_ARG, "row stride smaller than a descriptor row (%zu < %d)",
-            qs < ts ? qs : ts, nbytes);
-    int st = ERP_OK;
-    uint8_t* dq = ctx->scratch<uint8_t>(S_Q, (size_t)nq * nbytes + 16, &st);
-    uint8_t* dt = ctx->scratch<uint8_t>(S_T, (size_t)nt * nbytes + 16, &st);
-    ERP_TRY(st);
-    const bool tc = bin_uses_tc(ctx, nq, nt);
-    return knn2_host_rows(ctx, q, nq, qs, t, nt, ts, (size_t)nbytes, dq, dt,
-                          [&](const void* cq, int n, int32_t* i2, float* d2) {
-                              return knn2_bin(ctx, static_cast<const uint8_t*>(cq), n, dt, nt, nbytes, tc, i2, d2, nullptr);
-                          }, d_idx2, d_dist2);
+    return knn2_match_dev("erp_knn2_match_bin_dev", ctx, RowKind::binary(nbytes), d_q, nq, d_t, nt, ratio, cross_check, d_out, d_n_out);
 }
 
 ERP_API int erp_knn2_match_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes,
                                const uint8_t* t, int nt, size_t t_stride_bytes, int nbytes,
                                float ratio, int cross_check, erp_dmatch* out, int* n_out)
 {
-    ERP_TRY(check_bin_args("erp_knn2_match_bin", ctx, nq, nt, nbytes));
-    ERP_ARG(n_out, ERP_E_ARG, "erp_knn2_match_bin: n_out is null");
-    *n_out = 0;
-    if (nq == 0) return ERP_OK;
-    ERP_ARG(out, ERP_E_ARG, "erp_knn2_match_bin: out is null");
-    DeviceGuard g(ctx->device);
-    int st = ERP_OK;
-    erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
-    int32_t* d_n = ctx->scratch<int32_t>(S_NOUT, 4, &st);
-    int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
-    float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
-    ERP_TRY(st);
-    ERP_TRY(knn2_bin_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, nbytes, idx2, dist2));
-    int32_t* rev = nullptr;
-    if (cross_check) {
-        rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
-        ERP_TRY(st);
-        ERP_TRY(bin_reverse(ctx, ctx->dev[S_Q].as<uint8_t>(), nq, ctx->dev[S_T].as<uint8_t>(), nt, nbytes, rev));
-    }
-    ERP_TRY(erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n));
-    return download_matches(ctx, d_out, d_n, (size_t)nq, out, n_out);
+    return knn2_match_host("erp_knn2_match_bin", ctx, RowKind::binary(nbytes), q, nq, q_stride_bytes, t, nt, t_stride_bytes, ratio,
+                           cross_check, out, n_out);
 }
 
 ERP_API int erp_knn2_raw_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes,
                              const uint8_t* t, int nt, size_t t_stride_bytes, int nbytes,
                              int32_t* idx2, float* dist2)
 {
-    ERP_TRY(check_bin_args("erp_knn2_raw_bin", ctx, nq, nt, nbytes));
-    if (nq == 0) return ERP_OK;
-    DeviceGuard g(ctx->device);
-    int st = ERP_OK;
-    int32_t* d_idx = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
-    float* d_dist = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
-    ERP_TRY(st);
-    ERP_TRY(knn2_bin_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, nbytes, d_idx, d_dist));
-    if (idx2) ERP_CUDA(cudaMemcpyAsync(idx2, d_idx, sizeof(int32_t) * 2 * (size_t)nq, cudaMemcpyDeviceToHost, ctx->stream));
-    if (dist2) ERP_CUDA(cudaMemcpyAsync(dist2, d_dist, sizeof(float) * 2 * (size_t)nq, cudaMemcpyDeviceToHost, ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
-    return ERP_OK;
+    return knn2_raw_host("erp_knn2_raw_bin", ctx, RowKind::binary(nbytes), q, nq, q_stride_bytes, t, nt, t_stride_bytes, idx2, dist2);
 }
 
 // ======================================================================================
@@ -833,7 +775,7 @@ ERP_API int erp_bearings_from_pixels(erp_ctx* ctx, const void* xy, size_t stride
     float* d_xy = ctx->scratch<float>(S_XY, (size_t)n * 2, &st);
     double* d_o = ctx->scratch<double>(S_L3, (size_t)n * 3, &st);
     ERP_TRY(st);
-    ERP_TRY(upload_rows(ctx, d_xy, xy, n, 8, stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy, xy, n, 8, stride_bytes));
     ERP_TRY(erp_bearings_dev(ctx, d_xy, 8, n, width, height, d_o, nullptr));
     ERP_CUDA(cudaMemcpyAsync(out3, d_o, sizeof(double) * 3 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     ERP_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1013,14 +955,14 @@ void graph_release(erp_ctx* ctx)
     ctx->graph = nullptr;
 }
 
-int graph_run(erp_ctx* ctx, const void* key, size_t key_bytes, const std::function<int()>& body)
+int graph_run(erp_ctx* ctx, const PairKey& key, const std::function<int()>& body)
 {
     static const bool off = [] { const char* e = getenv("ERP_B200_GRAPH"); return e && atoi(e) == 0; }();
     if (off) return body();
     if (!ctx->graph) ctx->graph = new GraphCache();
     GraphCache& g = *ctx->graph;
     if (g.disabled) return body();
-    std::vector<uint8_t> k((const uint8_t*)key, (const uint8_t*)key + key_bytes);
+    std::vector<uint8_t> k((const uint8_t*)&key, (const uint8_t*)&key + sizeof key);
     const void* extra[2] = {(const void*)(intptr_t)ctx->engine, (const void*)ctx->comm};
     k.insert(k.end(), (const uint8_t*)extra, (const uint8_t*)extra + sizeof extra);
     if (g.exec && g.key == k && g.key_gen == ctx->scratch_gen) {
@@ -1102,7 +1044,7 @@ int pose_chain_buffers(erp_ctx* ctx, int m_cap, PoseBuffers* b)
 
 } // namespace erp
 
-static int check_ransac_args(const char* who, erp_ctx* ctx, int H, int S, int metric, uint64_t hyp_offset)
+int erp::check_ransac_args(const char* who, erp_ctx* ctx, int H, int S, int metric, uint64_t hyp_offset)
 {
     ERP_ARG(ctx && H >= 1, ERP_E_ARG, "%s: bad argument", who);
     ERP_ARG(S >= 8 && S <= 32, ERP_E_ARG, "%s: sample size must be in [8,32], got %d", who, S);
@@ -1146,8 +1088,8 @@ ERP_API int erp_ransac_pixels(erp_ctx* ctx, int width, int height, const void* l
     ERP_TRY(st);
     PoseBuffers b;
     ERP_TRY(pose_chain_buffers(ctx, m, &b));
-    ERP_TRY(upload_rows(ctx, d_xy, left_xy, m, 8, stride_bytes));
-    ERP_TRY(upload_rows(ctx, d_xy + (size_t)m * 2, right_xy, m, 8, stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy, left_xy, m, 8, stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy + (size_t)m * 2, right_xy, m, 8, stride_bytes));
     const bool tc = ransac_uses_tc(ctx, H, m, metric);
     ScoreTcBuffers sb = {};
     if (tc) {
@@ -1163,25 +1105,118 @@ ERP_API int erp_ransac_pixels(erp_ctx* ctx, int width, int height, const void* l
 }
 
 // gather + bearings -> hypothesis search -> mask + refit on the device-resident match list of a pair (stage events 2, 3)
-static int pose_after_match(erp_ctx* ctx, const erp_dmatch* d_matches, int nq, const int32_t* d_n_matches,
-                            const void* d_left_xy, const void* d_right_xy, size_t kp_stride_bytes, int width, int height,
-                            uint64_t seed, int H, int S, int metric, float tau, uint8_t* d_mask, erp_ransac_result* d_result)
+static int pose_after_match(erp_ctx* ctx, int nq, const PairArgs& a)
 {
     PoseBuffers b;
     ERP_TRY(pose_chain_buffers(ctx, nq, &b));
-    const bool tc = ransac_uses_tc(ctx, H, nq, metric);
+    const bool tc = ransac_uses_tc(ctx, a.H, nq, a.metric);
     ScoreTcBuffers sb = {};
     if (tc) {
-        ERP_TRY(score_tc_buffers(ctx, H < RANSAC_CHUNK ? H : RANSAC_CHUNK, nq, &sb));
+        ERP_TRY(score_tc_buffers(ctx, a.H < RANSAC_CHUNK ? a.H : RANSAC_CHUNK, nq, &sb));
         ERP_CUDA(cudaMemsetAsync(sb.w, 0, W_WORDS_BYTES, ctx->stream));
     }
-    ERP_TRY(gather_bearings_chain(ctx, d_matches, nq, d_n_matches, d_left_xy, d_right_xy, kp_stride_bytes, 0, width, height,
+    ERP_TRY(gather_bearings_chain(ctx, a.matches, nq, a.n_matches, a.left_xy, a.right_xy, a.kp_stride, 0, a.width, a.height,
                                   b.l3, b.r3, b.l4, b.r4, sb.Ks, sb.w));
     ERP_CUDA(record_timing(ctx, ctx->ev_stage[2]));
-    ERP_TRY(pose_chain_tail(ctx, b.l3, b.r3, b.l4, b.r4, nq, d_n_matches, seed, 0, H, S, metric, tau, tc, false,
-                            d_mask ? d_mask : b.mask, d_result));
+    ERP_TRY(pose_chain_tail(ctx, b.l3, b.r3, b.l4, b.r4, nq, a.n_matches, a.seed, 0, a.H, a.S, a.metric, a.tau, tc, false,
+                            a.mask ? a.mask : b.mask, a.result));
     ERP_CUDA(record_timing(ctx, ctx->ev_stage[3]));
     return ERP_OK;
+}
+
+// the checks every pair call makes before its own
+static int check_pair_args(const char* who, erp_ctx* ctx, RowKind k, int nq, int nt, const PairArgs& a)
+{
+    ERP_TRY(check_knn_args(who, ctx, nq, nt, k));
+    ERP_TRY(check_ransac_args(who, ctx, a.H, a.S, a.metric, 0));
+    ERP_ARG(a.matches && a.n_matches && a.result && a.width > 0 && a.height > 0, ERP_E_ARG, "%s: bad argument", who);
+    ERP_ARG(a.left_xy && a.right_xy && a.kp_stride >= 8 && a.kp_stride % 4 == 0, ERP_E_ARG, "%s: bad keypoints", who);
+    return ERP_OK;
+}
+
+static int pair_pose_dev(const char* who, erp_ctx* ctx, RowKind k, const void* d_q, int nq, const void* d_t, int nt, const PairArgs& a)
+{
+    ERP_TRY(check_pair_args(who, ctx, k, nq, nt, a));
+    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "%s: no query descriptors", who);
+    DeviceGuard g(ctx->device);
+    return graph_run(ctx, {k.bin ? PAIR_BIN : PAIR_F32, d_q, d_t, nq, nt, k.dim, a}, [&]() -> int {
+    ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
+    ERP_TRY(knn2_match_dev(who, ctx, k, d_q, nq, d_t, nt, a.ratio, a.cross_check, a.matches, a.n_matches));
+    ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
+    return pose_after_match(ctx, nq, a);
+    });
+}
+
+int erp::pair_pose_download(erp_ctx* ctx, const char* who, cudaEvent_t ready, const PairArgs& dev, const PairArgs& out)
+{
+    // everything is enqueued: the host waits for the match list only (the pose chain keeps running), learns the match
+    // count and brings the records back on the copy stream while the hypotheses are being scored
+    int32_t n = 0;
+    ERP_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ready, 0));
+    ERP_CUDA(cudaMemcpyAsync(&n, dev.n_matches, sizeof n, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
+    *out.n_matches = n;
+    if (n > 0) ERP_CUDA(cudaMemcpyAsync(out.matches, dev.matches, sizeof(erp_dmatch) * (size_t)n, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    ERP_CUDA(cudaMemcpyAsync(out.result, dev.result, sizeof *out.result, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out.mask && n > 0) ERP_CUDA(cudaMemcpyAsync(out.mask, dev.mask, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
+    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
+    if (n < out.S) {
+        set_error("%s: %d matches for sample size %d", who, n, out.S);
+        return ERP_E_TOO_FEW_POINTS;
+    }
+    return ERP_OK;
+}
+
+static int pair_pose_host(const char* who, erp_ctx* ctx, RowKind k, const void* q, int nq, size_t qs, const void* t, int nt, size_t ts,
+                          const PairArgs& a)
+{
+    ERP_TRY(check_pair_args(who, ctx, k, nq, nt, a));
+    *a.n_matches = 0;
+    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "%s: no query descriptors", who);
+    const size_t row = k.row_bytes();
+    ERP_ARG(q && t && qs >= row && ts >= row, ERP_E_ARG, "%s: bad descriptor buffers", who);
+    DeviceGuard g(ctx->device);
+    int st = ERP_OK;
+    PairArgs dev = a;
+    dev.matches = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
+    dev.n_matches = ctx->scratch<int32_t>(S_NOUT, 4, &st);
+    float* d_xy = ctx->scratch<float>(S_XY, ((size_t)nq + nt) * 2, &st);           // left pairs, then right pairs
+    dev.left_xy = d_xy;
+    dev.right_xy = d_xy + (size_t)nq * 2;
+    dev.kp_stride = 8;
+    uint8_t* dq = ctx->scratch<uint8_t>(S_Q, (size_t)nq * row + 16, &st);
+    uint8_t* dt = ctx->scratch<uint8_t>(S_T, (size_t)nt * row + 16, &st);
+    PoseBuffers b;
+    ERP_TRY(pose_chain_buffers(ctx, nq, &b));
+    ERP_TRY(st);
+    dev.mask = b.mask;
+    dev.result = b.res;
+    int bounds[9];
+    // binary pairs are not chunked: the cut of chunk_bounds was tuned for 256-byte float rows
+    if (!k.bin && chunk_bounds(nq, nt, is_pageable(q), bounds) > 1) {
+        // large pair: the descriptors travel in chunks behind the search (knn2_host), the keypoints follow on the copy
+        // stream and are awaited by the gather; the chain is enqueued directly (launch cost hides behind the uploads)
+        int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
+        float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
+        ERP_TRY(st);
+        ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
+        ERP_TRY(knn2_host(ctx, k, q, nq, qs, t, nt, ts, idx2, dist2));
+        ERP_TRY(upload_rows(ctx, ctx->copy_stream, d_xy, a.left_xy, nq, 8, a.kp_stride));
+        ERP_TRY(upload_rows(ctx, ctx->copy_stream, d_xy + (size_t)nq * 2, a.right_xy, nt, 8, a.kp_stride));
+        ERP_CUDA(cudaEventRecord(ctx->ev_copy[9], ctx->copy_stream));
+        ERP_TRY(filter_matches(ctx, k, dq, nq, dt, nt, idx2, dist2, a.ratio, a.cross_check, dev.matches, dev.n_matches));
+        ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
+        ERP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy[9], 0));
+        ERP_TRY(pose_after_match(ctx, nq, dev));
+    } else {
+        ERP_TRY(upload_rows(ctx, ctx->stream, dt, t, nt, row, ts));
+        ERP_TRY(upload_rows(ctx, ctx->stream, dq, q, nq, row, qs));
+        ERP_TRY(upload_rows(ctx, ctx->stream, d_xy, a.left_xy, nq, 8, a.kp_stride));
+        ERP_TRY(upload_rows(ctx, ctx->stream, d_xy + (size_t)nq * 2, a.right_xy, nt, 8, a.kp_stride));
+        ERP_TRY(pair_pose_dev(who, ctx, k, dq, nq, dt, nt, dev));
+    }
+    return pair_pose_download(ctx, who, ctx->ev_stage[1], dev, a);
 }
 
 ERP_API int erp_pair_pose_dev(erp_ctx* ctx, const float* d_q, int nq, const float* d_t, int nt, int dim, float ratio, int cross_check,
@@ -1189,42 +1224,9 @@ ERP_API int erp_pair_pose_dev(erp_ctx* ctx, const float* d_q, int nq, const floa
                               uint64_t seed, int H, int S, int metric, float tau,
                               erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result)
 {
-    ERP_TRY(check_knn_args("erp_pair_pose_dev", ctx, nq, nt, dim));
-    ERP_TRY(check_ransac_args("erp_pair_pose_dev", ctx, H, S, metric, 0));
-    ERP_ARG(d_matches && d_n_matches && d_result && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose_dev: bad argument");
-    ERP_ARG(d_left_xy && d_right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose_dev: bad keypoints");
-    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "erp_pair_pose_dev: no query descriptors");
-    DeviceGuard g(ctx->device);
-    const uint64_t key[] = {(uint64_t)(uintptr_t)d_q, (uint64_t)(uintptr_t)d_t, (uint64_t)(uintptr_t)d_left_xy, (uint64_t)(uintptr_t)d_right_xy, (uint64_t)(uintptr_t)d_matches, (uint64_t)(uintptr_t)d_n_matches, (uint64_t)(uintptr_t)d_mask, (uint64_t)(uintptr_t)d_result, (uint64_t)nq, (uint64_t)nt, (uint64_t)dim, (uint64_t)cross_check, (uint64_t)width, (uint64_t)height, (uint64_t)H, (uint64_t)S, (uint64_t)metric, (uint64_t)__builtin_bit_cast(uint32_t, ratio), (uint64_t)__builtin_bit_cast(uint32_t, tau), (uint64_t)seed, (uint64_t)kp_stride_bytes};      // every argument, no padding bytes
-    return graph_run(ctx, key, sizeof key, [&]() -> int {
-    ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
-    ERP_TRY(erp_knn2_match_dev(ctx, d_q, nq, d_t, nt, dim, ratio, cross_check, d_matches, d_n_matches));
-    ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
-    return pose_after_match(ctx, d_matches, nq, d_n_matches, d_left_xy, d_right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
-                            d_mask, d_result);
-    });
-}
-
-// everything is enqueued: the host waits for the MATCH stage only (the pose chain keeps running), learns the match
-// count and brings the records back on the copy stream while the hypotheses are being scored
-static int pair_pose_download(erp_ctx* ctx, const char* who, const erp_dmatch* d_out, const int32_t* d_n, const PoseBuffers& b, int S,
-                              erp_dmatch* matches_out, int* n_matches, erp_ransac_result* result, uint8_t* mask)
-{
-    int32_t n = 0;
-    ERP_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_stage[1], 0));
-    ERP_CUDA(cudaMemcpyAsync(&n, d_n, sizeof n, cudaMemcpyDeviceToHost, ctx->copy_stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
-    *n_matches = n;
-    if (n > 0) ERP_CUDA(cudaMemcpyAsync(matches_out, d_out, sizeof(erp_dmatch) * (size_t)n, cudaMemcpyDeviceToHost, ctx->copy_stream));
-    ERP_CUDA(cudaMemcpyAsync(result, b.res, sizeof *result, cudaMemcpyDeviceToHost, ctx->stream));
-    if (mask && n > 0) ERP_CUDA(cudaMemcpyAsync(mask, b.mask, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
-    if (n < S) {
-        set_error("%s: %d matches for sample size %d", who, n, S);
-        return ERP_E_TOO_FEW_POINTS;
-    }
-    return ERP_OK;
+    return pair_pose_dev("erp_pair_pose_dev", ctx, RowKind::f32(dim), d_q, nq, d_t, nt,
+                         {ratio, cross_check, d_left_xy, d_right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
+                          d_matches, d_n_matches, d_mask, d_result});
 }
 
 ERP_API int erp_pair_pose(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes, const float* t, int nt, size_t t_stride_bytes,
@@ -1233,60 +1235,9 @@ ERP_API int erp_pair_pose(erp_ctx* ctx, const float* q, int nq, size_t q_stride_
                           uint64_t seed, int H, int S, int metric, float tau,
                           erp_dmatch* matches_out, int* n_matches, erp_ransac_result* result, uint8_t* mask)
 {
-    ERP_TRY(check_knn_args("erp_pair_pose", ctx, nq, nt, dim));
-    ERP_TRY(check_ransac_args("erp_pair_pose", ctx, H, S, metric, 0));
-    ERP_ARG(n_matches && result && matches_out && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose: bad argument");
-    ERP_ARG(left_xy && right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose: bad keypoints");
-    *n_matches = 0;
-    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "erp_pair_pose: no query descriptors");
-    const size_t row = (size_t)dim * sizeof(float);
-    ERP_ARG(q && t && q_stride_bytes >= row && t_stride_bytes >= row, ERP_E_ARG, "erp_pair_pose: bad descriptor buffers");
-    DeviceGuard g(ctx->device);
-    int st = ERP_OK;
-    erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
-    int32_t* d_n = ctx->scratch<int32_t>(S_NOUT, 4, &st);
-    float* d_xy = ctx->scratch<float>(S_XY, ((size_t)nq + nt) * 2, &st);           // left pairs, then right pairs
-    float* dq = ctx->scratch<float>(S_Q, (size_t)nq * dim + 4, &st);
-    float* dt = ctx->scratch<float>(S_T, (size_t)nt * dim + 4, &st);
-    PoseBuffers b;
-    ERP_TRY(pose_chain_buffers(ctx, nq, &b));
-    ERP_TRY(st);
-    int bounds[9];
-    if (chunk_bounds(nq, nt, is_pageable(q), bounds) > 1) {
-        // large pair: the descriptors travel in chunks behind the search (knn2_host), the keypoints follow on the copy
-        // stream and are awaited by the gather; the chain is enqueued directly (launch cost hides behind the uploads)
-        int32_t* idx2 = ctx->scratch<int32_t>(S_IDX2, (size_t)nq * 2 + 2, &st);
-        float* dist2 = ctx->scratch<float>(S_DIST2, (size_t)nq * 2 + 2, &st);
-        ERP_TRY(st);
-        ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
-        ERP_TRY(knn2_host(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, dim, idx2, dist2));
-        {
-            cudaStream_t main_stream = ctx->stream;
-            struct Swap { erp_ctx* c; cudaStream_t m; ~Swap() { c->stream = m; } } sw{ctx, main_stream};
-            ctx->stream = ctx->copy_stream;
-            ERP_TRY(upload_rows(ctx, d_xy, left_xy, nq, 8, kp_stride_bytes));
-            ERP_TRY(upload_rows(ctx, d_xy + (size_t)nq * 2, right_xy, nt, 8, kp_stride_bytes));
-            ERP_CUDA(cudaEventRecord(ctx->ev_copy[9], ctx->copy_stream));
-        }
-        int32_t* rev = nullptr;
-        if (cross_check) {
-            rev = ctx->scratch<int32_t>(S_REVQ, (size_t)nt, &st);
-            ERP_TRY(st);
-            ERP_TRY(erp_nn1_reverse_dev(ctx, dq, nq, dt, nt, dim, 0, rev, nullptr));
-        }
-        ERP_TRY(erp_match_filter_dev(ctx, idx2, dist2, nq, ratio, rev, 0, d_out, d_n));
-        ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
-        ERP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy[9], 0));
-        ERP_TRY(pose_after_match(ctx, d_out, nq, d_n, d_xy, d_xy + (size_t)nq * 2, 8, width, height, seed, H, S, metric, tau, b.mask, b.res));
-    } else {
-        ERP_TRY(upload_rows(ctx, dt, t, nt, row, t_stride_bytes));
-        ERP_TRY(upload_rows(ctx, dq, q, nq, row, q_stride_bytes));
-        ERP_TRY(upload_rows(ctx, d_xy, left_xy, nq, 8, kp_stride_bytes));
-        ERP_TRY(upload_rows(ctx, d_xy + (size_t)nq * 2, right_xy, nt, 8, kp_stride_bytes));
-        ERP_TRY(erp_pair_pose_dev(ctx, dq, nq, dt, nt, dim, ratio, cross_check, d_xy, d_xy + (size_t)nq * 2, 8, width, height,
-                                  seed, H, S, metric, tau, d_out, d_n, b.mask, b.res));
-    }
-    return pair_pose_download(ctx, "erp_pair_pose", d_out, d_n, b, S, matches_out, n_matches, result, mask);
+    return pair_pose_host("erp_pair_pose", ctx, RowKind::f32(dim), q, nq, q_stride_bytes, t, nt, t_stride_bytes,
+                          {ratio, cross_check, left_xy, right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
+                           matches_out, n_matches, mask, result});
 }
 
 ERP_API int erp_pair_pose_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, int nbytes, float ratio,
@@ -1294,21 +1245,9 @@ ERP_API int erp_pair_pose_bin_dev(erp_ctx* ctx, const uint8_t* d_q, int nq, cons
                                   int height, uint64_t seed, int H, int S, int metric, float tau,
                                   erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result)
 {
-    ERP_TRY(check_bin_args("erp_pair_pose_bin_dev", ctx, nq, nt, nbytes));
-    ERP_TRY(check_ransac_args("erp_pair_pose_bin_dev", ctx, H, S, metric, 0));
-    ERP_ARG(d_matches && d_n_matches && d_result && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose_bin_dev: bad argument");
-    ERP_ARG(d_left_xy && d_right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose_bin_dev: bad keypoints");
-    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "erp_pair_pose_bin_dev: no query descriptors");
-    DeviceGuard g(ctx->device);
-    // the leading tag keeps the graph of this call apart from erp_pair_pose_dev's with the same pointers and sizes
-    const uint64_t key[] = {0x48414d4d494e47ull, (uint64_t)(uintptr_t)d_q, (uint64_t)(uintptr_t)d_t, (uint64_t)(uintptr_t)d_left_xy, (uint64_t)(uintptr_t)d_right_xy, (uint64_t)(uintptr_t)d_matches, (uint64_t)(uintptr_t)d_n_matches, (uint64_t)(uintptr_t)d_mask, (uint64_t)(uintptr_t)d_result, (uint64_t)nq, (uint64_t)nt, (uint64_t)nbytes, (uint64_t)cross_check, (uint64_t)width, (uint64_t)height, (uint64_t)H, (uint64_t)S, (uint64_t)metric, (uint64_t)__builtin_bit_cast(uint32_t, ratio), (uint64_t)__builtin_bit_cast(uint32_t, tau), (uint64_t)seed, (uint64_t)kp_stride_bytes};
-    return graph_run(ctx, key, sizeof key, [&]() -> int {
-    ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
-    ERP_TRY(erp_knn2_match_bin_dev(ctx, d_q, nq, d_t, nt, nbytes, ratio, cross_check, d_matches, d_n_matches));
-    ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
-    return pose_after_match(ctx, d_matches, nq, d_n_matches, d_left_xy, d_right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
-                            d_mask, d_result);
-    });
+    return pair_pose_dev("erp_pair_pose_bin_dev", ctx, RowKind::binary(nbytes), d_q, nq, d_t, nt,
+                         {ratio, cross_check, d_left_xy, d_right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
+                          d_matches, d_n_matches, d_mask, d_result});
 }
 
 ERP_API int erp_pair_pose_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_stride_bytes, const uint8_t* t, int nt,
@@ -1317,31 +1256,9 @@ ERP_API int erp_pair_pose_bin(erp_ctx* ctx, const uint8_t* q, int nq, size_t q_s
                               uint64_t seed, int H, int S, int metric, float tau,
                               erp_dmatch* matches_out, int* n_matches, erp_ransac_result* result, uint8_t* mask)
 {
-    ERP_TRY(check_bin_args("erp_pair_pose_bin", ctx, nq, nt, nbytes));
-    ERP_TRY(check_ransac_args("erp_pair_pose_bin", ctx, H, S, metric, 0));
-    ERP_ARG(n_matches && result && matches_out && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose_bin: bad argument");
-    ERP_ARG(left_xy && right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose_bin: bad keypoints");
-    *n_matches = 0;
-    ERP_ARG(nq >= 1, ERP_E_TOO_FEW_POINTS, "erp_pair_pose_bin: no query descriptors");
-    ERP_ARG(q && t && q_stride_bytes >= (size_t)nbytes && t_stride_bytes >= (size_t)nbytes, ERP_E_ARG,
-            "erp_pair_pose_bin: bad descriptor buffers");
-    DeviceGuard g(ctx->device);
-    int st = ERP_OK;
-    erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
-    int32_t* d_n = ctx->scratch<int32_t>(S_NOUT, 4, &st);
-    float* d_xy = ctx->scratch<float>(S_XY, ((size_t)nq + nt) * 2, &st);           // left pairs, then right pairs
-    uint8_t* dq = ctx->scratch<uint8_t>(S_Q, (size_t)nq * nbytes + 16, &st);
-    uint8_t* dt = ctx->scratch<uint8_t>(S_T, (size_t)nt * nbytes + 16, &st);
-    PoseBuffers b;
-    ERP_TRY(pose_chain_buffers(ctx, nq, &b));
-    ERP_TRY(st);
-    ERP_TRY(upload_rows(ctx, dt, t, nt, (size_t)nbytes, t_stride_bytes));
-    ERP_TRY(upload_rows(ctx, dq, q, nq, (size_t)nbytes, q_stride_bytes));
-    ERP_TRY(upload_rows(ctx, d_xy, left_xy, nq, 8, kp_stride_bytes));
-    ERP_TRY(upload_rows(ctx, d_xy + (size_t)nq * 2, right_xy, nt, 8, kp_stride_bytes));
-    ERP_TRY(erp_pair_pose_bin_dev(ctx, dq, nq, dt, nt, nbytes, ratio, cross_check, d_xy, d_xy + (size_t)nq * 2, 8, width, height,
-                                  seed, H, S, metric, tau, d_out, d_n, b.mask, b.res));
-    return pair_pose_download(ctx, "erp_pair_pose_bin", d_out, d_n, b, S, matches_out, n_matches, result, mask);
+    return pair_pose_host("erp_pair_pose_bin", ctx, RowKind::binary(nbytes), q, nq, q_stride_bytes, t, nt, t_stride_bytes,
+                          {ratio, cross_check, left_xy, right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
+                           matches_out, n_matches, mask, result});
 }
 
 // ======================================================================================
@@ -1477,8 +1394,8 @@ ERP_API int erp_find(erp_ctx* ctx, int width, int height, const void* left_xy, c
     ERP_TRY(st);
     PoseBuffers b;
     ERP_TRY(pose_chain_buffers(ctx, match_size, &b));
-    ERP_TRY(upload_rows(ctx, d_xy, left_xy, match_size, 8, stride_bytes));
-    ERP_TRY(upload_rows(ctx, d_xy + (size_t)match_size * 2, right_xy, match_size, 8, stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy, left_xy, match_size, 8, stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy + (size_t)match_size * 2, right_xy, match_size, 8, stride_bytes));
     ERP_TRY(bearings_pair_chain(ctx, d_xy, d_xy + (size_t)match_size * 2, 8, match_size, width, height, b.l3, b.r3, b.l4, b.r4,
                                 nullptr, nullptr));
     return initial_guess_dev(ctx, b.l3, b.r3, match_size, samples, H, S, R_vec_out, T_vec_out, nullptr, nullptr, nullptr, nullptr);

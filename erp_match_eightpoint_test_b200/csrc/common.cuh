@@ -245,12 +245,60 @@ int pose_chain_buffers(erp_ctx* ctx, int m_cap, PoseBuffers* b);
 int pose_chain_tail(erp_ctx* ctx, const double* dl, const double* dr, const float* dl4, const float* dr4, int m_cap, const int32_t* d_m,
                     uint64_t seed, uint64_t hyp_offset, int H, int S, int metric, float tau, bool k_ready, bool reduce,
                     uint8_t* d_mask, erp_ransac_result* d_res);
-// graph cache (api.cu).  key: every argument of the call (bytes); body: enqueues the call on ctx->stream without
-// touching the host again.  The first call with a key runs directly, the second is captured, the rest replay.
-int graph_run(erp_ctx* ctx, const void* key, size_t key_bytes, const std::function<int()>& body);
+// ---- host entry points (api.cu): one implementation serves float and binary descriptors
+// A descriptor kind: float rows of `dim` values (L2) or binary rows of `dim` bytes (Hamming).
+struct RowKind {
+    bool bin;
+    int dim;
+    static RowKind f32(int dim) { return {false, dim}; }
+    static RowKind binary(int nbytes) { return {true, nbytes}; }
+    size_t row_bytes() const { return bin ? (size_t)dim : (size_t)dim * sizeof(float); }
+    int check_dim(const char* who) const;                          // ERP_E_DIM outside the kind's range
+    // engine of a search of nq rows against nt under ctx->engine: ERP_ENGINE_EXACT_SIMT, _TCGEN05 or _TCGEN05_1X.  Float
+    // rows on a shape a forced tensor engine cannot serve: ERP_E_DIM, or SIMT with `fallback` (the cross-check search).
+    int engine(erp_ctx* ctx, int nq, int nt, bool fallback, int* out) const;
+    // the 2-NN on that engine.  `forward`: the search of the query rows; float rows record the SIMT search's statistics
+    // and timing here (the other searches record their own), the cross-check search leaves them to the forward one.
+    int knn2(erp_ctx* ctx, int engine, bool forward, const void* d_q, int nq, const void* d_t, int nt,
+             int32_t* d_idx2, float* d_dist2, double* d_d2) const;
+};
+int check_knn_args(const char* who, erp_ctx* ctx, int nq, int nt, RowKind k);
+int check_ransac_args(const char* who, erp_ctx* ctx, int H, int S, int metric, uint64_t hyp_offset);
+// the keypoint, RANSAC and output arguments of a pair call (erp_pair_pose*), in the order of the C ABI: host pointers for
+// a host-buffer call, device pointers for a device call
+struct PairArgs {
+    float ratio;
+    int cross_check;
+    const void *left_xy, *right_xy;
+    size_t kp_stride;
+    int width, height;
+    uint64_t seed;
+    int H, S, metric;
+    float tau;
+    erp_dmatch* matches;
+    int32_t* n_matches;
+    uint8_t* mask;
+    erp_ransac_result* result;
+};
+// graph key of a device pair call: the entry's tag, then every argument.  It is compared bytewise: no padding bytes.
+enum PairEntry : uint64_t { PAIR_F32 = 1, PAIR_BIN, PAIR_DIST };
+struct PairKey {
+    uint64_t entry;
+    const void *q, *t;
+    int64_t nq, nt, dim;
+    PairArgs a;
+};
+static_assert(sizeof(PairArgs) == 8 * sizeof(uint64_t) + 8 * sizeof(int32_t) && sizeof(PairKey) == 6 * sizeof(uint64_t) + sizeof(PairArgs),
+              "a pair-call graph key must have no padding bytes");
+// graph cache (api.cu).  body: enqueues the call on ctx->stream without touching the host again.  The first call with a
+// key runs directly, the second is captured, the rest replay.
+int graph_run(erp_ctx* ctx, const PairKey& key, const std::function<int()>& body);
 void graph_release(erp_ctx* ctx);
+// host side of a pair call: waits for the stage event `ready` (the match list is final), brings back the matches (dev ->
+// out) and the result; ERP_E_TOO_FEW_POINTS below S matches
+int pair_pose_download(erp_ctx* ctx, const char* who, cudaEvent_t ready, const PairArgs& dev, const PairArgs& out);
 int download_matches(erp_ctx* ctx, const erp_dmatch* d_out, const int32_t* d_n, size_t cap, erp_dmatch* out, int* n_out);
-int upload_rows(erp_ctx* ctx, void* d_dst, const void* src, int rows, size_t row_bytes, size_t stride);
+int upload_rows(erp_ctx* ctx, cudaStream_t stream, void* d_dst, const void* src, int rows, size_t row_bytes, size_t stride);
 void stage_release(erp_ctx* ctx);
 // multi-GPU (dist.cu)
 int comm_allreduce_best(erp_ctx* ctx, uint64_t* d_packed);

@@ -421,39 +421,32 @@ ERP_API int erp_comm_cross_check_dev(erp_ctx* ctx, int32_t* d_best_q, double* d_
     return comm_cross_check(ctx, d_best_q, d_best_d2, nt);
 }
 
-ERP_API int erp_pair_pose_dist_dev(erp_ctx* ctx, const float* d_q_shard, int nq_total, const float* d_t, int nt, int dim,
-                                   float ratio, int cross_check,
-                                   const void* d_left_xy, const void* d_right_xy, size_t kp_stride_bytes, int width, int height,
-                                   uint64_t seed, int H_total, int S, int metric, float tau,
-                                   erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result)
+// the sharded pair on G > 1 ranks: checks, then match -> exchange -> gather -> hypothesis search -> mask + refit
+static int pair_pose_dist_dev(erp_ctx* ctx, const float* d_q_shard, int nq_total, const float* d_t, int nt, int dim, const PairArgs& a)
 {
-    ERP_ARG(ctx, ERP_E_ARG, "erp_pair_pose_dist_dev: null context");
+    const char* who = "erp_pair_pose_dist_dev";
     const int G = comm_size(ctx), rank = comm_rank(ctx);
-    if (G == 1)
-        return erp_pair_pose_dev(ctx, d_q_shard, nq_total, d_t, nt, dim, ratio, cross_check, d_left_xy, d_right_xy, kp_stride_bytes,
-                                 width, height, seed, H_total, S, metric, tau, d_matches, d_n_matches, d_mask, d_result);
-    ERP_ARG(nq_total >= 1 && nt >= 2, ERP_E_TOO_FEW_TRAIN, "erp_pair_pose_dist_dev: nq %d, nt %d", nq_total, nt);
-    ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "erp_pair_pose_dist_dev: descriptor dimension %d", dim);
-    ERP_ARG(d_t && d_matches && d_n_matches && d_result && width > 0 && height > 0, ERP_E_ARG, "erp_pair_pose_dist_dev: bad argument");
-    ERP_ARG(d_left_xy && d_right_xy && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG, "erp_pair_pose_dist_dev: bad keypoints");
-    ERP_ARG(S >= 8 && S <= 32 && metric >= 0 && metric <= 2, ERP_E_ARG, "erp_pair_pose_dist_dev: sample size / metric");
-    ERP_ARG(H_total >= G && (uint64_t)H_total <= 0xFFFFFFFFull, ERP_E_ARG, "erp_pair_pose_dist_dev: %d hypotheses for %d ranks", H_total, G);
+    ERP_ARG(nq_total >= 1 && nt >= 2, ERP_E_TOO_FEW_TRAIN, "%s: nq %d, nt %d", who, nq_total, nt);
+    ERP_TRY(RowKind::f32(dim).check_dim(who));
+    ERP_ARG(d_t && a.matches && a.n_matches && a.result && a.width > 0 && a.height > 0, ERP_E_ARG, "%s: bad argument", who);
+    ERP_ARG(a.left_xy && a.right_xy && a.kp_stride >= 8 && a.kp_stride % 4 == 0, ERP_E_ARG, "%s: bad keypoints", who);
+    ERP_TRY(check_ransac_args(who, ctx, a.H, a.S, a.metric, 0));
+    ERP_ARG(a.H >= G, ERP_E_ARG, "%s: %d hypotheses for %d ranks", who, a.H, G);
     DeviceGuard g(ctx->device);
     int lo, hi, hlo, hhi;
     shard_range(nq_total, rank, G, &lo, &hi);
-    shard_range(H_total, rank, G, &hlo, &hhi);
-    ERP_ARG(hi == lo || d_q_shard, ERP_E_ARG, "erp_pair_pose_dist_dev: null query shard");
-    const uint64_t key[] = {(uint64_t)(uintptr_t)d_q_shard, (uint64_t)(uintptr_t)d_t, (uint64_t)(uintptr_t)d_left_xy, (uint64_t)(uintptr_t)d_right_xy, (uint64_t)(uintptr_t)d_matches, (uint64_t)(uintptr_t)d_n_matches, (uint64_t)(uintptr_t)d_mask, (uint64_t)(uintptr_t)d_result, (uint64_t)nq_total, (uint64_t)nt, (uint64_t)dim, (uint64_t)cross_check, (uint64_t)width, (uint64_t)height, (uint64_t)H_total, (uint64_t)S, (uint64_t)metric, (uint64_t)__builtin_bit_cast(uint32_t, ratio), (uint64_t)__builtin_bit_cast(uint32_t, tau), (uint64_t)seed, (uint64_t)kp_stride_bytes};      // every argument, no padding bytes
+    shard_range(a.H, rank, G, &hlo, &hhi);
+    ERP_ARG(hi == lo || d_q_shard, ERP_E_ARG, "%s: null query shard", who);
     // slots of the match exchange: [header | up to cap records] per rank, in the peer window when there is one
     const int cap = cdiv(nq_total, G), slot = cap + 1;
     Comm* win = window_ensure(ctx, WindowLayout::SLOTS + (size_t)slot * G * sizeof(erp_dmatch));
-    return graph_run(ctx, key, sizeof key, [&]() -> int {
+    return graph_run(ctx, {PAIR_DIST, d_q_shard, d_t, nq_total, nt, dim, a}, [&]() -> int {
     int st = ERP_OK;
     erp_dmatch* slots = win ? reinterpret_cast<erp_dmatch*>(win->win + WindowLayout::SLOTS)
                             : ctx->scratch<erp_dmatch>(S_XCHG, (size_t)slot * G, &st);
     PoseBuffers b;
     ERP_TRY(pose_chain_buffers(ctx, nq_total, &b));
-    const bool tc = ransac_uses_tc(ctx, hhi - hlo, nq_total, metric);
+    const bool tc = ransac_uses_tc(ctx, hhi - hlo, nq_total, a.metric);
     ScoreTcBuffers sb = {};
     if (tc) ERP_TRY(score_tc_buffers(ctx, (hhi - hlo) < RANSAC_CHUNK ? (hhi - hlo) : RANSAC_CHUNK, nq_total, &sb));
     ERP_TRY(st);
@@ -461,7 +454,7 @@ ERP_API int erp_pair_pose_dist_dev(erp_ctx* ctx, const float* d_q_shard, int nq_
 
     ERP_CUDA(record_timing(ctx, ctx->ev_stage[0]));
     ERP_CUDA(cudaMemsetAsync(mine, 0, sizeof(erp_dmatch), ctx->stream));
-    ERP_TRY(match_shard_dev(ctx, d_q_shard, lo, hi, d_t, nt, dim, ratio, cross_check, mine + 1, &mine->queryIdx));
+    ERP_TRY(match_shard_dev(ctx, d_q_shard, lo, hi, d_t, nt, dim, a.ratio, a.cross_check, mine + 1, &mine->queryIdx));
     ERP_CUDA(record_timing(ctx, ctx->ev_stage[1]));
     if (win) {
         // peer stores over NVLink + epoch flags; the gather below waits for the flags of all ranks
@@ -472,16 +465,31 @@ ERP_API int erp_pair_pose_dist_dev(erp_ctx* ctx, const float* d_q_shard, int nq_
         ERP_NCCL(nccl().AllGather(mine, slots, (size_t)slot * sizeof(erp_dmatch), ncclInt8, ctx->comm->comm, ctx->stream));
     }
     if (tc) ERP_CUDA(cudaMemsetAsync(sb.w, 0, W_WORDS_BYTES, ctx->stream));
-    ERP_TRY(gather_slots_chain(ctx, slots, G, slot, nq_total, d_matches, d_n_matches, d_left_xy, d_right_xy, kp_stride_bytes,
-                               width, height, b.l3, b.r3, b.l4, b.r4, sb.Ks, sb.w,
+    ERP_TRY(gather_slots_chain(ctx, slots, G, slot, nq_total, a.matches, a.n_matches, a.left_xy, a.right_xy, a.kp_stride,
+                               a.width, a.height, b.l3, b.r3, b.l4, b.r4, sb.Ks, sb.w,
                                win ? reinterpret_cast<uint32_t*>(win->win + WindowLayout::CTL) : nullptr,
                                win ? reinterpret_cast<uint32_t*>(win->win + WindowLayout::SLOT_FLAG) : nullptr));
     ERP_CUDA(record_timing(ctx, ctx->ev_stage[2]));
-    ERP_TRY(pose_chain_tail(ctx, b.l3, b.r3, b.l4, b.r4, nq_total, d_n_matches, seed, (uint64_t)hlo, hhi - hlo, S, metric, tau, tc, true,
-                            d_mask ? d_mask : b.mask, d_result));
+    ERP_TRY(pose_chain_tail(ctx, b.l3, b.r3, b.l4, b.r4, nq_total, a.n_matches, a.seed, (uint64_t)hlo, hhi - hlo, a.S, a.metric, a.tau, tc,
+                            true, a.mask ? a.mask : b.mask, a.result));
     ERP_CUDA(record_timing(ctx, ctx->ev_stage[3]));
     return ERP_OK;
     });
+}
+
+ERP_API int erp_pair_pose_dist_dev(erp_ctx* ctx, const float* d_q_shard, int nq_total, const float* d_t, int nt, int dim,
+                                   float ratio, int cross_check,
+                                   const void* d_left_xy, const void* d_right_xy, size_t kp_stride_bytes, int width, int height,
+                                   uint64_t seed, int H_total, int S, int metric, float tau,
+                                   erp_dmatch* d_matches, int32_t* d_n_matches, uint8_t* d_mask, erp_ransac_result* d_result)
+{
+    ERP_ARG(ctx, ERP_E_ARG, "erp_pair_pose_dist_dev: null context");
+    if (comm_size(ctx) == 1)
+        return erp_pair_pose_dev(ctx, d_q_shard, nq_total, d_t, nt, dim, ratio, cross_check, d_left_xy, d_right_xy, kp_stride_bytes,
+                                 width, height, seed, H_total, S, metric, tau, d_matches, d_n_matches, d_mask, d_result);
+    return pair_pose_dist_dev(ctx, d_q_shard, nq_total, d_t, nt, dim,
+                              {ratio, cross_check, d_left_xy, d_right_xy, kp_stride_bytes, width, height, seed, H_total, S, metric, tau,
+                               d_matches, d_n_matches, d_mask, d_result});
 }
 
 namespace erp {
@@ -498,16 +506,14 @@ static int upload_sharded(erp_ctx* ctx, const float* q, int lo, int hi, size_t q
     float* dq = ctx->scratch<float>(S_Q, (size_t)(hi - lo) * dim + 4, &st);
     float* dt = ctx->scratch<float>(S_T, (size_t)tcap * G * dim + 4, &st);
     ERP_TRY(st);
-    ERP_TRY(upload_rows(ctx, dq, reinterpret_cast<const char*>(q) + (size_t)lo * qs, hi - lo, row, qs));
+    ERP_TRY(upload_rows(ctx, ctx->stream, dq, reinterpret_cast<const char*>(q) + (size_t)lo * qs, hi - lo, row, qs));
     const int t0 = rank * tcap < nt ? rank * tcap : nt, t1 = (rank + 1) * tcap < nt ? (rank + 1) * tcap : nt;
-    ERP_TRY(upload_rows(ctx, dt + (size_t)t0 * dim, reinterpret_cast<const char*>(t) + (size_t)t0 * ts, t1 - t0, row, ts));
+    ERP_TRY(upload_rows(ctx, ctx->stream, dt + (size_t)t0 * dim, reinterpret_cast<const char*>(t) + (size_t)t0 * ts, t1 - t0, row, ts));
     if (G > 1)
         ERP_NCCL(nccl().AllGather(dt + (size_t)rank * tcap * dim, dt, (size_t)tcap * dim, ncclFloat, ctx->comm->comm, ctx->stream));
     *dq_out = dq; *dt_out = dt;
     return ERP_OK;
 }
-
-static int upload_xy(erp_ctx* ctx, float* d_dst, const void* src, int rows, size_t stride) { return upload_rows(ctx, d_dst, src, rows, 8, stride); }
 
 } // namespace erp
 
@@ -524,43 +530,36 @@ ERP_API int erp_pair_pose_dist(erp_ctx* ctx, const float* q, int nq, size_t q_st
     ERP_ARG(n_matches && result && matches_out && q && t && left_xy && right_xy, ERP_E_ARG, "erp_pair_pose_dist: null argument");
     *n_matches = 0;
     ERP_ARG(nq >= 1 && nt >= 2, ERP_E_TOO_FEW_TRAIN, "erp_pair_pose_dist: nq %d, nt %d", nq, nt);
-    ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "erp_pair_pose_dist: descriptor dimension %d", dim);
+    ERP_TRY(RowKind::f32(dim).check_dim("erp_pair_pose_dist"));
     const size_t row = (size_t)dim * sizeof(float);
     ERP_ARG(q_stride_bytes >= row && t_stride_bytes >= row && kp_stride_bytes >= 8 && kp_stride_bytes % 4 == 0, ERP_E_ARG,
             "erp_pair_pose_dist: bad stride");
     DeviceGuard g(ctx->device);
+    const PairArgs out = {ratio, cross_check, left_xy, right_xy, kp_stride_bytes, width, height, seed, H, S, metric, tau,
+                          matches_out, n_matches, mask, result};
+    PairArgs dev = out;
     const int G = comm_size(ctx), rank = comm_rank(ctx);
     int lo, hi;
     shard_range(nq, rank, G, &lo, &hi);
     int st = ERP_OK;
-    erp_dmatch* d_out = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
-    int32_t* d_n = ctx->scratch<int32_t>(S_NOUT, 4, &st);
+    dev.matches = ctx->scratch<erp_dmatch>(S_OUT, (size_t)nq, &st);
+    dev.n_matches = ctx->scratch<int32_t>(S_NOUT, 4, &st);
     float* d_xy = ctx->scratch<float>(S_XY, ((size_t)nq + nt) * 2, &st);
+    dev.left_xy = d_xy;
+    dev.right_xy = d_xy + (size_t)nq * 2;
+    dev.kp_stride = 8;
     PoseBuffers b;
     ERP_TRY(pose_chain_buffers(ctx, nq, &b));
     ERP_TRY(st);
+    dev.mask = b.mask;
+    dev.result = b.res;
     float *dq, *dt;
     ERP_TRY(upload_sharded(ctx, q, lo, hi, q_stride_bytes, t, nt, t_stride_bytes, dim, &dq, &dt));
-    ERP_TRY(upload_xy(ctx, d_xy, left_xy, nq, kp_stride_bytes));
-    ERP_TRY(upload_xy(ctx, d_xy + (size_t)nq * 2, right_xy, nt, kp_stride_bytes));
-    ERP_TRY(erp_pair_pose_dist_dev(ctx, dq, nq, dt, nt, dim, ratio, cross_check, d_xy, d_xy + (size_t)nq * 2, 8, width, height,
-                                   seed, H, S, metric, tau, d_out, d_n, b.mask, b.res));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy, left_xy, nq, 8, kp_stride_bytes));
+    ERP_TRY(upload_rows(ctx, ctx->stream, d_xy + (size_t)nq * 2, right_xy, nt, 8, kp_stride_bytes));
+    ERP_TRY(pair_pose_dist_dev(ctx, dq, nq, dt, nt, dim, dev));
     // the host waits for the exchange only; the records come back while the hypotheses are being scored
-    int32_t n = 0;
-    ERP_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_stage[2], 0));
-    ERP_CUDA(cudaMemcpyAsync(&n, d_n, sizeof n, cudaMemcpyDeviceToHost, ctx->copy_stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
-    *n_matches = n;
-    if (n > 0) ERP_CUDA(cudaMemcpyAsync(matches_out, d_out, sizeof(erp_dmatch) * (size_t)n, cudaMemcpyDeviceToHost, ctx->copy_stream));
-    ERP_CUDA(cudaMemcpyAsync(result, b.res, sizeof *result, cudaMemcpyDeviceToHost, ctx->stream));
-    if (mask && n > 0) ERP_CUDA(cudaMemcpyAsync(mask, b.mask, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->stream));
-    ERP_CUDA(cudaStreamSynchronize(ctx->copy_stream));
-    if (n < S) {
-        set_error("erp_pair_pose_dist: %d matches for sample size %d", n, S);
-        return ERP_E_TOO_FEW_POINTS;
-    }
-    return ERP_OK;
+    return pair_pose_download(ctx, "erp_pair_pose_dist", ctx->ev_stage[2], dev, out);
 }
 
 ERP_API int erp_knn2_match_dist(erp_ctx* ctx, const float* q, int nq, size_t q_stride_bytes, const float* t, int nt, size_t t_stride_bytes,
@@ -570,9 +569,7 @@ ERP_API int erp_knn2_match_dist(erp_ctx* ctx, const float* q, int nq, size_t q_s
     if (comm_size(ctx) == 1) return erp_knn2_match(ctx, q, nq, q_stride_bytes, t, nt, t_stride_bytes, dim, ratio, cross_check, out, n_out);
     ERP_ARG(n_out, ERP_E_ARG, "erp_knn2_match_dist: n_out is null");
     *n_out = 0;
-    ERP_ARG(nq >= 0 && nt >= 0, ERP_E_ARG, "erp_knn2_match_dist: negative size");
-    ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "erp_knn2_match_dist: descriptor dimension %d", dim);
-    ERP_ARG(nq == 0 || nt >= 2, ERP_E_TOO_FEW_TRAIN, "erp_knn2_match_dist: k=2 needs at least 2 train descriptors, got %d", nt);
+    ERP_TRY(check_knn_args("erp_knn2_match_dist", ctx, nq, nt, RowKind::f32(dim)));
     if (nq == 0) return ERP_OK;
     const size_t row = (size_t)dim * sizeof(float);
     ERP_ARG(q && t && q_stride_bytes >= row && t_stride_bytes >= row, ERP_E_ARG, "erp_knn2_match_dist: bad descriptor buffers");
@@ -593,9 +590,8 @@ ERP_API int erp_knn2_match_dist(erp_ctx* ctx, const float* q, int nq, size_t q_s
 ERP_API int erp_knn2_match_dist_dev(erp_ctx* ctx, const float* d_q_shard, int nq_total, const float* d_t, int nt, int dim,
                                     float ratio, int cross_check, erp_dmatch* d_out, int32_t* d_n_out)
 {
-    ERP_ARG(ctx && d_n_out && nq_total >= 0 && nt >= 0, ERP_E_ARG, "erp_knn2_match_dist_dev: bad argument");
-    ERP_ARG(dim > 0 && dim % 4 == 0 && dim <= 512, ERP_E_DIM, "erp_knn2_match_dist_dev: descriptor dimension %d", dim);
-    ERP_ARG(nq_total == 0 || nt >= 2, ERP_E_TOO_FEW_TRAIN, "erp_knn2_match_dist_dev: k=2 needs at least 2 train descriptors, got %d", nt);
+    ERP_ARG(ctx && d_n_out, ERP_E_ARG, "erp_knn2_match_dist_dev: bad argument");
+    ERP_TRY(check_knn_args("erp_knn2_match_dist_dev", ctx, nq_total, nt, RowKind::f32(dim)));
     DeviceGuard g(ctx->device);
     int lo, hi;
     shard_range(nq_total, comm_rank(ctx), comm_size(ctx), &lo, &hi);

@@ -294,8 +294,13 @@ def test_host_call_with_query_chunks_equals_single_call(tmp_path):
         sys.path.insert(0, ".")
         import erp_match_eightpoint_test_b200 as erp
         from erp_match_eightpoint_test_b200 import binding, synth
-        q, t, _ = synth.descriptor_pair(3001, 2500, 64, seed=9)
         ctx = erp.Context(0)
+        # AUTO, first in the process (no earlier search left a train operand in scratch): at 7 chunks the first one has
+        # 256 rows (2.56e6 pairs, below the tensor-core threshold of a search on its own), the later ones 512 rows
+        qa, ta, _ = synth.descriptor_pair(3001, 10000, 64, seed=10)
+        idx, dist = ctx.knn2_raw(qa, ta)
+        np.save(sys.argv[1] + "_idx_auto.npy", idx); np.save(sys.argv[1] + "_dist_auto.npy", dist)
+        q, t, _ = synth.descriptor_pair(3001, 2500, 64, seed=9)
         for eng in (binding.ENGINE_EXACT_SIMT, binding.ENGINE_TCGEN05, binding.ENGINE_TCGEN05_1X):
             ctx.set_engine(eng)
             idx, dist = ctx.knn2_raw(q, t)
@@ -304,6 +309,13 @@ def test_host_call_with_query_chunks_equals_single_call(tmp_path):
             np.save(sys.argv[1] + f"_idx{eng}.npy", idx); np.save(sys.argv[1] + f"_dist{eng}.npy", dist)
             np.save(sys.argv[1] + f"_m{eng}.npy", m)
             print(eng, st["rescanned"])
+        qb, tb, _ = synth.binary_pair(3001, 2500, 32, seed=11)
+        for eng in (binding.ENGINE_EXACT_SIMT, binding.ENGINE_TCGEN05_1X):
+            ctx.set_engine(eng)
+            idx, dist = ctx.knn2_raw_bin(qb, tb)
+            np.save(sys.argv[1] + f"_idx_bin{eng}.npy", idx); np.save(sys.argv[1] + f"_dist_bin{eng}.npy", dist)
+            for cross in (False, True):
+                np.save(sys.argv[1] + f"_m{int(cross)}_bin{eng}.npy", ctx.knn2_match_bin(qb, tb, 0.8, cross))
         # the whole pair through one host-buffer call: with more than one chunk the descriptors travel behind the search
         ctx.set_engine(binding.ENGINE_AUTO)
         rng = np.random.default_rng(3)
@@ -317,7 +329,7 @@ def test_host_call_with_query_chunks_equals_single_call(tmp_path):
     """)
     import os
     outs = {}
-    for chunks in ("1", "3", "7"):                   # 3 and 7: a short first chunk, then even ones (api.cu: knn2_host)
+    for chunks in ("1", "3", "7"):                   # 3 and 7: a short first chunk, then even ones (api.cu: chunk_bounds)
         env = dict(os.environ, ERP_B200_HOST_CHUNKS=chunks)
         base = str(tmp_path / f"c{chunks}")
         r = subprocess.run([sys.executable, "-c", code, base], env=env, capture_output=True, text=True, timeout=300,
@@ -329,7 +341,8 @@ def test_host_call_with_query_chunks_equals_single_call(tmp_path):
             a = np.load(outs["1"] + f"_{what}{eng}.npy")
             for chunks in ("3", "7"):
                 assert a.tobytes() == np.load(outs[chunks] + f"_{what}{eng}.npy").tobytes(), (eng, what, chunks)
-    for what in ("pm0", "pm1", "pres0", "pres1"):
+    bin_outs = [f"{what}_bin{eng}" for eng in (binding.ENGINE_EXACT_SIMT, binding.ENGINE_TCGEN05_1X) for what in ("idx", "dist", "m0", "m1")]
+    for what in ["idx_auto", "dist_auto"] + bin_outs + ["pm0", "pm1", "pres0", "pres1"]:
         a = np.load(outs["1"] + f"_{what}.npy")
         assert len(a) > 8
         for chunks in ("3", "7"):
