@@ -94,27 +94,17 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     uint8_t* q_smem = smem;                                   // [SUB][KCH] chunks
     uint8_t* t_smem = smem + SUB * KCH * B_QCH;               // NS slots
     uint64_t* bars = reinterpret_cast<uint64_t*>(t_smem + NS * B_TCH);
-    uint64_t* full = bars;              // [NS]  TMA -> MMA
-    uint64_t* empty = bars + NS;        // [NS]  MMA -> TMA
-    uint64_t* qfull = bars + 2 * NS;    // query sub-tiles landed
-    uint64_t* qempty = qfull + 1;       // query sub-tiles no longer read
-    uint64_t* tfull = qfull + 2;        // [2] accumulator ready
-    uint64_t* tempty = qfull + 4;       // [2] accumulator drained
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(qfull + 6);
-    static_assert((2 * NS + 6) * 8 + 4 <= B_BARS, "barrier block");
+    using Pipe = PairPipe<SUB, KCH, NS, B_BM, B_BN, 128>;
+    const Pipe pipe(q_smem, t_smem, bars);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + Pipe::N_BARS);
+    static_assert(Pipe::N_BARS * 8 + 4 <= B_BARS, "barrier block");
     static_assert(b_smem(KCH) <= TC_SMEM_LIMIT, "shared memory budget");
-    const PairPipe<SUB, KCH, NS, B_BM, B_BN, 128> pipe{q_smem, t_smem, full, empty, qfull, qempty, tfull, tempty};
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int W_ALLOC = B_EPI_THREADS / 32, W_TMA = W_ALLOC + 2, W_MMA = W_ALLOC + 3;   // W_ALLOC + 1 idles
 
     if (warp == W_TMA && lane == 0) { tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_t); }
-    if (warp == W_MMA && lane == 0) {
-        for (int i = 0; i < NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        mbar_init(qfull, 1); mbar_init(qempty, 1);
-        for (int i = 0; i < 2; i++) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], B_EPI_THREADS / 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    if (warp == W_MMA && lane == 0) pipe.init(B_EPI_THREADS / 32);
     const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     // the feeder warpgroup needs few registers; the eight epilogue warps take them over (128 accumulator columns in flight)
@@ -127,7 +117,7 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         // ================================================================ MMA issuer
         if (lane == 0)
             pipe.issue(tmem_base, SegIter(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x),
-                       [](uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t accumulate) { tc_mma_i8(d_tmem, a, b, B_IDESC_I8, accumulate); },
+                       [](uint32_t d_tmem, uint32_t q, int c, uint32_t b) { mma_chunk<tc_mma_i8>(d_tmem, q + c * B_QCH, b, B_IDESC_I8, c != 0); },
                        [](int, uint32_t, uint32_t) {});
     }
     } else {
@@ -148,7 +138,7 @@ knn2_bin_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
 #pragma unroll
                 for (int sub = 0; sub < SUB; sub++, tile_n++) {
                     const uint32_t acc = tile_n & 1;
-                    mbar_wait(&tfull[acc], (tile_n >> 1) & 1);
+                    mbar_wait(&pipe.tfull[acc], (tile_n >> 1) & 1);
                     tc_fence_after();
                     const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * B_BN + cg * B_EPI_COLS;
                     uint32_t va[32], vb[32], vc[32], vd[32];

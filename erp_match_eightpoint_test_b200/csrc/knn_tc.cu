@@ -4,11 +4,13 @@
 // Replaces cv::DescriptorMatcher::knnMatch(k=2) of /root/reference/src/feature_matcher.cpp:45 in its
 // exact-L2 limit (SURVEY D1).  Pipeline, all on ctx->stream, no host synchronisation:
 //
-//   split_kernel (x2)   fp32 rows -> [hi | lo] TF32 pairs (hi = rna_tf32(v), lo = rna_tf32(v - hi)),
-//                       query rows pre-scaled by -2 (exact), train norms |t|^2, max norm
+//   split_kernel (x2)   fp32 rows -> TF32 pairs (hi = rna_tf32(v), lo = rna_tf32(v - hi)), interleaved in
+//                       32-float chunks [hi_0 | lo_0 | hi_1 | lo_1 | ...], query rows pre-scaled by -2
+//                       (exact), train norms |t|^2, max norm
 //   knn2_tc_kernel      persistent (one CTA per SM owns a contiguous range of (query tile, train tile)
-//                       units, stream-K style, so SMs finish together), warp specialised:
-//                       TMA (128B-swizzled K-major boxes) -> smem ring
+//                       units, stream-K style, so SMs finish together), warp specialised, on the query-pair
+//                       pipeline of tc_common.cuh (PairPipe, one query sub-tile of 2 x KCH chunks):
+//                       TMA (128B-swizzled K-major boxes) -> smem ring, a train tile's chunks in row order
 //                       -> tcgen05.mma kind::tf32, three products per 32-wide k chunk
 //                       (lo*hi + hi*hi + hi*lo) accumulated in a TMEM tile of 128 queries x 256 train
 //                       rows, double buffered (2 x 256 columns) so the epilogue of tile i overlaps
@@ -32,7 +34,6 @@ namespace erp {
 constexpr int BM = 128;                 // queries per tile  (UMMA M, TMEM lanes)
 constexpr int BN = 256;                 // train rows per tile (UMMA N, TMEM columns per accumulator)
 constexpr int KC = 32;                  // floats per k chunk: one 128-byte swizzle atom
-constexpr int UK = 8;                   // UMMA K for kind::tf32
 constexpr int Q_CHUNK_BYTES = BM * KC * 4;   // 16 KB
 constexpr int T_CHUNK_BYTES = BN * KC * 4;   // 32 KB
 constexpr int EPI_GROUPS = 2;           // column groups per tile: 2 x 4 epilogue warps, two per scheduler
@@ -41,7 +42,7 @@ constexpr int TC_THREADS = 128 + EPI_THREADS;   // warps 0..7 epilogue, then TME
 constexpr int EPI_COLS = BN / EPI_GROUPS;       // columns of a tile each epilogue thread scans
 constexpr int TOPK = 4;
 constexpr int MAX_SEG = 64 / (TOPK * EPI_GROUPS);     // segments per query tile: refine_kernel holds <= 64 candidates
-constexpr int SMEM_LIMIT = 232448;      // 227 KB
+constexpr int SMEM_LIMIT = TC_SMEM_LIMIT;       // the budget of n_slots (tests/test_gpu_pipeline_plans.py reads the formula by name)
 constexpr int SMEM_TAIL = 2 * BN * 4 + 256;     // |t|^2 of two tiles + mbarriers + the TMEM base address
 // certificate slack: |s_tc - s_exact| <= KAPPA * (|q|^2 + max|t|^2).  3xTF32 drops lo*lo (2^-22),
 // rounds lo to tf32 (2^-23) and accumulates 3*D/8 partial sums in fp32 (<= 2^-18 for D = 128);
@@ -54,10 +55,10 @@ __host__ __device__ constexpr int tc_smem(int kch) { return 2 * kch * Q_CHUNK_BY
 constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 
 // ------------------------------------------------------------------------------------------
-// prep: fp32 rows -> [hi | lo] (dpad each), norms
+// prep: fp32 rows -> hi and lo (dpad each, interleaved by k chunk), norms
 // ------------------------------------------------------------------------------------------
 
-// one warp per row.  out: n x (2*dpad).  norm (optional): n_pad floats, rows >= n get +inf.
+// one warp per row.  out: n x (2*dpad), chunk c of hi at 2c * KC, of lo at (2c + 1) * KC.  norm (optional): n_pad floats, rows >= n get +inf.
 // LPR lanes own one row (4 floats per lane and pass); a warp covers 32 / LPR rows
 template <int LPR>
 __global__ void __launch_bounds__(256)
@@ -77,9 +78,9 @@ split_kernel(const float* __restrict__ x, int n, int dim, int dpad, float scale,
             float4 hi = make_float4(tf32_rna(s.x), tf32_rna(s.y), tf32_rna(s.z), tf32_rna(s.w));
             float4 lo = make_float4(tf32_rna(__fsub_rn(s.x, hi.x)), tf32_rna(__fsub_rn(s.y, hi.y)),
                                     tf32_rna(__fsub_rn(s.z, hi.z)), tf32_rna(__fsub_rn(s.w, hi.w)));
-            float* o = out + (size_t)row * 2 * dpad + k;
+            float* o = out + (size_t)row * 2 * dpad + (k & ~(KC - 1)) + k;
             *reinterpret_cast<float4*>(o) = hi;
-            *reinterpret_cast<float4*>(o + dpad) = lo;
+            *reinterpret_cast<float4*>(o + KC) = lo;
         }
     }
     if (norm) {
@@ -109,6 +110,72 @@ static int launch_prep(erp_ctx* ctx, const float* x, int n, int dim, int dpad, f
     return ERP_OK;
 }
 
+// ---- running top-4 of one query row -----------------------------------------------------------
+// A column is a candidate iff its approximate score is below
+//     min( 4th best so far,  2nd best so far + slack )      (slack_of, tc_common.cuh).
+// Columns above "2nd best + 2 eps" can never be one of the exact two nearest neighbours, so they need not be kept: the
+// rare insert path then runs ~2 ln(n) times per row instead of 4 ln(n) or 8 ln(n), and the list's certificate bound is
+// that same minimum (both terms only decrease while the scan proceeds).
+__device__ __forceinline__ void top4_insert(float s, int idx, float (&bs)[4], int (&bi)[4])
+{
+    // strict <: equal scores keep the earlier (lower) train index
+    if (s < bs[2]) {
+        bs[3] = bs[2]; bi[3] = bi[2];
+        if (s < bs[1]) {
+            bs[2] = bs[1]; bi[2] = bi[1];
+            if (s < bs[0]) { bs[1] = bs[0]; bi[1] = bi[0]; bs[0] = s; bi[0] = idx; }
+            else { bs[1] = s; bi[1] = idx; }
+        } else { bs[2] = s; bi[2] = idx; }
+    } else { bs[3] = s; bi[3] = idx; }
+}
+
+// 32 accumulator columns of one query row.  Common case: s = acc + |t|^2 (32 independent adds), a min
+// tree and ONE warp-uniform threshold test.  Rare case: only the groups of 8 columns that some lane
+// needs are re-read from TMEM in a rolled loop, and only the columns below the threshold are visited
+// -- the insert cascade exists once per call site, which keeps the loop inside the instruction cache
+// (fully unrolled it was 60 KB and 3x slower).  Re-computed scores are bit-identical to the first pass.
+__device__ __forceinline__ void scan_chunk(const uint32_t (&v)[32], uint32_t taddr, const float4* __restrict__ tn4, int col0,
+                                           float slack, float (&bs)[4], int (&bi)[4])
+{
+    float gm[4];
+#pragma unroll
+    for (int g = 0; g < 4; g++) {
+        float4 na = tn4[g * 2], nb = tn4[g * 2 + 1];
+        float s0 = __fadd_rn(__uint_as_float(v[g * 8 + 0]), na.x), s1 = __fadd_rn(__uint_as_float(v[g * 8 + 1]), na.y);
+        float s2 = __fadd_rn(__uint_as_float(v[g * 8 + 2]), na.z), s3 = __fadd_rn(__uint_as_float(v[g * 8 + 3]), na.w);
+        float s4 = __fadd_rn(__uint_as_float(v[g * 8 + 4]), nb.x), s5 = __fadd_rn(__uint_as_float(v[g * 8 + 5]), nb.y);
+        float s6 = __fadd_rn(__uint_as_float(v[g * 8 + 6]), nb.z), s7 = __fadd_rn(__uint_as_float(v[g * 8 + 7]), nb.w);
+        gm[g] = fminf(fminf(fminf(s0, s1), fminf(s2, s3)), fminf(fminf(s4, s5), fminf(s6, s7)));
+    }
+    const float thr = fminf(bs[3], __fadd_rn(bs[1], slack));
+    const unsigned mine = (gm[0] < thr ? 1u : 0u) | (gm[1] < thr ? 2u : 0u) | (gm[2] < thr ? 4u : 0u) | (gm[3] < thr ? 8u : 0u);
+    unsigned need = __reduce_or_sync(0xffffffffu, mine);
+    while (need) {                                  // warp-uniform
+        const int g = __ffs(need) - 1;
+        need &= need - 1;
+        uint32_t w[8];
+        tc_ld8(taddr + g * 8, w);
+        tc_wait_ld8(w);
+        const float4 na = tn4[g * 2], nb = tn4[g * 2 + 1];
+        if ((mine >> g) & 1u) {
+            float e[8];
+            e[0] = __fadd_rn(__uint_as_float(w[0]), na.x); e[1] = __fadd_rn(__uint_as_float(w[1]), na.y);
+            e[2] = __fadd_rn(__uint_as_float(w[2]), na.z); e[3] = __fadd_rn(__uint_as_float(w[3]), na.w);
+            e[4] = __fadd_rn(__uint_as_float(w[4]), nb.x); e[5] = __fadd_rn(__uint_as_float(w[5]), nb.y);
+            e[6] = __fadd_rn(__uint_as_float(w[6]), nb.z); e[7] = __fadd_rn(__uint_as_float(w[7]), nb.w);
+            unsigned m = (e[0] < thr ? 1u : 0u) | (e[1] < thr ? 2u : 0u) | (e[2] < thr ? 4u : 0u) | (e[3] < thr ? 8u : 0u) |
+                         (e[4] < thr ? 16u : 0u) | (e[5] < thr ? 32u : 0u) | (e[6] < thr ? 64u : 0u) | (e[7] < thr ? 128u : 0u);
+            while (m) {                             // usually a single column
+                const int j = __ffs(m) - 1;
+                m &= m - 1;
+                const float x = j == 0 ? e[0] : j == 1 ? e[1] : j == 2 ? e[2] : j == 3 ? e[3] : j == 4 ? e[4] : j == 5 ? e[5] : j == 6 ? e[6] : e[7];
+                if (x < fminf(bs[3], __fadd_rn(bs[1], slack))) top4_insert(x, col0 + g * 8 + j, bs, bi);
+            }
+        }
+        __syncwarp();
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // the distance kernel
 // ------------------------------------------------------------------------------------------
@@ -135,18 +202,16 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
     extern __shared__ __align__(1024) uint8_t smem[];
     // the 128B swizzle atoms need a 1024-byte aligned base; the budget has no room for a round-up
     if ((smem_u32(smem) & 1023u) != 0) __trap();
-    uint8_t* q_smem = smem;                                   // 2*KCH chunks: hi 0..KCH-1, lo KCH..2KCH-1
     uint8_t* t_smem = smem + 2 * KCH * Q_CHUNK_BYTES;         // NS slots
     float* tn_smem = reinterpret_cast<float*>(t_smem + NS * T_CHUNK_BYTES);   // [2][BN], follows the accumulator parity
     uint64_t* bars = reinterpret_cast<uint64_t*>(tn_smem + 2 * BN);
-    uint64_t* full = bars;              // [NS]  TMA -> MMA
-    uint64_t* empty = bars + NS;        // [NS]  MMA -> TMA
-    uint64_t* qfull = bars + 2 * NS;    // Q tile landed
-    uint64_t* qempty = qfull + 1;       // Q tile no longer read
-    uint64_t* tfull = qfull + 2;        // [2] accumulator ready
-    uint64_t* tempty = qfull + 4;       // [2] accumulator (and its |t|^2 buffer) drained
-    uint64_t* nfull = qfull + 6;        // [2] |t|^2 of the tile landed
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(qfull + 8);
+    // one query sub-tile of 2*KCH chunks hi_0, lo_0, hi_1, ... (the split rows' order), which is also the order in which a
+    // train tile's chunks pass the ring
+    using Pipe = PairPipe<1, 2 * KCH, NS, BM, BN, KC>;
+    const Pipe pipe(smem, t_smem, bars);
+    uint64_t* nfull = bars + Pipe::N_BARS;      // [2] |t|^2 of the tile landed
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(nfull + 2);
+    static_assert((Pipe::N_BARS + 2) * 8 + 4 <= SMEM_TAIL - 2 * BN * 4, "barrier block");
 
     // the scheduler favours the highest warp id among eligible warps: the single-thread feeders
     // (TMA, MMA) sit on top so that the epilogue warps never delay them
@@ -158,83 +223,25 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
         tma_prefetch_desc(&map_t);
     }
     if (warp == W_MMA && lane == 0) {
-        for (int i = 0; i < NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        mbar_init(qfull, 1); mbar_init(qempty, 1);
-        for (int i = 0; i < 2; i++) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], EPI_THREADS / 32); mbar_init(&nfull[i], 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int i = 0; i < 2; i++) mbar_init(&nfull[i], 1);
+        pipe.init(EPI_THREADS / 32);
     }
     const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     if (warp == W_TMA) {
         // ================================================================ TMA producer
-        if (lane == 0) {
-            uint32_t slot = 0, ph = 0, item_n = 0;
-            SegIter it(p.n_qtiles, p.n_ttiles, p.units_per_cta, blockIdx.x);
-            int qtile, t_begin, t_end, seg;
-            for (; it.next(qtile, t_begin, t_end, seg); item_n++) {
-                mbar_wait(qempty, (item_n & 1) ^ 1);
-                mbar_expect_tx(qfull, 2 * KCH * Q_CHUNK_BYTES);
-#pragma unroll
-                for (int c = 0; c < 2 * KCH; c++)
-                    tma_load_2d(&map_q, qfull, q_smem + c * Q_CHUNK_BYTES, c * KC, qtile * BM);
-                for (int tt = t_begin; tt < t_end; tt++) {
-#pragma unroll
-                    for (int c = 0; c < KCH; c++) {
-#pragma unroll
-                        for (int half = 0; half < 2; half++) {      // hi chunk c, then lo chunk c
-                            mbar_wait(&empty[slot], ph ^ 1);
-                            mbar_expect_tx(&full[slot], T_CHUNK_BYTES);
-                            tma_load_2d(&map_t, &full[slot], t_smem + slot * T_CHUNK_BYTES, (half * KCH + c) * KC, tt * BN);
-                            if (++slot == NS) { slot = 0; ph ^= 1; }
-                        }
-                    }
-                }
-            }
-        }
+        if (lane == 0) pipe.produce(&map_q, &map_t, SegIter(p.n_qtiles, p.n_ttiles, p.units_per_cta, blockIdx.x));
     } else if (warp == W_MMA) {
         // ================================================================ MMA issuer
-        if (lane == 0) {
-            uint32_t slot = 0, ph = 0, item_n = 0, tile_n = 0;
-            const uint32_t q_base = smem_u32(q_smem), t_base = smem_u32(t_smem);
-            SegIter it(p.n_qtiles, p.n_ttiles, p.units_per_cta, blockIdx.x);
-            int qtile, t_begin, t_end, seg;
-            for (; it.next(qtile, t_begin, t_end, seg); item_n++) {
-                mbar_wait(qfull, item_n & 1);
-                for (int tt = t_begin; tt < t_end; tt++, tile_n++) {
-                    const uint32_t acc = tile_n & 1;
-                    mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
-                    tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + acc * BN;
-#pragma unroll
-                    for (int c = 0; c < KCH; c++) {
-                        const uint32_t a_hi = q_base + c * Q_CHUNK_BYTES, a_lo = q_base + (KCH + c) * Q_CHUNK_BYTES;
-                        // ---- T hi chunk c: lo*hi then hi*hi
-                        mbar_wait(&full[slot], ph);
-                        tc_fence_after();
-                        uint32_t b = t_base + slot * T_CHUNK_BYTES;
-#pragma unroll
-                        for (int k = 0; k < KC / UK; k++)
-                            tc_mma_tf32(d_tmem, smem_desc_sw128(a_lo + k * UK * 4), smem_desc_sw128(b + k * UK * 4), IDESC, (c | k) != 0);
-#pragma unroll
-                        for (int k = 0; k < KC / UK; k++)
-                            tc_mma_tf32(d_tmem, smem_desc_sw128(a_hi + k * UK * 4), smem_desc_sw128(b + k * UK * 4), IDESC, 1);
-                        tc_commit(&empty[slot]);
-                        if (++slot == NS) { slot = 0; ph ^= 1; }
-                        // ---- T lo chunk c: hi*lo
-                        mbar_wait(&full[slot], ph);
-                        tc_fence_after();
-                        b = t_base + slot * T_CHUNK_BYTES;
-#pragma unroll
-                        for (int k = 0; k < KC / UK; k++)
-                            tc_mma_tf32(d_tmem, smem_desc_sw128(a_hi + k * UK * 4), smem_desc_sw128(b + k * UK * 4), IDESC, 1);
-                        tc_commit(&empty[slot]);
-                        if (++slot == NS) { slot = 0; ph ^= 1; }
-                    }
-                    tc_commit(&tfull[acc]);
-                }
-                tc_commit(qempty);
-            }
-        }
+        if (lane == 0)
+            pipe.issue(tmem_base, SegIter(p.n_qtiles, p.n_ttiles, p.units_per_cta, blockIdx.x),
+                       [](uint32_t d_tmem, uint32_t q, int c, uint32_t b) {
+                           // ring chunk c is T hi_j (c = 2j: lo*hi, then hi*hi) or T lo_j (c = 2j + 1: hi*lo)
+                           const uint32_t q_hi = q + (c & ~1) * Q_CHUNK_BYTES, q_lo = q_hi + Q_CHUNK_BYTES;
+                           if ((c & 1) == 0) mma_chunk<tc_mma_tf32>(d_tmem, q_lo, b, IDESC, c != 0);
+                           mma_chunk<tc_mma_tf32>(d_tmem, q_hi, b, IDESC, true);
+                       },
+                       [](int, uint32_t, uint32_t) {});
     } else if (warp == W_NORM) {
         // ================================================================ |t|^2 producer
         // one bulk copy of 1 KB per tile into the buffer of the accumulator parity; it may be
@@ -246,7 +253,7 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
             while (it.next(qtile, t_begin, t_end, seg)) {
                 for (int tt = t_begin; tt < t_end; tt++, tile_n++) {
                     const uint32_t acc = tile_n & 1;
-                    mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
+                    mbar_wait(&pipe.tempty[acc], ((tile_n >> 1) & 1) ^ 1);
                     mbar_expect_tx(&nfull[acc], BN * 4);
                     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                                  ::"r"(smem_u32(tn_smem + acc * BN)), "l"(p.tn + (size_t)tt * BN), "r"(BN * 4), "r"(smem_u32(&nfull[acc]))
@@ -272,7 +279,7 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
             for (int tt = t_begin; tt < t_end; tt++, tile_n++) {
                 const uint32_t acc = tile_n & 1;
                 mbar_wait(&nfull[acc], (tile_n >> 1) & 1);
-                mbar_wait(&tfull[acc], (tile_n >> 1) & 1);
+                mbar_wait(&pipe.tfull[acc], (tile_n >> 1) & 1);
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * BN + cg * EPI_COLS;
                 // |t|^2 of this warp's columns: every lane reads the same 16 bytes (shared-memory broadcast)
@@ -293,7 +300,7 @@ knn2_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant_
                 // accumulator drained: hand it back to the MMA warp
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive(&tempty[acc]);
+                if (lane == 0) mbar_arrive(&pipe.tempty[acc]);
             }
             const int qg = qtile * BM + row;
             if (qg < p.nq) {

@@ -185,21 +185,16 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     uint8_t* aug_t = t_smem + NS * F_TCH;                     // [2][F_AUG_T] norm operand by train-tile parity, then the query side
     uint8_t* aug_q = aug_t + 2 * F_AUG_T;
     uint64_t* bars = reinterpret_cast<uint64_t*>(aug_q + F_AUG_Q);
-    uint64_t* full = bars;              // [NS]  TMA -> MMA
-    uint64_t* empty = bars + NS;        // [NS]  MMA -> TMA
-    uint64_t* qfull = bars + 2 * NS;    // query pair landed
-    uint64_t* qempty = qfull + 1;       // query pair no longer read
-    uint64_t* tfull = qfull + 2;        // [2] accumulator ready
-    uint64_t* tempty = qfull + 4;       // [2] accumulator drained
-    uint64_t* nfull = qfull + 6;        // [2] norm operand of a train tile landed
-    uint64_t* nempty = qfull + 8;       // [2] ... and read by the MMAs of both sub-tiles
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(qfull + 10);
-    static_assert((2 * NS + 10) * 8 + 4 <= F_BARS, "barrier block");
+    using Pipe = PairPipe<F_SUB, KCH, NS, F_BM, F_BN, F_KC>;
+    const Pipe pipe(q_smem, t_smem, bars);
+    uint64_t* nfull = bars + Pipe::N_BARS;      // [2] norm operand of a train tile landed
+    uint64_t* nempty = nfull + 2;               // [2] ... and read by the MMAs of both sub-tiles
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(nfull + 4);
+    static_assert((Pipe::N_BARS + 4) * 8 + 4 <= F_BARS, "barrier block");
     float* thr_sh = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + F_BARS);   // [F_SUB][F_BM] row thresholds
     static_assert(F_SUB * KCH * F_QCH + NS * F_TCH + 2 * F_AUG_T + F_AUG_Q + F_BARS + F_SUB * F_BM * 4 <= f_smem(KCH),
                   "threshold exchange area");
     static_assert(f_smem(KCH) <= TC_SMEM_LIMIT, "shared memory budget");
-    const PairPipe<F_SUB, KCH, NS, F_BM, F_BN, F_KC> pipe{q_smem, t_smem, full, empty, qfull, qempty, tfull, tempty};
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     TCC_DECL;
@@ -207,13 +202,8 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
 
     if (warp == W_TMA && lane == 0) { tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_t); tma_prefetch_desc(&map_aug); }
     if (warp == W_MMA && lane == 0) {
-        for (int i = 0; i < NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        mbar_init(qfull, 1); mbar_init(qempty, 1);
-        for (int i = 0; i < 2; i++) {
-            mbar_init(&tfull[i], 1); mbar_init(&tempty[i], F_EPI_THREADS / 32);
-            mbar_init(&nfull[i], 1); mbar_init(&nempty[i], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int i = 0; i < 2; i++) { mbar_init(&nfull[i], 1); mbar_init(&nempty[i], 1); }
+        pipe.init(F_EPI_THREADS / 32);
     }
     // query side of the norm step: the same 8 halves in both 16-byte halves of every row, which the swizzle cannot change
     for (int i = threadIdx.x; i < F_AUG_Q / 2; i += F_THREADS)
@@ -232,7 +222,7 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
         if (lane == 0) {
             const uint64_t aq_desc = smem_desc_sw32(smem_u32(aug_q));
             pipe.issue(tmem_base, SegIter(p.n_qpairs, p.n_ttiles, p.units_per_cta, blockIdx.x),
-                       [](uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t accumulate) { tc_mma_f16(d_tmem, a, b, F_IDESC, accumulate); },
+                       [](uint32_t d_tmem, uint32_t q, int c, uint32_t b) { mma_chunk<tc_mma_f16>(d_tmem, q + c * F_QCH, b, F_IDESC, c != 0); },
                        [&](int sub, uint32_t tt_n, uint32_t d_tmem) {
                            // the norm step
                            const uint32_t nb = tt_n & 1;
@@ -317,7 +307,7 @@ knn2_tc1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
                 for (int sub = 0; sub < F_SUB; sub++, tile_n++) {
                     const uint32_t acc = tile_n & 1;
                     TCC_CLOCK(c0);
-                    mbar_wait(&tfull[acc], (tile_n >> 1) & 1);
+                    mbar_wait(&pipe.tfull[acc], (tile_n >> 1) & 1);
                     TCC_CLOCK(c1);
                     tc_fence_after();
                     const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + acc * F_BN + cg * F_EPI_COLS;

@@ -24,7 +24,8 @@
 // Work is cut stream-K style over (pair of hypothesis tiles, correspondence tile) units -- each 32 KB
 // correspondence tile that TMA brings in feeds two 128-row accumulators, which halves the L2 -> shared
 // memory traffic per MMA (with one it was the limiter: tensor pipe 42 % active).  A pair cut between two
-// CTAs adds its partial counts atomically.
+// CTAs adds its partial counts atomically.  Producer and MMA issuer are the query-pair pipeline of tc_common.cuh
+// (PairPipe, the pair double-buffered); the counting epilogue keeps its own software pipeline.
 #include "score_common.cuh"
 #include "tc_common.cuh"
 
@@ -40,7 +41,8 @@ constexpr int S_EPI_GROUPS = 2;
 constexpr int S_EPI_THREADS = S_EPI_GROUPS * 128;
 constexpr int S_THREADS = 128 + S_EPI_THREADS;
 constexpr int S_EPI_COLS = SN_ROWS / S_EPI_GROUPS;
-constexpr int S_SMEM = 2 * S_SUB * SA_BYTES + S_NSLOT * SB_BYTES + 256;
+constexpr int S_BARS = 256;                  // mbarriers, TMEM slot and the epilogue's threshold word
+constexpr int S_SMEM = 2 * S_SUB * SA_BYTES + S_NSLOT * SB_BYTES + S_BARS;
 static_assert(S_SMEM <= TC_SMEM_LIMIT, "shared memory budget");
 constexpr uint32_t S_IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(SN_ROWS >> 3) << 17) | ((uint32_t)(SM_ROWS >> 4) << 24);
 // |res_tc - res_chain| <= S_KAPPA * sqrt(2) * max_c |l_c||r_c|: 3xTF32 (2^-20) + the chain's own
@@ -139,16 +141,14 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
 {
     extern __shared__ __align__(1024) uint8_t smem[];
     if ((smem_u32(smem) & 1023u) != 0) __trap();
-    uint8_t* a_smem = smem;                               // [2 buffers][S_SUB] hypothesis tiles
-    uint8_t* b_smem = smem + 2 * S_SUB * SA_BYTES;        // [S_NSLOT] correspondence tiles
-    uint64_t* bars = reinterpret_cast<uint64_t*>(b_smem + S_NSLOT * SB_BYTES);
-    uint64_t* full = bars;                  // [S_NSLOT]
-    uint64_t* empty = bars + S_NSLOT;       // [S_NSLOT]
-    uint64_t* afull = bars + 2 * S_NSLOT;   // [2]
-    uint64_t* aempty = afull + 2;           // [2]
-    uint64_t* tfull = afull + 4;            // [2]
-    uint64_t* tempty = afull + 6;           // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(afull + 8);
+    // [2 buffers][S_SUB] hypothesis tiles of one k chunk (32 floats), then the S_NSLOT correspondence slots
+    using Pipe = PairPipe<S_SUB, 1, S_NSLOT, SM_ROWS, SN_ROWS, 32, 2>;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 2 * S_SUB * SA_BYTES + S_NSLOT * SB_BYTES);
+    const Pipe pipe(smem, smem + 2 * S_SUB * SA_BYTES, bars);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + Pipe::N_BARS);
+    // the epilogue's threshold word, clear of the barriers and the TMEM slot
+    constexpr int HI_SH = 192;
+    static_assert(Pipe::N_BARS * 8 + 4 <= HI_SH && HI_SH + 4 <= S_BARS, "barrier block");
 
     // roles: warps 0..7 epilogue, then TMEM allocator, idle, TMA producer, MMA issuer.  The scheduler
     // favours the highest warp id among eligible warps: the two single-thread feeders sit on top so
@@ -157,14 +157,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
     constexpr int W_ALLOC = S_EPI_THREADS / 32, W_TMA = W_ALLOC + 2, W_MMA = W_ALLOC + 3;
 
     if (warp == W_TMA && lane == 0) { tma_prefetch_desc(&map_e); tma_prefetch_desc(&map_k); }
-    if (warp == W_MMA && lane == 0) {
-        for (int i = 0; i < S_NSLOT; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; i++) {
-            mbar_init(&afull[i], 1); mbar_init(&aempty[i], 1);
-            mbar_init(&tfull[i], 1); mbar_init(&tempty[i], S_EPI_THREADS / 32);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    if (warp == W_MMA && lane == 0) pipe.init(S_EPI_THREADS / 32);
     const uint32_t tmem_base = tmem_alloc(warp == W_ALLOC, tmem_slot);
 
     // the four feeder warps need few registers; the eight epilogue warps take them over (128 accumulator columns in flight)
@@ -173,57 +166,16 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
     if (warp == W_TMA) {
         // ================================================================ TMA producer
         if (lane == 0) {
-            uint32_t slot = 0, ph = 0, seg_n = 0;
             const ScoreShape sh(p);
-            SegIter it(sh.n_htiles, sh.n_ctiles, sh.units_per_cta, blockIdx.x);
-            int ht, c0, c1, seg;
-            for (; it.next(ht, c0, c1, seg); seg_n++) {
-                c0 += sh.ct_begin; c1 += sh.ct_begin;
-                const uint32_t ab = seg_n & 1;
-                mbar_wait(&aempty[ab], ((seg_n >> 1) & 1) ^ 1);
-                mbar_expect_tx(&afull[ab], S_SUB * SA_BYTES);
-#pragma unroll
-                for (int sub = 0; sub < S_SUB; sub++)
-                    tma_load_2d(&map_e, &afull[ab], a_smem + (ab * S_SUB + sub) * SA_BYTES, 0, (ht * S_SUB + sub) * SM_ROWS);
-                for (int ct = c0; ct < c1; ct++) {
-                    mbar_wait(&empty[slot], ph ^ 1);
-                    mbar_expect_tx(&full[slot], SB_BYTES);
-                    tma_load_2d(&map_k, &full[slot], b_smem + slot * SB_BYTES, 0, ct * SN_ROWS);
-                    if (++slot == S_NSLOT) { slot = 0; ph ^= 1; }
-                }
-            }
+            pipe.produce(&map_e, &map_k, SegIter(sh.n_htiles, sh.n_ctiles, sh.units_per_cta, blockIdx.x), sh.ct_begin);
         }
     } else if (warp == W_MMA) {
         // ================================================================ MMA issuer
         if (lane == 0) {
-            uint32_t slot = 0, ph = 0, seg_n = 0, tile_n = 0;
-            const uint32_t a_base = smem_u32(a_smem), b_base = smem_u32(b_smem);
             const ScoreShape sh(p);
-            SegIter it(sh.n_htiles, sh.n_ctiles, sh.units_per_cta, blockIdx.x);
-            int ht, c0, c1, seg;
-            for (; it.next(ht, c0, c1, seg); seg_n++) {
-                const uint32_t ab = seg_n & 1;
-                mbar_wait(&afull[ab], (seg_n >> 1) & 1);
-                for (int ct = c0; ct < c1; ct++) {
-                    mbar_wait(&full[slot], ph);
-                    const uint32_t b = b_base + slot * SB_BYTES;
-#pragma unroll
-                    for (int sub = 0; sub < S_SUB; sub++, tile_n++) {
-                        const uint32_t acc = tile_n & 1;
-                        const uint32_t a = a_base + (ab * S_SUB + sub) * SA_BYTES;
-                        mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
-                        tc_fence_after();
-                        const uint32_t d_tmem = tmem_base + acc * SN_ROWS;
-#pragma unroll
-                        for (int k = 0; k < 4; k++)
-                            tc_mma_tf32(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), S_IDESC, k != 0);
-                        tc_commit(&tfull[acc]);
-                    }
-                    tc_commit(&empty[slot]);
-                    if (++slot == S_NSLOT) { slot = 0; ph ^= 1; }
-                }
-                tc_commit(&aempty[ab]);
-            }
+            pipe.issue(tmem_base, SegIter(sh.n_htiles, sh.n_ctiles, sh.units_per_cta, blockIdx.x),
+                       [](uint32_t d_tmem, uint32_t a, int, uint32_t b) { mma_chunk<tc_mma_tf32>(d_tmem, a, b, S_IDESC, false); },
+                       [](int, uint32_t, uint32_t) {});
         }
     }
     } else {
@@ -238,7 +190,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
         if (!(delta < INFINITY)) hi = INFINITY;                         // non-finite input: every finite residual may be an inlier
         // the threshold is re-read (volatile) after every hand-back of an accumulator: the counting depends on that load, so
         // the assembler cannot sink the TMEM loads into the counting code and delay the hand-back
-        volatile float* hi_sh = reinterpret_cast<volatile float*>(reinterpret_cast<uint8_t*>(bars) + 192);
+        volatile float* hi_sh = reinterpret_cast<volatile float*>(reinterpret_cast<uint8_t*>(bars) + HI_SH);
         *hi_sh = hi;
         uint32_t tile_n = 0;
         const ScoreShape sh(p);
@@ -259,14 +211,14 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
             const uint32_t lane_base = tmem_base + ((uint32_t)(ew * 32) << 16) + cg * S_EPI_COLS;
             if (c0 < c1) {
                 const uint32_t acc = tile_n & 1;
-                mbar_wait(&tfull[acc], (tile_n >> 1) & 1);
+                mbar_wait(&pipe.tfull[acc], (tile_n >> 1) & 1);
                 tc_fence_after();
                 const uint32_t taddr = lane_base + acc * SN_ROWS;
                 tc_ld32(taddr, va); tc_ld32(taddr + 32, vb); tc_ld32(taddr + 64, vc); tc_ld32(taddr + 96, vd);
                 tc_wait_ld32(va); tc_wait_ld32(vb); tc_wait_ld32(vc); tc_wait_ld32(vd);
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive(&tempty[acc]);
+                if (lane == 0) mbar_arrive(&pipe.tempty[acc]);
                 tile_n++;
             }
             for (int ct = c0; ct < c1; ct++) {
@@ -281,7 +233,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
                     count_chunk(va, hv, acc4[sub]);
                     count_chunk(vb, hv, acc4[sub]);
                     if (has_next) {
-                        mbar_wait(&tfull[acc], (tile_n >> 1) & 1);
+                        mbar_wait(&pipe.tfull[acc], (tile_n >> 1) & 1);
                         tc_fence_after();
                         tc_ld32(taddr, va); tc_ld32(taddr + 32, vb);
                     }
@@ -292,7 +244,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
                         tc_wait_ld32(va); tc_wait_ld32(vb); tc_wait_ld32(vc); tc_wait_ld32(vd);
                         tc_fence_before();
                         __syncwarp();
-                        if (lane == 0) mbar_arrive(&tempty[acc]);
+                        if (lane == 0) mbar_arrive(&pipe.tempty[acc]);
                         tile_n++;
                     }
                 }

@@ -1,7 +1,7 @@
 // tc_common.cuh -- what the tcgen05 kernels share (knn_tc.cu and knn_tc1.cu: distances, knn_bin.cu: Hamming distances,
 // score_tc.cu: residuals): inline-PTX wrappers (mbarrier, TMA, tcgen05 / TMEM), TMEM allocation, the tensor-map encoder,
-// the stream-K planner and the launcher; and the query-pair pipeline (TMA producer, MMA ring walk, accumulator drain) of
-// knn_tc1.cu and knn_bin.cu.
+// the stream-K planner and the launcher; and the query-pair pipeline (barriers, TMA producer, MMA ring walk, accumulator
+// drain) that all four kernels run on.
 #pragma once
 
 #include "common.cuh"
@@ -128,7 +128,6 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32])
         : "r"(taddr)
         : "memory");
 }
-__device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // shared-memory matrix descriptor: K-major, 128-byte swizzle, rows of 128 bytes, 8-row groups of
 // 1024 bytes (SBO), descriptor version 1 (sm_100).  addr may point inside the first swizzle row
@@ -154,9 +153,6 @@ __device__ __forceinline__ uint64_t smem_desc_sw32(uint32_t addr)
     d |= (uint64_t)6 << 61;                          // SWIZZLE_32B
     return d;
 }
-// instruction descriptor: D fp32, A/B tf32, both K-major, N = 256, M = 128
-
-
 // wait for this thread's outstanding tcgen05.ld; the registers are operands so that no use of
 // them can be scheduled above the wait
 __device__ __forceinline__ void tc_wait_ld32(uint32_t (&v)[32])
@@ -278,95 +274,13 @@ inline int launch_tc_kernel(erp_ctx* ctx, const char* name, int grid, int block,
 }
 
 
-// ---- running top-4 of one query row, shared by the two distance kernels -----------------------
-// A column is a candidate iff its approximate score is below
-//     min( 4th best so far,  2nd best so far + slack ),      slack = 2 * kappa * (|q|^2 + max|t|^2).
-// Columns above "2nd best + 2 eps" can never be one of the exact two nearest neighbours (their exact
-// distance exceeds the exact distance of the approximate runner-up), so they need not be kept: the
-// rare insert path then runs ~2 ln(n) times per row instead of 4 ln(n) or 8 ln(n), and the list's
-// certificate bound is that same minimum (both terms only decrease while the scan proceeds).
+// Columns whose approximate score is above "2nd best so far + slack" can never be one of the exact two nearest neighbours
+// (their exact distance exceeds the exact distance of the approximate runner-up): both distance kernels keep only columns
+// below it.  slack = 2 * kappa * (|q|^2 + max|t|^2) for a score error of at most kappa * (|q|^2 + max|t|^2).
 __device__ __forceinline__ float slack_of(float qn, float tn_max, float kappa)
 {
     return __fmul_rn(__fmul_rn(2.0002f * kappa, __fadd_rn(qn, tn_max)), 1.0f);
 }
-// sorted insert for any K (ascending; strict <: equal scores keep the earlier index); all stages are independent
-template <int K>
-__device__ __forceinline__ void topk_insert(float s, int idx, float (&bs)[K], int (&bi)[K])
-{
-#pragma unroll
-    for (int j = K - 1; j > 0; j--) {
-        const bool up = s < bs[j - 1], here = s < bs[j];
-        bs[j] = up ? bs[j - 1] : (here ? s : bs[j]);
-        bi[j] = up ? bi[j - 1] : (here ? idx : bi[j]);
-    }
-    const bool first = s < bs[0];
-    bs[0] = first ? s : bs[0];
-    bi[0] = first ? idx : bi[0];
-}
-__device__ __forceinline__ void top4_insert(float s, int idx, float (&bs)[4], int (&bi)[4])
-{
-    // strict <: equal scores keep the earlier (lower) train index
-    if (s < bs[2]) {
-        bs[3] = bs[2]; bi[3] = bi[2];
-        if (s < bs[1]) {
-            bs[2] = bs[1]; bi[2] = bi[1];
-            if (s < bs[0]) { bs[1] = bs[0]; bi[1] = bi[0]; bs[0] = s; bi[0] = idx; }
-            else { bs[1] = s; bi[1] = idx; }
-        } else { bs[2] = s; bi[2] = idx; }
-    } else { bs[3] = s; bi[3] = idx; }
-}
-
-// 32 accumulator columns of one query row.  Common case: s = acc + |t|^2 (32 independent adds), a min
-// tree and ONE warp-uniform threshold test.  Rare case: only the groups of 8 columns that some lane
-// needs are re-read from TMEM in a rolled loop, and only the columns below the threshold are visited
-// -- the insert cascade exists once per call site, which keeps the loop inside the instruction cache
-// (fully unrolled it was 60 KB and 3x slower).  Re-computed scores are bit-identical to the first pass.
-template <int K>
-__device__ __forceinline__ void scan_chunk(const uint32_t (&v)[32], uint32_t taddr, const float4* __restrict__ tn4, int col0,
-                                           float slack, float (&bs)[K], int (&bi)[K])
-{
-    float gm[4];
-#pragma unroll
-    for (int g = 0; g < 4; g++) {
-        float4 na = tn4[g * 2], nb = tn4[g * 2 + 1];
-        float s0 = __fadd_rn(__uint_as_float(v[g * 8 + 0]), na.x), s1 = __fadd_rn(__uint_as_float(v[g * 8 + 1]), na.y);
-        float s2 = __fadd_rn(__uint_as_float(v[g * 8 + 2]), na.z), s3 = __fadd_rn(__uint_as_float(v[g * 8 + 3]), na.w);
-        float s4 = __fadd_rn(__uint_as_float(v[g * 8 + 4]), nb.x), s5 = __fadd_rn(__uint_as_float(v[g * 8 + 5]), nb.y);
-        float s6 = __fadd_rn(__uint_as_float(v[g * 8 + 6]), nb.z), s7 = __fadd_rn(__uint_as_float(v[g * 8 + 7]), nb.w);
-        gm[g] = fminf(fminf(fminf(s0, s1), fminf(s2, s3)), fminf(fminf(s4, s5), fminf(s6, s7)));
-    }
-    const float thr = fminf(bs[K - 1], __fadd_rn(bs[1], slack));
-    const unsigned mine = (gm[0] < thr ? 1u : 0u) | (gm[1] < thr ? 2u : 0u) | (gm[2] < thr ? 4u : 0u) | (gm[3] < thr ? 8u : 0u);
-    unsigned need = __reduce_or_sync(0xffffffffu, mine);
-    while (need) {                                  // warp-uniform
-        const int g = __ffs(need) - 1;
-        need &= need - 1;
-        uint32_t w[8];
-        tc_ld8(taddr + g * 8, w);
-        tc_wait_ld8(w);
-        const float4 na = tn4[g * 2], nb = tn4[g * 2 + 1];
-        if ((mine >> g) & 1u) {
-            float e[8];
-            e[0] = __fadd_rn(__uint_as_float(w[0]), na.x); e[1] = __fadd_rn(__uint_as_float(w[1]), na.y);
-            e[2] = __fadd_rn(__uint_as_float(w[2]), na.z); e[3] = __fadd_rn(__uint_as_float(w[3]), na.w);
-            e[4] = __fadd_rn(__uint_as_float(w[4]), nb.x); e[5] = __fadd_rn(__uint_as_float(w[5]), nb.y);
-            e[6] = __fadd_rn(__uint_as_float(w[6]), nb.z); e[7] = __fadd_rn(__uint_as_float(w[7]), nb.w);
-            unsigned m = (e[0] < thr ? 1u : 0u) | (e[1] < thr ? 2u : 0u) | (e[2] < thr ? 4u : 0u) | (e[3] < thr ? 8u : 0u) |
-                         (e[4] < thr ? 16u : 0u) | (e[5] < thr ? 32u : 0u) | (e[6] < thr ? 64u : 0u) | (e[7] < thr ? 128u : 0u);
-            while (m) {                             // usually a single column
-                const int j = __ffs(m) - 1;
-                m &= m - 1;
-                const float x = j == 0 ? e[0] : j == 1 ? e[1] : j == 2 ? e[2] : j == 3 ? e[3] : j == 4 ? e[4] : j == 5 ? e[5] : j == 6 ? e[6] : e[7];
-                if (x < fminf(bs[K - 1], __fadd_rn(bs[1], slack))) {
-                    if (K == 4) top4_insert(x, col0 + g * 8 + j, reinterpret_cast<float (&)[4]>(bs), reinterpret_cast<int (&)[4]>(bi));
-                    else topk_insert<K>(x, col0 + g * 8 + j, bs, bi);
-                }
-            }
-        }
-        __syncwarp();
-    }
-}
-
 // Candidate list of the one-product engine (knn_tc1.cu), 8 entries per (query row, list): [0], [1] = the two best scores so far in
 // order (all the threshold needs), [2..7] = a FIFO of the other columns that were within the slack of the runner-up when
 // they arrived (newest first).  An entry pushed out of the FIFO lowers floor_thr to its score (and with it the threshold),
@@ -511,34 +425,63 @@ static __device__ unsigned long long erp_clk[8];
 #define TCC_FLUSH()
 #endif
 
-// ---- the query-pair pipeline of knn_tc1.cu and knn_bin.cu --------------------------------------------------------------
+// one 128-byte k chunk of a K-major operand pair as four instructions over 32 bytes of every row; acc = false: the first
+// one overwrites the accumulator
+template <auto Mma>
+__device__ __forceinline__ void mma_chunk(uint32_t d_tmem, uint32_t a, uint32_t b, uint32_t idesc, bool acc)
+{
+#pragma unroll
+    for (int k = 0; k < 4; k++) Mma(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), idesc, acc || k != 0);
+}
+
+// ---- the query-pair pipeline of the four tcgen05 kernels --------------------------------------------------------------
+// knn_tc1.cu (f16) and knn_bin.cu (i8): four instructions per k chunk; score_tc.cu: one tf32 k chunk, hypothesis tiles
+// double-buffered (QB = 2); knn_tc.cu (3xTF32): one sub-tile of 2 x KCH chunks, hi and lo interleaved, up to eight
+// instructions per chunk.
 // SUB resident query sub-tiles of BM rows share every train tile of BN rows.  A row is KCH k chunks of one 128-byte swizzle
-// row (CK elements of the tensor maps).  The query sub-tiles sit in q_smem as [SUB][KCH] chunks, loaded once per segment;
-// the train chunks pass through a ring of NS slots in t_smem, the KCH chunks of a train tile in consecutive slots.  The
-// product of a sub-tile and a train tile goes to one of the two TMEM accumulators of BN columns, alternately.
-// Barriers: full / empty [NS] (chunk landed / read by the MMAs of the last sub-tile), qfull / qempty (query sub-tiles
-// landed / no longer read), tfull / tempty [2] (accumulator ready / drained, one arrival per epilogue warp).
-template <int SUB, int KCH, int NS, int BM, int BN, int CK>
+// row (CK elements of the tensor maps).  The query sub-tiles sit in q_smem as [QB][SUB][KCH] chunks, loaded once per
+// segment into buffer seg_n % QB; the train chunks pass through a ring of NS slots in t_smem, the KCH chunks of a train tile
+// in consecutive slots.  The product of a sub-tile and a train tile goes to one of the two TMEM accumulators of BN columns,
+// alternately.
+// Barriers, N_BARS of them from the constructor's base: full / empty [NS] (chunk landed / read by the MMAs of the last
+// sub-tile), qfull / qempty [QB] (query sub-tiles landed / no longer read), tfull / tempty [2] (accumulator ready /
+// drained, one arrival per epilogue warp).
+template <int SUB, int KCH, int NS, int BM, int BN, int CK, int QB = 1>
 struct PairPipe {
     static constexpr int QCH = BM * 128, TCH = BN * 128;    // bytes of a k chunk of a query sub-tile and of a train tile
+    static constexpr int N_BARS = 2 * NS + 2 * QB + 4;
     uint8_t* q_smem;
     uint8_t* t_smem;
     uint64_t *full, *empty, *qfull, *qempty, *tfull, *tempty;
 
-    // TMA producer (one thread)
-    __device__ __forceinline__ void produce(const CUtensorMap* map_q, const CUtensorMap* map_t, SegIter it) const
+    __device__ PairPipe(uint8_t* q, uint8_t* t, uint64_t* bars)
+        : q_smem(q), t_smem(t), full(bars), empty(bars + NS), qfull(bars + 2 * NS), qempty(qfull + QB), tfull(qempty + QB),
+          tempty(tfull + 2) {}
+
+    // one thread, after the kernel's own barriers: the fence publishes those too
+    __device__ __forceinline__ void init(int epi_warps) const
+    {
+        for (int i = 0; i < NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
+        for (int i = 0; i < QB; i++) { mbar_init(&qfull[i], 1); mbar_init(&qempty[i], 1); }
+        for (int i = 0; i < 2; i++) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], epi_warps); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+
+    // TMA producer (one thread); train tile tt of the plan is row block tt + t_off of map_t
+    __device__ __forceinline__ void produce(const CUtensorMap* map_q, const CUtensorMap* map_t, SegIter it, int t_off = 0) const
     {
         uint32_t slot = 0, ph = 0, seg_n = 0;
         int qp, t0, t1, seg;
         for (; it.next(qp, t0, t1, seg); seg_n++) {
-            mbar_wait(qempty, (seg_n & 1) ^ 1);
-            mbar_expect_tx(qfull, SUB * KCH * QCH);
+            const uint32_t qb = seg_n % QB;
+            mbar_wait(&qempty[qb], ((seg_n / QB) & 1) ^ 1);
+            mbar_expect_tx(&qfull[qb], SUB * KCH * QCH);
 #pragma unroll
             for (int sub = 0; sub < SUB; sub++)
 #pragma unroll
                 for (int c = 0; c < KCH; c++)
-                    tma_load_2d(map_q, qfull, q_smem + (sub * KCH + c) * QCH, c * CK, (qp * SUB + sub) * BM);
-            for (int tt = t0; tt < t1; tt++) {
+                    tma_load_2d(map_q, &qfull[qb], q_smem + ((qb * SUB + sub) * KCH + c) * QCH, c * CK, (qp * SUB + sub) * BM);
+            for (int tt = t0 + t_off; tt < t1 + t_off; tt++) {
 #pragma unroll
                 for (int c = 0; c < KCH; c++) {
                     mbar_wait(&empty[slot], ph ^ 1);
@@ -550,9 +493,10 @@ struct PairPipe {
         }
     }
 
-    // MMA issuer (one thread).  mma(d_tmem, a_desc, b_desc, accumulate) is one instruction over 32 bytes of every row.
-    // After the k chunks of a (sub-tile, train tile), hook(sub, tt_n, d_tmem) may add to the accumulator before it is
-    // committed to the epilogue; tt_n counts the train tiles of the CTA.
+    // MMA issuer (one thread).  mma(d_tmem, q, c, b) issues the products of k chunk c: q is the shared-memory address of the
+    // sub-tile's query chunks, b that of the train slot holding chunk c.  After the k chunks of a (sub-tile, train tile),
+    // hook(sub, tt_n, d_tmem) may add to the accumulator before it is committed to the epilogue; tt_n counts the train
+    // tiles of the CTA.
     template <class Mma, class Hook>
     __device__ __forceinline__ void issue(uint32_t tmem_base, SegIter it, Mma mma, Hook hook) const
     {
@@ -562,7 +506,8 @@ struct PairPipe {
         uint32_t tt_n = 0;
         int qp, t0, t1, seg;
         for (; it.next(qp, t0, t1, seg); seg_n++) {
-            mbar_wait(qfull, seg_n & 1);
+            const uint32_t qb = seg_n % QB;
+            mbar_wait(&qfull[qb], (seg_n / QB) & 1);
             for (int tt = t0; tt < t1; tt++, tt_n++) {
                 const uint32_t s0 = slot, p0 = ph;
 #pragma unroll
@@ -572,6 +517,7 @@ struct PairPipe {
                     mbar_wait(&tempty[acc], ((tile_n >> 1) & 1) ^ 1);
                     TCC_ADD(3, clock64() - m0); TCC_ADD(4, 1);
                     const uint32_t d_tmem = tmem_base + acc * BN;
+                    const uint32_t q = q_base + (qb * SUB + sub) * KCH * QCH;
                     uint32_t sl = s0, pp = p0;
 #pragma unroll
                     for (int c = 0; c < KCH; c++) {
@@ -579,9 +525,7 @@ struct PairPipe {
                         if (sub == 0) mbar_wait(&full[sl], pp);
                         TCC_ADD(5, clock64() - f0);
                         tc_fence_after();
-                        const uint32_t a = q_base + (sub * KCH + c) * QCH, b = t_base + sl * TCH;
-#pragma unroll
-                        for (int k = 0; k < 4; k++) mma(d_tmem, smem_desc_sw128(a + k * 32), smem_desc_sw128(b + k * 32), (c | k) != 0);
+                        mma(d_tmem, q, c, t_base + sl * TCH);
                         if (sub == SUB - 1) tc_commit(&empty[sl]);
                         if (++sl == NS) { sl = 0; pp ^= 1; }
                     }
@@ -590,7 +534,7 @@ struct PairPipe {
                     if (sub == SUB - 1) { slot = sl; ph = pp; }
                 }
             }
-            tc_commit(qempty);
+            tc_commit(&qempty[qb]);
         }
         TCC_FLUSH();
     }
@@ -613,6 +557,5 @@ struct PairPipe {
         if ((threadIdx.x & 31) == 0) mbar_arrive(&tempty[acc]);
     }
 };
-
 
 } // namespace erp
