@@ -248,7 +248,8 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
                         tile_n++;
                     }
                 }
-                // zero-filled columns past m have res = 0 exactly and were counted
+                // zero-filled columns past m have res = 0 exactly and were counted -- unless the hypothesis row is NaN
+                // (a sample with non-finite bearings): then nothing was counted, see the clamp below
                 pad_total += S_EPI_COLS - min(max(sh.m - colbase, 0), S_EPI_COLS);
             }
 #pragma unroll
@@ -256,7 +257,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_e, const __grid_constant
                 const int h = (ht * S_SUB + sub) * SM_ROWS + row;
                 if (h < sh.H) {
                     int n = pair_total(acc4[sub]);
-                    if (0.f < hi) n -= pad_total;
+                    if (0.f < hi) n = max(n - pad_total, 0);     // a finite row counted its pads: n >= pad_total
                     if (n) atomicAdd(p.upper + h, n);
                 }
             }
