@@ -461,7 +461,9 @@ __device__ void decompose_pose(const M3& Ec, float* pose)
 // rotation, ~15 rotations) was 40 % of the minimal-sample solver; here the eigenvalue comes from Newton's iteration on
 // the characteristic cubic started at 0 (monotone from below: the cubic is increasing and concave up to its first
 // root) and v3 from the largest cross product of two rows of M - lambda I: ~150 flops, one square root.  The result is
-// the same matrix to working precision; a (numerically) double smallest singular value falls back to the SVD.
+// the same matrix to working precision; a (numerically) double smallest singular value falls back to the SVD.  Next to a
+// double root Newton converges only linearly (each step halves the distance), so a loop that ends at its cap with steps
+// still above their rounding noise has not found lambda3 (sigma3 close to sigma2) and falls back as well.
 __device__ __forceinline__ bool rank2_project_fast(const M3& E, M3& Ec)
 {
     double m[6];                                  // M = E^T E, upper triangle: 00 01 02 11 12 22
@@ -477,13 +479,20 @@ __device__ __forceinline__ bool rank2_project_fast(const M3& E, M3& Ec)
     const double c2 = tr;
     const double c1 = (m[0] * m[3] - m[1] * m[1]) + (m[0] * m[5] - m[2] * m[2]) + (m[3] * m[5] - m[4] * m[4]);
     const double dE = det3(E), c0 = dE * dE;
-    double x = 0.0;
+    double x = 0.0, step = INFINITY, df = 0.0;
     for (int it = 0; it < 12; it++) {
-        const double f = ((x - c2) * x + c1) * x - c0, df = (3.0 * x - 2.0 * c2) * x + c1;
+        const double f = ((x - c2) * x + c1) * x - c0;
+        df = (3.0 * x - 2.0 * c2) * x + c1;
         if (!(df > 0.0)) return false;            // the two smallest eigenvalues (nearly) coincide
-        const double step = f / df;
+        step = f / df;
         x -= step;
         if (fabs(step) <= 1e-17 * tr) break;
+    }
+    // at the cap: converged only if the last step was at the rounding noise of f / df (the Horner terms of f round to a
+    // few ulp each), where the steps of a found root stall; a larger step is the linear approach to a double root
+    if (!(fabs(step) <= 1e-17 * tr)) {
+        const double ax = fabs(x);
+        if (!(fabs(step) <= 16.0 * DBL_EPSILON * (((ax + c2) * ax + c1) * ax + c0) / df)) return false;
     }
     if (!(x >= 0.0)) x = 0.0;
     // rows of A = M - x I
@@ -803,7 +812,13 @@ solve1_kernel(const double* __restrict__ Gin, int max_sweeps, double* __restrict
 // several digits per step: one 9 x 9 Cholesky factorisation and a handful of triangular solves on one thread, ~5 us.
 // mu = 1e-12 trace(G) keeps the factorisation defined for noise-free input (an exactly singular G).  The sign follows
 // E_best.  Only used for the RANSAC refit (sign-invariant consumers); the reference-mode solves keep OpenCV's Jacobi.
-__device__ void refit_inverse_iteration(const double* Gp /* packed upper triangle */, const double* x0, double* __restrict__ Eout,
+// The iteration stops when an iterate changes by less than 1e-14, or when the change stops halving and x is an
+// eigenvector to the rounding floor of G: ||G x - (x^T G x) x|| <= 64 eps trace(G), the floor the Jacobi solves stop at
+// too (the error of x is then at most that residual over the gap lambda2 - lambda1).  Each step shrinks the error only
+// by (lambda1 + mu) / (lambda2 + mu): on a low-parallax pair, where the two smallest eigenvalues are both noise and
+// within a factor of a few, the change stops halving long before the floor and the cap may come first.  It then returns
+// false without writing anything, and the caller solves the same G with the one-warp Jacobi.
+__device__ bool refit_inverse_iteration(const double* Gp /* packed upper triangle */, const double* x0, double* __restrict__ Eout,
                                         float* __restrict__ pose)
 {
     double L[9][9];
@@ -838,7 +853,9 @@ __device__ void refit_inverse_iteration(const double* Gp /* packed upper triangl
 #pragma unroll
         for (int i = 0; i < 9; i++) x[i] *= s;
     }
+    const double floor2 = (64.0 * DBL_EPSILON * trace) * (64.0 * DBL_EPSILON * trace);
     double prev = INFINITY;
+    bool converged = false;
     for (int it = 0; it < 24; it++) {
         double y[9];
 #pragma unroll
@@ -863,21 +880,42 @@ __device__ void refit_inverse_iteration(const double* Gp /* packed upper triangl
         double diff = 0.0;
 #pragma unroll
         for (int i = 0; i < 9; i++) { const double v = y[i] * s; diff = fmax(diff, fabs(v - x[i])); x[i] = v; }
-        // converged, or at the rounding floor of the solves (the change no longer shrinks)
-        if (diff < 1e-14 || (it > 0 && diff >= 0.5 * prev)) break;
+        // a change below 1e-14 leaves an error of at most 1e-14 r / (1 - r), r = lambda1 / lambda2, which is below the
+        // floor 64 eps trace / (lambda2 - lambda1) for every r
+        if (diff < 1e-14) { converged = true; break; }
+        const bool stalled = it > 0 && diff >= 0.5 * prev;
         prev = diff;
+        // the change no longer halves: at the rounding floor of the solves, or lambda1 / lambda2 >= 1/2 and still far
+        // from it; the residual tells the two apart (also at the cap)
+        if (!stalled && it < 23) continue;
+        double gx[9], rho = 0.0;
+#pragma unroll
+        for (int i = 0; i < 9; i++) {
+            double v = 0.0;
+#pragma unroll
+            for (int k = 0; k < 9; k++) v = __fma_rn(Gp[tri(i, k)], x[k], v);
+            gx[i] = v;
+            rho = __fma_rn(x[i], v, rho);
+        }
+        double res2 = 0.0;
+#pragma unroll
+        for (int i = 0; i < 9; i++) { const double d = __fma_rn(-rho, x[i], gx[i]); res2 = __fma_rn(d, d, res2); }
+        if (res2 <= floor2) { converged = true; break; }
     }
+    if (!converged) return false;
     M3 E;
 #pragma unroll
     for (int k = 0; k < 9; k++) E.v[k] = x[k];
     finish_hypothesis<true>(E, Eout, pose);
+    return true;
 }
 
 // ------------------------------------------------------------------ end of a RANSAC call, one launch
 // Inlier mask of the winning model, the Gram matrix of its inliers and the least-squares refit (eight_point.cpp:16-50 on
 // the inlier set): every block marks 256 correspondences and reduces their 45 Gram entries in a fixed order; the last
 // block to finish (one ticket) sums the per-block partials in block order (deterministic), solves the 9 x 9 system on its
-// first warp and writes the whole erp_ransac_result.  cnt: [0] inliers, [1] ticket (both zeroed by the caller).
+// first warp (inverse iteration on lane 0; the one-warp Jacobi when that does not converge) and writes the whole
+// erp_ransac_result.  cnt: [0] inliers, [1] ticket (both zeroed by the caller).
 constexpr int FIN_THREADS = 256;
 template <int METRIC>
 __global__ void __launch_bounds__(FIN_THREADS)
@@ -889,7 +927,8 @@ finish_kernel(const double* __restrict__ Eb, const uint64_t* __restrict__ packed
     __shared__ float Es[9];
     __shared__ double red[FIN_THREADS / 32][45];
     __shared__ double Gs[45];
-    __shared__ int last;
+    __shared__ Solve1Smem s1;
+    __shared__ int last, jacobi;
     const int m = dev_len(m_dev, m_cap);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     if (threadIdx.x == 0) scale_E(Eb, Es);
@@ -954,8 +993,11 @@ finish_kernel(const double* __restrict__ Eb, const uint64_t* __restrict__ packed
     __syncthreads();
     if (threadIdx.x < 45) Gs[threadIdx.x] = (((part[threadIdx.x] + part[45 + threadIdx.x]) + part[90 + threadIdx.x]) + part[135 + threadIdx.x]) + part[180 + threadIdx.x];
     __syncthreads();
+    if (threadIdx.x >= 32) return;
+    if (threadIdx.x == 0) jacobi = !refit_inverse_iteration(Gs, Eb, out->E_refit, out->pose);
+    __syncwarp();
+    if (jacobi) solve1_warp<true>(s1, Gs, 30, out->E_refit, out->pose);      // warp-uniform
     if (threadIdx.x != 0) return;
-    refit_inverse_iteration(Gs, Eb, out->E_refit, out->pose);
     {
         const uint64_t packed = *packed_dev;
         out->packed = packed;

@@ -16,6 +16,7 @@ import erp_match_eightpoint_test_b200 as erp
 import oracle as O
 from conftest import GOLDEN, e_dist
 from erp_match_eightpoint_test_b200 import binding, synth
+from test_gpu_geometry_edges import planted_reference, rank2_bar
 
 pytestmark = pytest.mark.gpu
 
@@ -210,19 +211,22 @@ def test_eight_point_batch_minimal_samples(ctx, scene, S):
     E, pose = ctx.eight_point_batch(l, r, samples=samples)
     Ephi, _ = ctx.eight_point_batch(l, r, H=H, S=S, seed=11, hyp_offset=0, want_pose=False)
     assert np.array_equal(E, Ephi)                         # device-drawn samples == replayed table
-    worst, n_bad = 0.0, 0
+    # every sample against the 50-digit projection of its 50-digit null vector, within the conditioning-aware bar of
+    # test_gpu_geometry_edges (kappa or kappa^2 of the S x 9 system, s1 / (s2 - s3) of the projected matrix)
+    A = np.einsum("hna,hnb->hnab", l[samples], r[samples]).reshape(H, S, 9)
+    sv, vt = np.linalg.svd(A)[1:]
+    worst = 0.0
     for h in range(H):
-        ref = O.eight_point(l[samples[h]], r[samples[h]], null_mode=1)
-        d = e_dist(E[h], ref["E"])
-        s = np.linalg.svd(np.einsum("na,nb->nab", l[samples[h]], r[samples[h]]).reshape(S, 9), compute_uv=False)
-        well = s[7] / s[0] > 1e-5                          # sample not (numerically) degenerate
-        if well:
-            worst = max(worst, d)
-            dr, dt, vok = _pose_close(pose[h], ref)
+        ref = planted_reference(l[samples[h]], r[samples[h]], {S: (sv[h], vt[h, -1])}, sizes=(S,))[S]
+        d, bar = e_dist(E[h], ref["Ec"]), rank2_bar(ref)
+        assert d <= bar, (h, d, bar, ref["kappa"], ref["sigma"])
+        worst = max(worst, d / bar)
+        if sv[h, 7] / sv[h, 0] > 1e-5:                     # the oracle and the pose are checked where the oracle's SVD is
+            oref = O.eight_point(l[samples[h]], r[samples[h]], null_mode=1)
+            assert e_dist(E[h], oref["E"]) < E_TOL
+            dr, dt, vok = _pose_close(pose[h], oref)
             assert dr < POSE_TOL * 10 and dt < POSE_TOL and vok, (h, dr, dt)
-        n_bad += d > E_TOL
-    assert worst < E_TOL, worst
-    assert n_bad <= H // 100
+    print("S=%d: worst error / bar %.2e" % (S, worst))
 
 
 def test_eight_point_estimation_and_golden(ctx, golden, scene):
